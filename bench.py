@@ -253,7 +253,14 @@ def main():
     ap.add_argument("--no-fit", action="store_true", help="skip the (untimed, separately reported) device hyper-parameter fit")
     ap.add_argument("--no-refresh-timing", action="store_true", help="skip the GP refresh timing loops (short profiler runs)")
     ap.add_argument("--no-extras", action="store_true", help="skip the sweep / strong / fp64 / reference-semantics / accuracy sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's result (best_value.npy, best_index.npy, float64) to DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.impl == "reference" and args.dump_outputs:
+        # the CPU arm scores as many candidates as fit its time budget, so its result is not reproducible
+        ap.error("--dump-outputs applies to the GPU path only, not to --impl reference")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -390,6 +397,11 @@ def main():
         e_j = clocks.pop("energy_j")
         clocks["energy_j_per_step"] = e_j / args.steps if wall >= 1.0 else None
     value = m_total * args.steps / (total_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # what score_sharded returns, identical on every rank; the index is exact in float64 (m_total < 2^53)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "best_value.npy"), np.array([result[0]], dtype=np.float64))
+        np.save(os.path.join(args.dump_outputs, "best_index.npy"), np.array([result[1]], dtype=np.float64))
 
     # ---- end-to-end: host candidates through the C-ABI host entry ------------------------------
     e2e = None
