@@ -62,8 +62,24 @@ enum {
   OMBO_ACQ_EI = 4,              /* optimisers.py:325-344 and its four copies              */
   OMBO_ACQ_CONSTRAINED_EI = 5,  /* cparego.py:486-496                                     */
   OMBO_ACQ_PARETO_EI = 6,       /* keep.py:142-150 (gp 0 = pareto model, gp 1 = scalar)   */
-  OMBO_ACQ_HV_POI = 7           /* emo.py:192-228                                         */
+  OMBO_ACQ_HV_POI = 7,          /* emo.py:192-228                                         */
+  OMBO_ACQ_EHVI_BOX = 8         /* exact EHVI, 2 <= n_obj <= 4, by box decomposition      */
 };
+
+/* OMBO_ACQ_EHVI_BOX: the exact expected hypervolume improvement for k = n_obj independent Gaussian objectives,
+ *   EHVI = sum_c prod_i (H_i(u_ci) - H_i(l_ci)),  H_i(t) = E[(t - y_i)^+] (H_i(-inf) = 0),
+ * over disjoint boxes [l_c, u_c] that tile the part of [-inf, ref] no front point dominates
+ * (host_prep.ehvi_boxes builds both tables).  It reuses the fields of ombo_acq:
+ *   n_obj   = k                      ref   = the reference point r
+ *   n_pf    = B, breakpoints per objective
+ *   stripes = DEVICE (k, B) f64: row i = -inf, the sorted distinct front coordinates of objective i, r_i,
+ *             padded with r_i to B
+ *   cells   = DEVICE (n_cells, 2, k) f64 holding integer breakpoint indices: [c][0] upper, [c][1] lower corner,
+ *             index 0 = -inf
+ * Each model's own variance is used (semantics is ignored).  Limits: 2 <= B <= OMBO_EHVI_BOX_MAX_BREAKS,
+ * 1 <= n_cells <= OMBO_EHVI_BOX_MAX_BOXES; indices outside [0, B) are clamped. */
+#define OMBO_EHVI_BOX_MAX_BREAKS 514        /* a front of up to 512 points */
+#define OMBO_EHVI_BOX_MAX_BOXES  (1 << 20)
 
 enum {
   OMBO_SC_WEIGHTED_SUM = 0, OMBO_SC_TCHEBICHEFF = 1, OMBO_SC_AUG_TCHEBICHEFF = 2,

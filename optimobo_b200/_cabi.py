@@ -19,6 +19,8 @@ PREC_FP64, PREC_FAST = 0, 1
 SEM_REFERENCE, SEM_EXACT = 0, 1
 (ACQ_NONE, ACQ_EHVI2D, ACQ_EHVI3D, ACQ_EXPECTED_DECOMP, ACQ_EI, ACQ_CONSTRAINED_EI,
  ACQ_PARETO_EI, ACQ_HV_POI) = range(8)
+ACQ_EHVI_BOX = 8
+EHVI_BOX_MAX_BREAKS, EHVI_BOX_MAX_BOXES = 514, 1 << 20
 (FIELD_L, FIELD_LINV, FIELD_ALPHA, FIELD_XS, FIELD_STATUS, FIELD_BHI, FIELD_BLO, FIELD_XS32,
  FIELD_ALPHA32) = range(9)
 

@@ -169,7 +169,8 @@ class AcquisitionSpec:
 
         if self.stripes is not None:
             a.stripes = up("stripes", self.stripes)
-            a.n_pf = self.stripes.shape[1] - 2
+            # EHVI2D: stripes are (2, P + 2); EHVI_BOX: the (k, B) breakpoint table
+            a.n_pf = self.stripes.shape[1] - (0 if self.kind == _cabi.ACQ_EHVI_BOX else 2)
         if self.cells is not None:
             a.cells = up("cells", self.cells)
             a.n_cells = self.cells.shape[0]
@@ -195,6 +196,17 @@ def spec_ehvi3d(max_point, PF, cache, semantics="reference"):
     k = cache.shape[1]
     return AcquisitionSpec(kind=_cabi.ACQ_EHVI3D, semantics=semantics, n_obj=k, ref=tuple(max_point),
                            best=host_prep.hypervolume(PF, max_point), cache=cache, n_models=k)
+
+
+def spec_ehvi_box(max_point, PF):
+    """Exact expected hypervolume improvement for 2 <= k <= 4 objectives: sum over the disjoint boxes of the region
+    no front point dominates (host_prep.ehvi_boxes) of prod_i (H_i(u_i) - H_i(l_i)), H_i(t) = E[(t - y_i)^+], with each
+    model's own mean and variance.  Not a reference acquisition; `semantics` does not apply."""
+    r = np.asarray(max_point, dtype=np.float64).reshape(-1)
+    table, boxes = host_prep.ehvi_boxes(PF, r)
+    k = len(r)
+    return AcquisitionSpec(kind=_cabi.ACQ_EHVI_BOX, n_obj=k, ref=tuple(r), stripes=table,
+                           cells=boxes.astype(np.float64), n_models=k)
 
 
 def spec_expected_decomposition(weights, agg_func, agg_function_min, cache, semantics="reference"):
@@ -513,6 +525,10 @@ def EHVI(X, models, max_point, PF, cache, semantics="reference", precision="fp64
 
 def EHVI_3D(X, models, max_point, PF, cache, semantics="reference", precision="fp64"):
     return evaluate(models, spec_ehvi3d(max_point, PF, cache, semantics), X, precision)
+
+
+def EHVI_box(X, models, max_point, PF, precision="fp64"):
+    return evaluate(models, spec_ehvi_box(max_point, PF), X, precision)
 
 
 def expected_decomposition(X, models, weights, agg_func, agg_function_min, cache, semantics="reference",

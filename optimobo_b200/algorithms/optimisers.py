@@ -5,14 +5,23 @@ from __future__ import annotations
 import numpy as np
 
 from .. import host_prep, result
-from ..acquisition import spec_ehvi, spec_ehvi3d, spec_ei, spec_expected_decomposition
+from ..acquisition import spec_ehvi, spec_ehvi3d, spec_ehvi_box, spec_ei, spec_expected_decomposition
 from .base import PoolOptimiserBase
 
 
 class MultiSurrogateOptimiser(PoolOptimiserBase):
     """One GP per objective; default acquisition 2-D EHVI (crude 3-D EHVI for 3 objectives), or the
     expected improvement over a scalarisation when `acquisition_func` is given
-    (optimisers.py:144-277)."""
+    (optimisers.py:144-277).
+
+    Additive knob `ehvi`: "reference" (default) keeps the reference's EHVI / crude 3-D EHVI above; "box" scores
+    every 2 to 4 objective problem with the exact EHVI over the box decomposition (`spec_ehvi_box`)."""
+
+    def __init__(self, test_problem, *args, ehvi="reference", **kwargs):
+        if ehvi not in ("reference", "box"):
+            raise ValueError(f"ehvi must be 'reference' or 'box' (got {ehvi!r})")
+        super().__init__(test_problem, *args, **kwargs)
+        self.ehvi = ehvi
 
     def _get_cached_samples(self, dimensions, sample_exponent):
         return host_prep.cached_samples(dimensions, sample_exponent, seed=int(self.rng.integers(0, 2 ** 31)))
@@ -30,7 +39,9 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
             ref_dir = np.asarray(ref_dirs[self.rng.integers(0, len(ref_dirs))])
             if acquisition_func is None:
                 pf = self._calc_pf(ysample)
-                if problem.n_obj == 2:
+                if self.ehvi == "box":
+                    spec = spec_ehvi_box(self.max_point, pf)
+                elif problem.n_obj == 2:
                     spec = spec_ehvi(self.max_point, pf, cached_samples, self.semantics)
                 else:
                     spec = spec_ehvi3d(self.max_point, pf, cached_samples, self.semantics)

@@ -10,6 +10,7 @@
 //   CONSTRAINED_EI    cparego.py:471-496
 //   PARETO_EI         keep.py:142-150
 //   HV_POI            emo.py:176-228
+//   EHVI_BOX          not in the reference: the exact k-objective EHVI over a box decomposition (k_acquire_box)
 // Arg-max replaces the inner optimiser call sites (differential_evolution at optimisers.py:87,
 // :118,:366; cparego.py:94,:544; emo.py:240; EA loops parego.py:242-270, keep.py:260-292):
 // warp shuffle -> block (smem) -> per-block partial -> one final block; ties resolve to the
@@ -304,10 +305,203 @@ int ombo_argmax_merge(ombo_ctx *ctx, int n_partials, ombo_best *best_dev, cudaSt
   return OMBO_OK;
 }
 
+// ---- K4 for OMBO_ACQ_EHVI_BOX: exact EHVI over the box decomposition -------------------------------
+// A CTA of 256 threads scores a tile of `tile` candidates (32, 16 or 8, chosen from B on the host):
+//   phase 1: V[cand][i][b] for every breakpoint t_b of every objective, spread over all threads (k*B Phi/phi pairs
+//            per candidate);
+//   phase 2: the boxes are staged BOX_CHUNK at a time as packed 16-bit indices; the G = 256 / tile slots of a
+//            candidate stride over them (the lanes of a warp: one box, different candidates), each box costing k table
+//            differences and multiplies; the slots are summed in a fixed order.
+// V keeps H(t) = E[(t - y)^+] below the mean and (t - r) + G(t), G(t) = E[(y - t)^+] = H(t) - (t - mu), at or above
+// it, so a box whose breakpoints both lie above the mean takes H(u) - H(l) = (u - l) + G(u) - G(l) without
+// subtracting two numbers ~ t - mu (the FP32 cancellation); a box that straddles the mean adds back r - mu.
+#define BOX_CHUNK 512
+
+// (n_boxes, 2, k) f64 breakpoint indices -> uint4 {u0 | u1 << 16, u2 | u3 << 16, l0 | l1 << 16, l2 | l3 << 16}; an
+// index outside [0, B) (or NaN) is clamped, so a malformed table cannot read past the V table
+__global__ void k_pack_boxes(const double *__restrict__ cells, int n_boxes, int k, int B, uint4 *__restrict__ out) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= n_boxes) return;
+  unsigned h[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  for (int s = 0; s < 2; ++s)
+    for (int i = 0; i < k; ++i) {
+      const double v = cells[((size_t)c * 2 + s) * k + i];
+      h[s * 4 + i] = v >= 0.0 ? (v < (double)(B - 1) ? (unsigned)v : (unsigned)(B - 1)) : 0u;
+    }
+  out[c] = make_uint4(h[0] | h[1] << 16, h[2] | h[3] << 16, h[4] | h[5] << 16, h[6] | h[7] << 16);
+}
+
+// odd candidate stride of V (in elements): the groups of one warp read the same box from different banks
+__host__ __device__ inline int box_cand_stride(int k, int B) { return (k * B) | 1; }
+
+template <typename T>
+__host__ __device__ inline size_t box_smem_bytes(int k, int B, int tile) {
+  return (size_t)BOX_CHUNK * 16 + (size_t)k * B * sizeof(T) + (size_t)tile * k * (3 * sizeof(T) + 4) +
+         (size_t)tile * box_cand_stride(k, B) * sizeof(T);
+}
+
+template <typename T, int K>
+__global__ void __launch_bounds__(ACQ_THREADS)
+k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double *__restrict__ var, long long m,
+              long long ld, long long index_base, const uint4 *__restrict__ boxes, double *__restrict__ out_acq,
+              ombo_best *__restrict__ partials) {
+  const int B = a.n_pf, n_boxes = a.n_cells, G = ACQ_THREADS / tile, cs = box_cand_stride(K, B);
+  uint4 *bx = reinterpret_cast<uint4 *>(acq_smem);                  // BOX_CHUNK staged boxes
+  T *V = reinterpret_cast<T *>(bx + BOX_CHUNK);                     // (tile, cs)
+  T *tr = V + tile * cs;                                            // (K, B) breakpoints t - r
+  T *sd = tr + K * B;                                               // (tile, K) sigma
+  T *rsd = sd + tile * K;                                           // (tile, K) 1 / sigma
+  T *shift = rsd + tile * K;                                        // (tile, K) r - mu
+  int *split = reinterpret_cast<int *>(shift + tile * K);           // (tile, K) first b with t_b - mu >= 0
+  const long long c0 = (long long)blockIdx.x * tile;
+
+  // the only FP64 arithmetic: t - r once per CTA and r - mu once per candidate and objective, so that t - mu =
+  // (t - r) + (r - mu) keeps its digits in FP32 when the front sits far from the origin (the FP64 pipe is narrow)
+  for (int e = threadIdx.x; e < K * B; e += ACQ_THREADS) tr[e] = (T)(a.stripes[e] - a.stripes[(e / B) * B + B - 1]);
+  for (int e = threadIdx.x; e < tile * K; e += ACQ_THREADS) {
+    const int j = e / K, i = e - j * K;
+    const long long c = c0 + j;
+    const double mv = c < m ? mu[i * ld + c] : 0.0, vv = c < m ? var[i * ld + c] : 1.0;
+    sd[e] = sqrt_t((T)vv);
+    rsd[e] = (T)1 / sd[e];
+    shift[e] = (T)(a.stripes[i * B + B - 1] - mv);
+    split[e] = B;                                                   // mu above every breakpoint
+  }
+  __syncthreads();
+  // phase 1: the V table
+  for (int e = threadIdx.x; e < tile * K * B; e += ACQ_THREADS) {
+    const int j = e / (K * B), ib = e - j * (K * B), i = ib / B, b = ib - i * B, jk = j * K + i;
+    T v = 0;                                                        // H(-inf) = 0
+    if (b > 0) {
+      const T c = shift[jk], s = sd[jk];
+      const T w = tr[ib] + c;                                       // t - mu
+      const T az = fabs(w * rsd[jk]);
+      const T g = s * phi(az) - fabs(w) * Phi(-az);                 // H(t) below the mean, G(t) above
+      v = w >= (T)0 ? tr[ib] + g : g;
+      if (tr[ib - 1] + c < (T)0 && w >= (T)0) split[jk] = b;        // one writer: t - mu is nondecreasing in b
+    }
+    V[j * cs + ib] = v;
+  }
+  __syncthreads();
+  // phase 2: the box sum.  Thread = (slot, candidate j): the lanes of a warp share a slot (tile 32; two slots at tile
+  // 16, four at 8), so they read one broadcast box and gather V of different candidates through the odd stride
+  const int j = threadIdx.x % tile, slot = threadIdx.x / tile;
+  const long long c = c0 + j;
+  T shj[K];
+  int spj[K];
+#pragma unroll
+  for (int i = 0; i < K; ++i) { shj[i] = shift[j * K + i]; spj[i] = split[j * K + i]; }
+  const T *Vj = V + j * cs;
+  T acc = 0;
+  for (int base = 0; base < n_boxes; base += BOX_CHUNK) {
+    const int n = min(BOX_CHUNK, n_boxes - base);
+    for (int e = threadIdx.x; e < n; e += ACQ_THREADS) bx[e] = boxes[base + e];
+    __syncthreads();
+    if (c < m) {
+      for (int q = slot; q < n; q += G) {
+        const uint4 p = bx[q];
+        const unsigned uu[4] = {p.x & 0xffffu, p.x >> 16, p.y & 0xffffu, p.y >> 16};
+        const unsigned ll[4] = {p.z & 0xffffu, p.z >> 16, p.w & 0xffffu, p.w >> 16};
+        T prod = 1;
+#pragma unroll
+        for (int i = 0; i < K; ++i) {
+          const int u = (int)uu[i], l = (int)ll[i];
+          T d = Vj[i * B + u] - Vj[i * B + l];
+          if (l < spj[i] && u >= spj[i]) d += shj[i];
+          prod = i == 0 ? d : prod * d;
+        }
+        acc += prod;
+      }
+    }
+    __syncthreads();
+  }
+  // the G slots of each candidate summed in a fixed order (bit-reproducible); the box stage is free after the loop
+  T *red = reinterpret_cast<T *>(bx);
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  double val = -INFINITY;
+  const bool owner = threadIdx.x < tile && c0 + threadIdx.x < m;
+  if (owner) {
+    T sum = 0;
+    for (int g = 0; g < G; ++g) sum += red[g * tile + threadIdx.x];
+    if (out_acq) out_acq[c0 + threadIdx.x] = (double)sum;
+    val = isnan(sum) ? -INFINITY : (double)sum;
+  }
+  // ---- K5: block arg-max ----
+  BestPair bb;
+  bb.v = val;
+  bb.i = owner ? index_base + c0 + threadIdx.x : 0x7fffffffffffffffLL;
+  bb = warp_best(bb);
+  __shared__ double sv[ACQ_THREADS / 32];
+  __shared__ long long si[ACQ_THREADS / 32];
+  if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = bb.v; si[threadIdx.x >> 5] = bb.i; }
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    BestPair q;
+    q.v = (threadIdx.x < ACQ_THREADS / 32) ? sv[threadIdx.x] : -INFINITY;
+    q.i = (threadIdx.x < ACQ_THREADS / 32) ? si[threadIdx.x] : 0x7fffffffffffffffLL;
+    q = warp_best(q);
+    if (threadIdx.x == 0) { partials[blockIdx.x].value = q.v; partials[blockIdx.x].index = q.i; }
+  }
+}
+
+// the largest tile whose shared memory leaves room for two CTAs per SM, else the largest that fits at all
+template <typename T>
+static int box_tile(int k, int B) {
+  for (int t = 32; t >= 8; t >>= 1) if (box_smem_bytes<T>(k, B, t) <= 110 * 1024) return t;
+  return box_smem_bytes<T>(k, B, 8) <= 220 * 1024 ? 8 : 0;          // + the static arg-max slots, under 227 KB
+}
+
+template <typename T, int K>
+static int launch_box(ombo_ctx *ctx, const ombo_acq *acq, const double *mu, const double *var, long long m,
+                      long long ld, long long index_base, double *out_acq, cudaStream_t s) {
+  const int tile = box_tile<T>(K, acq->n_pf);
+  OMBO_CHECK(tile > 0, "EHVI_BOX: %d breakpoints x %d objectives do not fit in shared memory", acq->n_pf, K);
+  const size_t smem = box_smem_bytes<T>(K, acq->n_pf, tile);
+  if (smem > 48 * 1024)
+    OMBO_CUDA(cudaFuncSetAttribute(k_acquire_box<T, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const long long blocks = (m + tile - 1) / tile;
+  int rc = ombo_ws_reserve(&ctx->ws_partial, &ctx->ws_partial_bytes, (size_t)blocks * sizeof(ombo_best));
+  if (rc) return rc;
+  k_acquire_box<T, K><<<(unsigned)blocks, ACQ_THREADS, smem, s>>>(*acq, tile, mu, var, m, ld, index_base,
+                                                                  (const uint4 *)ctx->ws_box, out_acq,
+                                                                  (ombo_best *)ctx->ws_partial);
+  ctx->launches += 1;
+  return (int)blocks;
+}
+
+static int ombo_acquire_box(ombo_ctx *ctx, const ombo_acq *acq, const double *mu, const double *var, long long m,
+                            long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
+                            cudaStream_t s, bool fp32) {
+  const int k = acq->n_obj;
+  int rc = ombo_ws_reserve(&ctx->ws_box, &ctx->ws_box_bytes, (size_t)acq->n_cells * sizeof(uint4));
+  if (rc) return rc;
+  k_pack_boxes<<<(acq->n_cells + 255) / 256, 256, 0, s>>>(acq->cells, acq->n_cells, k, acq->n_pf,
+                                                          (uint4 *)ctx->ws_box);
+  ctx->launches += 1;
+  fp32 = fp32 && !ctx->knobs.acq_fp64;
+  int blocks;
+  if (k == 2) blocks = fp32 ? launch_box<float, 2>(ctx, acq, mu, var, m, ld, index_base, out_acq, s)
+                            : launch_box<double, 2>(ctx, acq, mu, var, m, ld, index_base, out_acq, s);
+  else if (k == 3) blocks = fp32 ? launch_box<float, 3>(ctx, acq, mu, var, m, ld, index_base, out_acq, s)
+                                 : launch_box<double, 3>(ctx, acq, mu, var, m, ld, index_base, out_acq, s);
+  else blocks = fp32 ? launch_box<float, 4>(ctx, acq, mu, var, m, ld, index_base, out_acq, s)
+                     : launch_box<double, 4>(ctx, acq, mu, var, m, ld, index_base, out_acq, s);
+  if (blocks < 0) return blocks;
+  if (best_dev) {
+    k_argmax_final<<<1, 1024, 0, s>>>((const ombo_best *)ctx->ws_partial, blocks, best_dev);
+    ctx->launches += 1;
+  }
+  OMBO_CUDA(cudaGetLastError());
+  return OMBO_OK;
+}
+
 int ombo_acquire(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var,
                  long long m, long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
                  cudaStream_t s, bool fp32) {
   if (m <= 0) return OMBO_OK;
+  if (acq->kind == OMBO_ACQ_EHVI_BOX)
+    return ombo_acquire_box(ctx, acq, mu, var, m, ld, index_base, out_acq, best_dev, s, fp32);
   int n_stage = 0;
   if (acq->kind == OMBO_ACQ_EHVI2D) n_stage = 2 * (acq->n_pf + 2);
   else if (acq->kind == OMBO_ACQ_HV_POI) n_stage = acq->n_cells * 2 * acq->n_obj;

@@ -100,6 +100,7 @@ int ombo_ctx_destroy(ombo_ctx *c) {
   if (c->ws_post) cudaFree(c->ws_post);
   if (c->ws_scratch) cudaFree(c->ws_scratch);
   if (c->ws_partial) cudaFree(c->ws_partial);
+  if (c->ws_box) cudaFree(c->ws_box);
   for (int i = 0; i < 2; ++i) {
     if (c->ws_stage[i]) cudaFree(c->ws_stage[i]);
     cudaEventDestroy(c->ev_copied[i]);
@@ -200,6 +201,15 @@ static int validate_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const omb
     case OMBO_ACQ_HV_POI:
       OMBO_CHECK(n_gp >= 2 && acq->n_obj == 2 && acq->cells && acq->n_cells >= 1, "HV_POI needs 2 GPs, n_obj = 2 and the cells");
       break;
+    case OMBO_ACQ_EHVI_BOX:
+      OMBO_CHECK(k >= 2 && k <= OMBO_MAX_OBJ && n_gp >= k && acq->stripes && acq->cells,
+                 "EHVI_BOX needs 2 <= n_obj <= %d, n_obj GPs, the breakpoint table and the boxes", OMBO_MAX_OBJ);
+      OMBO_CHECK(acq->n_pf >= 2 && acq->n_pf <= OMBO_EHVI_BOX_MAX_BREAKS,
+                 "EHVI_BOX: %d breakpoints per objective, supported 2..%d (a front of up to %d points)", acq->n_pf,
+                 OMBO_EHVI_BOX_MAX_BREAKS, OMBO_EHVI_BOX_MAX_BREAKS - 2);
+      OMBO_CHECK(acq->n_cells >= 1 && acq->n_cells <= OMBO_EHVI_BOX_MAX_BOXES,
+                 "EHVI_BOX: %d boxes, supported 1..%d", acq->n_cells, OMBO_EHVI_BOX_MAX_BOXES);
+      break;
     default: ombo_set_error("score: unknown acquisition kind %d", acq->kind); return OMBO_ERR_INVALID;
   }
   OMBO_CHECK(acq->semantics == OMBO_SEM_REFERENCE || acq->semantics == OMBO_SEM_EXACT, "score: unknown semantics");
@@ -257,6 +267,7 @@ static int score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_po
         case OMBO_ACQ_EI: want_var = (g == 0); break;
         case OMBO_ACQ_PARETO_EI: want_var = (g == 1); break;
         case OMBO_ACQ_HV_POI: want_var = (g < 2); break;
+        case OMBO_ACQ_EHVI_BOX: want_var = (g < acq->n_obj); break;
         default: want_var = true;
       }
     }

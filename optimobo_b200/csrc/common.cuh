@@ -69,6 +69,7 @@ struct ombo_ctx {
   void *ws_post;      size_t ws_post_bytes;      // posterior mu/var chunk buffers
   void *ws_scratch;   size_t ws_scratch_bytes;   // FP64 K* tiles (L2 resident) / fast-path scratch
   void *ws_partial;   size_t ws_partial_bytes;   // per-block arg-max partials
+  void *ws_box;       size_t ws_box_bytes;       // EHVI_BOX boxes as packed 16-bit breakpoint indices
   void *ws_stage[2];  size_t ws_stage_bytes;     // host-entry H2D staging (double buffered)
   void *ws_best;                                  // 16 B device best for the host entry
   ombo_best *pinned_best;                         // pinned host landing zone

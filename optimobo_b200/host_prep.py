@@ -66,6 +66,62 @@ def ehvi_stripes(PF, ref_point):
     return np.stack([y1, y2])
 
 
+def ehvi_boxes(PF, ref_point):
+    """Disjoint boxes tiling {z <= r : no front point dominates z} (minimisation), for the exact EHVI of
+    2 <= k <= 4 objectives.  Points not <= r are dropped and the first front is taken; the region is sliced on the
+    last objective between consecutive distinct values t_j < z_k <= t_{j+1}, and each slice holds the (k-1)-D
+    decomposition for the front of the points with f_k <= t_j.
+
+    Returns (table, boxes):
+      table (k, B) float64: row i = [-inf, sorted distinct front coordinates of objective i, r_i], padded with r_i;
+      boxes (n_boxes, 2, k) int64 indices into the rows: [c][0] upper, [c][1] lower corner, 0 = -inf.
+    An empty front gives the single box [-inf, r]."""
+    r = np.asarray(ref_point, dtype=np.float64).reshape(-1)
+    k = len(r)
+    if not 2 <= k <= 4:
+        raise ValueError(f"ehvi_boxes takes 2 to 4 objectives (got {k})")
+    P = np.asarray(PF, dtype=np.float64).reshape(-1, k)
+    P = calc_pf(P[np.all(P <= r, axis=1)])
+    P = np.unique(P, axis=0)
+    rows = [np.concatenate(([-np.inf], np.unique(P[:, i]), [r[i]])) for i in range(k)]
+    lo, hi = _slice_boxes(P, r)
+    boxes = np.empty((len(lo), 2, k), dtype=np.int64)
+    for i in range(k):
+        boxes[:, 0, i] = np.searchsorted(rows[i], hi[:, i], side="left")
+        boxes[:, 1, i] = np.searchsorted(rows[i], lo[:, i], side="left")
+    B = max(len(row) for row in rows)
+    table = np.stack([np.concatenate((row, np.full(B - len(row), r[i]))) for i, row in enumerate(rows)])
+    return table, boxes
+
+
+def _slice_boxes(P, r):
+    """(lower, upper) corners, each (n_boxes, k), of the decomposition ehvi_boxes describes; P is a front <= r."""
+    k = len(r)
+    if k == 2:
+        # slice j of f2 between t_j and t_{j+1}: f1 is free up to the least f1 of the points with f2 <= t_j
+        t = np.unique(P[:, 1])
+        edges = np.concatenate(([-np.inf], t, [r[1]]))
+        S = P[np.argsort(P[:, 1], kind="stable")]
+        run = np.minimum.accumulate(S[:, 0]) if len(S) else S[:, 0]
+        last = np.searchsorted(S[:, 1], t, side="right") - 1          # last point with f2 <= t_j
+        right = np.concatenate(([r[0]], run[last]))
+        keep = edges[1:] > edges[:-1]
+        lo = np.column_stack([np.full(keep.sum(), -np.inf), edges[:-1][keep]])
+        hi = np.column_stack([right[keep], edges[1:][keep]])
+        return lo, hi
+    t = np.unique(P[:, -1])
+    edges = np.concatenate(([-np.inf], t, [r[-1]]))
+    los, his = [], []
+    for j in range(len(edges) - 1):
+        if edges[j + 1] <= edges[j]:
+            continue
+        sub = calc_pf(P[P[:, -1] <= edges[j], :-1])
+        lo, hi = _slice_boxes(sub, r[:-1])
+        los.append(np.column_stack([lo, np.full(len(lo), edges[j])]))
+        his.append(np.column_stack([hi, np.full(len(hi), edges[j + 1])]))
+    return np.concatenate(los), np.concatenate(his)
+
+
 def cache_covariance(cache):
     """(C00, C01) of np.cov(cache[:,0], cache[:,1]); the reference's EHVI passes
     var0*C00, var0*C01 as 'sigma' (util_functions.py:163,167; SURVEY section 0.4)."""
