@@ -108,11 +108,16 @@ __device__ double scalarise(const ombo_acq &a, const double *F) {
 }
 
 // ---- EI ----------------------------------------------------------------------------------
+// T = float: best - mu and var + eps are formed in FP64 before the cast (a pool far from the origin keeps the digits of
+// its spread), and below g = -5, where g Phi(g) + phi(g) cancels and then flushes, the lane switches to FP64: the
+// result is a double, so EI down to ~1e-300 (g ~ -37) survives.  Natural pools rarely have such lanes.
 template <typename T>
-__device__ __forceinline__ T ei_value(T mu, T var, T best, T eps) {
-  T s = sqrt_t(var + eps);
-  T g = (best - mu) / (s + (T)1e-10);
-  return s * (g * Phi(g) + phi(g));
+__device__ __forceinline__ double ei_value(double mu, double var, double best, double eps) {
+  T s = sqrt_t((T)(var + eps));
+  T g = (T)(best - mu) / (s + (T)1e-10);
+  if (sizeof(T) == sizeof(double) || !(g < (T)-5)) return s * (g * Phi(g) + phi(g));
+  const double sd = sqrt(var + eps), gd = (best - mu) / (sd + 1e-10);
+  return fmax(sd * (gd * Phi(gd) + phi(gd)), 0.0);       // below g ~ -37 the FP64 terms cancel to +-subnormals
 }
 
 extern __shared__ __align__(16) double acq_smem[];
@@ -140,7 +145,7 @@ k_acquire(ombo_acq a, int n_gp, const double *__restrict__ mu, const double *__r
   if (c < m) {
     T mus[OMBO_MAX_GP], vars[OMBO_MAX_GP];
     for (int g = 0; g < n_gp; ++g) { mus[g] = (T)mu[g * ld + c]; vars[g] = (T)var[g * ld + c]; }
-    T r = (T)nan("");
+    double r = nan("");
     switch (a.kind) {
       case OMBO_ACQ_EHVI2D: {
         const int P = a.n_pf;
@@ -173,17 +178,18 @@ k_acquire(ombo_acq a, int n_gp, const double *__restrict__ mu, const double *__r
         }
         r = total / (T)S;
       } break;
+      // the EI family reads its inputs as doubles (ei_value)
       case OMBO_ACQ_EI:
-        r = ei_value<T>(mus[0], vars[0], (T)a.best, (T)a.var_eps[0]);
+        r = ei_value<T>(mu[c], var[c], a.best, a.var_eps[0]);
         break;
       case OMBO_ACQ_CONSTRAINED_EI: {
-        r = ei_value<T>(mus[0], vars[0], (T)a.best, (T)a.var_eps[0]);
-        T pof = 1;
-        for (int g = 1; g < n_gp; ++g) pof *= Phi(((T)0 - mus[g]) / sqrt_t(vars[g] + (T)a.var_eps[g]));
+        r = ei_value<T>(mu[c], var[c], a.best, a.var_eps[0]);
+        double pof = 1;           // a mostly infeasible pool is a product of small probabilities: accumulated in FP64
+        for (int g = 1; g < n_gp; ++g) pof *= Phi_wide(((T)0 - mus[g]) / sqrt_t(vars[g] + (T)a.var_eps[g]));
         r = r * pof;
       } break;
       case OMBO_ACQ_PARETO_EI:
-        r = mus[0] * ei_value<T>(mus[1], vars[1], (T)a.best, (T)a.var_eps[1]);
+        r = mu[c] * ei_value<T>(mu[ld + c], var[ld + c], a.best, a.var_eps[1]);
         break;
       case OMBO_ACQ_HV_POI: {
         const int k = 2;     // emo.py:21 "Only works for 2D so far"
@@ -195,7 +201,10 @@ k_acquire(ombo_acq a, int n_gp, const double *__restrict__ mu, const double *__r
           T p = 1, vol = 1;
           bool valid = true;
           for (int i = 0; i < k; ++i) {
-            T pi = Phi((U[i] - mus[i]) / sd[i]) - Phi((Lo[i] - mus[i]) / sd[i]);
+            const T za = (U[i] - mus[i]) / sd[i], zb = (Lo[i] - mus[i]) / sd[i];
+            // FP32: a cell above the mean (za > zb > 0) takes the difference of the two upper tails, which keeps its
+            // digits where Phi(za) - Phi(zb) is a difference of two numbers near 1
+            T pi = (sizeof(T) == sizeof(float) && zb > (T)0) ? Phi(-zb) - Phi(-za) : Phi(za) - Phi(zb);
             p = (i == 0) ? pi : p * pi;
             valid = valid && (U[i] > mus[i]);
             T e = U[i] - fmax_t(Lo[i], mus[i]);
@@ -331,6 +340,11 @@ __global__ void k_pack_boxes(const double *__restrict__ cells, int n_boxes, int 
   out[c] = make_uint4(h[0] | h[1] << 16, h[2] | h[3] << 16, h[4] | h[5] << 16, h[6] | h[7] << 16);
 }
 
+// s h(-az) = s phi(az) - |w| Phi(-az), az = |w| / s: H(t) below the mean, G(t) above it.  FP32 takes the tail-safe
+// h_norm (far from the mean the two terms cancel, and turn negative once phi flushes)
+__device__ __forceinline__ double shortfall_tail(double s, double az, double w) { return s * phi(az) - fabs(w) * Phi(-az); }
+__device__ __forceinline__ float shortfall_tail(float s, float az, float) { return s * h_norm(-az); }
+
 // odd candidate stride of V (in elements): the groups of one warp read the same box from different banks
 __host__ __device__ inline int box_cand_stride(int k, int B) { return (k * B) | 1; }
 
@@ -376,7 +390,7 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
       const T c = shift[jk], s = sd[jk];
       const T w = tr[ib] + c;                                       // t - mu
       const T az = fabs(w * rsd[jk]);
-      const T g = s * phi(az) - fabs(w) * Phi(-az);                 // H(t) below the mean, G(t) above
+      const T g = shortfall_tail(s, az, w);                         // H(t) below the mean, G(t) above
       v = w >= (T)0 ? tr[ib] + g : g;
       if (tr[ib - 1] + c < (T)0 && w >= (T)0) split[jk] = b;        // one writer: t - mu is nondecreasing in b
     }
