@@ -152,6 +152,13 @@ int ombo_gp_nlml_grad(ombo_ctx *ctx, const ombo_gp_spec *spec, void *state, doub
  * products (2.0 tensor units per MAC instead of 3.0).  Chosen only when the refresh was asked for it (spec bit 2),
  * d <= 12 and the conditioning proxy is below the measured limit (DESIGN.md section 4). */
 #define OMBO_GP_F8C_PLANES 4
+
+/* ombo_acq.reserved bit 0 (EHVI2D): the stripes come from a valid staircase -- a front sorted by objective 2,
+ * mutually non-dominated and inside the reference point, as spec_ehvi builds it.  With this bit, exact semantics,
+ * the fast precision mode, two f8c-plane GPs and only `best` requested, ombo_score skips the full variance of the
+ * candidates a variance bound proves cannot win (same result; DESIGN.md section 4).  That path synchronises the
+ * stream once (it reads the number of survivors back).  A caller that leaves `reserved` 0 keeps the unpruned path. */
+#define OMBO_ACQ_FRONT_VALID 1
 typedef struct {
   int32_t n, d, kernel, reserved;
   double sigma_f2, sigma_n2;

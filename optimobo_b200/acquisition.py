@@ -149,6 +149,7 @@ class AcquisitionSpec:
     cells: np.ndarray | None = None
     cache: np.ndarray | None = None
     n_models: int = 1
+    reserved: int = 0          # ombo_acq.reserved (EHVI2D: _cabi.ACQ_FRONT_VALID)
     _dev: dict = field(default_factory=dict, repr=False)
 
     def c_struct(self, device):
@@ -160,6 +161,7 @@ class AcquisitionSpec:
             for i, v in enumerate(src):
                 dst[i] = float(v)
         a.cache_c00, a.cache_c01 = self.cache_c
+        a.reserved = self.reserved
 
         def up(name, arr):
             key = (name, str(device))
@@ -185,9 +187,11 @@ def spec_ehvi(max_point, PF, cache, semantics="reference"):
     PF = np.atleast_2d(np.asarray(PF, dtype=np.float64))
     if PF.shape[1] != 2:
         raise ValueError("EHVI is 2-objective; use spec_ehvi3d for 3 objectives")
+    valid = host_prep.front_is_staircase(PF, max_point)
     return AcquisitionSpec(kind=_cabi.ACQ_EHVI2D, semantics=semantics, n_obj=2, ref=tuple(max_point),
                            stripes=host_prep.ehvi_stripes(PF, max_point),
-                           cache_c=host_prep.cache_covariance(cache), n_models=2)
+                           cache_c=host_prep.cache_covariance(cache), n_models=2,
+                           reserved=_cabi.ACQ_FRONT_VALID if valid else 0)
 
 
 def spec_ehvi3d(max_point, PF, cache, semantics="reference"):

@@ -2,6 +2,10 @@
 #include <stdarg.h>
 #include <stdlib.h>
 
+#include <cub/device/device_select.cuh>
+#include <cub/iterator/counting_input_iterator.cuh>
+
+#include "acq_math.cuh"
 #include "candidates.cuh"
 
 static thread_local char g_err[1024] = "";
@@ -71,7 +75,7 @@ int ombo_ctx_create(int device, ombo_ctx **out) {
     k.fast_nocache = getenv("OMBO_FAST_NOCACHE") != nullptr;
     k.fast_zerocache = getenv("OMBO_FAST_ZEROCACHE") != nullptr;
     k.fast_mean_in_main = getenv("OMBO_FAST_MEAN_IN_MAIN") != nullptr;
-    k.fast_gen_warps = geti("OMBO_FAST_GEN_WARPS", 8);
+    k.fast_gen_warps = geti("OMBO_FAST_GEN_WARPS", 0);
     k.f8_max_run = geti("OMBO_F8_MAXRUN", 0);
     { const char *e = getenv("OMBO_F8_TG"); k.f8_tg = e ? atof(e) : 3.0; }
     k.chunk_log2 = geti("OMBO_CHUNK_LOG2", OMBO_CHUNK_DEV_LOG2);
@@ -81,6 +85,10 @@ int ombo_ctx_create(int device, ombo_ctx **out) {
     { const char *e = getenv("OMBO_F8C_KAPPA"); k.f8c_kappa = e ? atof(e) : OMBO_F8C_KAPPA_DEFAULT; }
     k.acq_fp64 = getenv("OMBO_ACQ_FP64") != nullptr;
     k.no_fuse = getenv("OMBO_NO_FUSE") != nullptr;
+    k.no_prune = getenv("OMBO_NO_PRUNE") != nullptr;
+    k.prune_depth = geti("OMBO_PRUNE_DEPTH", 1) >= 2 ? 2 : 1;
+    { const char *e = getenv("OMBO_PRUNE_CAP"); k.prune_cap = e ? atoll(e) : 0; }
+    k.prune_log = getenv("OMBO_PRUNE_LOG") != nullptr;
   }
   OMBO_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; ++i) {
@@ -108,7 +116,8 @@ int ombo_ctx_destroy(ombo_ctx *c) {
   }
   if (c->prof_ev[0]) for (int i = 0; i < 2 * OMBO_PROF_MAX; ++i) cudaEventDestroy(c->prof_ev[i]);
   if (c->prof_dev) cudaFree(c->prof_dev);
-  if (c->f8_sched) cudaFree(c->f8_sched);
+  for (int i = 0; i < 2; ++i) if (c->f8_sched[i]) cudaFree(c->f8_sched[i]);
+  if (c->ws_prune) cudaFree(c->ws_prune);
   if (c->ws_best) cudaFree(c->ws_best);
   if (c->pinned_best) cudaFreeHost(c->pinned_best);
   cudaStreamDestroy(c->copy_stream);
@@ -227,7 +236,8 @@ static void fill_pool_dev(PoolDev &pd, const ombo_pool *pool) {
 // scores rows [first, first+count) of the pool; X_dev points at row `first` (or NULL -> generator)
 static int score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const void *X_dev,
                       long long first, long long count, const ombo_acq *acq, int precision, double *out_mu,
-                      double *out_var, double *out_acq, long long out_ld, ombo_best *best_dev, cudaStream_t s) {
+                      double *out_var, double *out_acq, long long out_ld, ombo_best *best_dev, cudaStream_t s,
+                      int bound_chunks = 0) {
   PoolDev pd;
   fill_pool_dev(pd, pool);
   pd.X = X_dev;
@@ -288,13 +298,179 @@ static int score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_po
     int rc = (precision == OMBO_PREC_FP64)
                  ? ombo_posterior_fp64(ctx, gd, pd, count, mu + (size_t)g * ld, var + (size_t)g * ld, want_var, s)
                  : ombo_posterior_fast(ctx, gd, pd, count, mu + (size_t)g * ld, var + (size_t)g * ld, want_var, s,
-                                       try_fuse ? &fq : nullptr, &fused);
+                                       try_fuse ? &fq : nullptr, &fused, bound_chunks);
     if (rc) return rc;
   }
   if (fused) return best_dev ? ombo_argmax_merge(ctx, fused, best_dev, s) : OMBO_OK;
   if (acq->kind != OMBO_ACQ_NONE)
     return ombo_acquire(ctx, acq, n_gp, mu, var, count, ld, pd.index_base, out_acq ? out_acq + first : nullptr,
                         best_dev, s, precision == OMBO_PREC_FAST);
+  return OMBO_OK;
+}
+
+// every pass of a pool (2^chunk_log2 candidates each) through score_pass
+static int score_passes(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
+                        int precision, double *out_mu, double *out_var, double *out_acq, ombo_best *best_dev,
+                        cudaStream_t s, int bound_chunks = 0) {
+  const size_t esz = pool->dtype == 0 ? 8 : 4;
+  const long long chunk = 1LL << ctx->knobs.chunk_log2;
+  for (long long first = 0; first < pool->m; first += chunk) {
+    long long count = pool->m - first < chunk ? pool->m - first : chunk;
+    const void *X = pool->X ? (const char *)pool->X + (size_t)first * pool->d * esz : nullptr;
+    int rc = score_pass(ctx, gps, n_gp, pool, X, first, count, acq, precision, out_mu, out_var, out_acq, pool->m,
+                        best_dev, s, bound_chunks);
+    if (rc) return rc;
+  }
+  return OMBO_OK;
+}
+
+// ---- pruned arg-max (fast mode, exact-semantics 2-D EHVI, only `best` asked for) ---------------------------------
+// The bound pass scores every candidate with its exact mean and an upper bound on each variance (posterior_fast8.cu,
+// BOUND schedule: the first OMBO_PRUNE_DEPTH chunks of V).  Over a valid front the exact EHVI never decreases in
+// either sigma (DESIGN.md section 4), so that score UB_i bounds the candidate's value from above.  The candidate with
+// the largest UB is scored in full; its value v0 is a lower bound on the pool's best, and only candidates with
+// UB_i >= v0 - tau can reach it.  Those are gathered into an explicit pool and scored in full, through the same
+// fused path as the unpruned call, so the winner and its value are the unpruned call's.
+//
+// tau covers the FP32 evaluation of ehvi2d_value on both sides (the computed function is monotone in sigma only up
+// to rounding): twice the FP32 contract of the acquisition (relative 1e-3 of the value, DESIGN.md section 4).
+#define OMBO_PRUNE_TAU 2e-3
+
+struct PruneHdr {                 // device, read back by one copy after the selection
+  ombo_best ub;                   // largest upper bound (value, global index)
+  ombo_best v0;                   // full score of that candidate (index: 0, it was scored alone)
+  ombo_best loc;                  // best survivor (index: position in the survivor list)
+  long long n_sel;                // survivors
+};
+static_assert(sizeof(PruneHdr) <= 64, "PruneHdr is read back through the context's 64-byte pinned buffer");
+
+struct PruneKeep {                // survivor test of local candidate i
+  const double *ub;
+  const PruneHdr *h;
+  __device__ bool operator()(long long i) const {
+    const double u = ub[i];
+    return isnan(u) || u >= h->v0.value - OMBO_PRUNE_TAU * h->ub.value;
+  }
+};
+
+__global__ void k_prune_init(PruneHdr *h) {
+  h->ub.value = h->v0.value = h->loc.value = -INFINITY;
+  h->ub.index = h->v0.index = h->loc.index = -1;
+  h->n_sel = 0;
+}
+
+// rows of the listed local candidates (idx == NULL: the one with the largest bound) into an explicit pool, converted
+// exactly as the kernels read them: the f32 values of an f32 pool, the f64 coordinates of an f64 or counter pool
+__global__ void k_prune_gather(PoolDev pool, long long m, const long long *__restrict__ idx,
+                               const PruneHdr *__restrict__ h, long long n, void *__restrict__ out, int out_f32) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n * pool.d) return;
+  const long long r = e / pool.d;
+  const int j = (int)(e % pool.d);
+  long long c = idx ? idx[r] : h->ub.index - pool.index_base;
+  if (c < 0 || c >= m) c = 0;                     // no finite bound: the host falls back before using this row
+  const double x = ombo_pool_coord(pool, c, j);
+  if (out_f32) ((float *)out)[e] = (float)x;
+  else ((double *)out)[e] = x;
+}
+
+// the threshold candidate and the best survivor, mapped to global indices, merged into the running best
+__global__ void k_prune_merge(const PruneHdr *__restrict__ h, const long long *__restrict__ idx, long long base,
+                              ombo_best *__restrict__ best) {
+  BestPair b;
+  b.v = h->v0.value; b.i = h->ub.index;
+  if (h->loc.index >= 0) {
+    const long long gi = base + idx[h->loc.index];
+    if (better(h->loc.value, gi, b.v, b.i)) { b.v = h->loc.value; b.i = gi; }
+  }
+  if (best->index < 0 || better(b.v, b.i, best->value, best->index)) { best->value = b.v; best->index = b.i; }
+}
+
+static bool prune_eligible(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
+                           int precision, const double *out_mu, const double *out_acq, const ombo_best *best_dev,
+                           cudaStream_t s) {
+  if (precision != OMBO_PREC_FAST || n_gp != 2 || acq->kind != OMBO_ACQ_EHVI2D || acq->semantics != OMBO_SEM_EXACT ||
+      !(acq->reserved & OMBO_ACQ_FRONT_VALID) || out_mu || out_acq || !best_dev || pool->m < 1 ||
+      ctx->knobs.no_prune || ctx->knobs.no_fuse || ctx->knobs.acq_fp64)
+    return false;
+  // timing experiments (OMBO_FAST_DBG) compute garbage; the bound is derived from the pass schedule, so a full launch
+  // on the rolling schedule (OMBO_F8_MAXRUN) would not share chunk 0's accumulation order with it
+  if (ctx->knobs.fast_dbg || ctx->knobs.f8_max_run > 0) return false;
+  for (int g = 0; g < 2; ++g)
+    if (!(gps[g].reserved & OMBO_GP_F8C_PLANES)) return false;
+  // model 1's launch must carry the fused acquisition in the bound pass and in the full one
+  const GpDev g1 = gp_dev_view(gps[1]);
+  return ombo_f8_can_fuse(ctx, g1, acq->n_pf, ctx->knobs.prune_depth, s) && ombo_f8_can_fuse(ctx, g1, acq->n_pf, 0, s);
+}
+
+static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, const ombo_acq *acq,
+                        ombo_best *best_dev, cudaStream_t s, bool *done) {
+  *done = false;
+  const long long m = pool->m;
+  const long long cap = ctx->knobs.prune_cap > 0 ? ctx->knobs.prune_cap : std::max(1LL << 16, m / 64);
+  const int out_f32 = pool->X && pool->dtype == 1;
+  const size_t resz = out_f32 ? 4 : 8;
+  auto up = [](size_t b) { return (b + 255) / 256 * 256; };
+  const cub::CountingInputIterator<long long> ids(0);
+  size_t cub_bytes = 0;
+  OMBO_CUDA(cub::DeviceSelect::If(nullptr, cub_bytes, ids, (long long *)nullptr, (long long *)nullptr, m,
+                                  PruneKeep{nullptr, nullptr}, s));
+  const size_t o_ub = up(sizeof(PruneHdr)), o_sel = o_ub + up((size_t)m * 8), o_rows = o_sel + up((size_t)m * 8),
+               o_cub = o_rows + up((size_t)std::min(cap, m) * pool->d * resz);
+  // O(m) workspace: a pool too large for it is scored the unpruned way, in its bounded passes
+  if (ombo_ws_reserve(&ctx->ws_prune, &ctx->ws_prune_bytes, o_cub + cub_bytes)) {
+    (void)cudaGetLastError();                       // the failed allocation is not sticky; clear it
+    return OMBO_OK;
+  }
+  int rc;
+  char *ws = (char *)ctx->ws_prune;
+  PruneHdr *h = (PruneHdr *)ws;
+  double *ub = (double *)(ws + o_ub);
+  long long *sel = (long long *)(ws + o_sel);
+  void *rows = ws + o_rows;
+  k_prune_init<<<1, 1, 0, s>>>(h);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  // bound pass: UB of every candidate and the largest
+  rc = score_passes(ctx, gps, 2, pool, acq, OMBO_PREC_FAST, nullptr, nullptr, ub, &h->ub, s, ctx->knobs.prune_depth);
+  if (rc) return rc;
+  // threshold: the full score of the candidate with the largest bound
+  PoolDev pd;
+  fill_pool_dev(pd, pool);
+  pd.X = pool->X;
+  k_prune_gather<<<1, 32, 0, s>>>(pd, m, nullptr, h, 1, rows, out_f32);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  ombo_pool sub = *pool;
+  sub.X = rows; sub.dtype = out_f32; sub.m = 1; sub.index_base = 0;
+  rc = score_passes(ctx, gps, 2, &sub, acq, OMBO_PREC_FAST, nullptr, nullptr, nullptr, &h->v0, s);
+  if (rc) return rc;
+  // survivors, in ascending index order
+  OMBO_CUDA(cub::DeviceSelect::If(ws + o_cub, cub_bytes, ids, sel, &h->n_sel, m, PruneKeep{ub, h}, s));
+  ctx->launches += 1;
+  PruneHdr hh;
+  OMBO_CUDA(cudaMemcpyAsync(ctx->pinned_best, h, sizeof(PruneHdr), cudaMemcpyDeviceToHost, s));
+  OMBO_CUDA(cudaStreamSynchronize(s));
+  memcpy(&hh, ctx->pinned_best, sizeof(PruneHdr));
+  if (ctx->knobs.prune_log)
+    fprintf(stderr, "[prune] m %lld survivors %lld ub_max %.9g at %lld v0 %.9g cap %lld\n", m, hh.n_sel, hh.ub.value,
+            (long long)hh.ub.index, hh.v0.value, cap);
+  // a threshold at or below zero prunes nothing worth the second pass; too many survivors cost more than they save
+  if (!std::isfinite(hh.ub.value) || !(hh.v0.value - OMBO_PRUNE_TAU * hh.ub.value > 0.0) || hh.n_sel > cap)
+    return OMBO_OK;
+  if (hh.n_sel > 0) {
+    const long long n = hh.n_sel;
+    k_prune_gather<<<(unsigned)((n * pool->d + 255) / 256), 256, 0, s>>>(pd, m, sel, h, n, rows, out_f32);
+    ctx->launches += 1;
+    OMBO_CUDA(cudaGetLastError());
+    sub.m = n;
+    rc = score_passes(ctx, gps, 2, &sub, acq, OMBO_PREC_FAST, nullptr, nullptr, nullptr, &h->loc, s);
+    if (rc) return rc;
+  }
+  k_prune_merge<<<1, 1, 0, s>>>(h, sel, pool->index_base, best_dev);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  *done = true;
   return OMBO_OK;
 }
 
@@ -307,16 +483,12 @@ int ombo_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *poo
   OMBO_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t s = (cudaStream_t)stream;
   if (best_dev) { rc = ombo_best_init(ctx, best_dev, s); if (rc) return rc; }
-  const size_t esz = pool->dtype == 0 ? 8 : 4;
-  const long long chunk = 1LL << ctx->knobs.chunk_log2;
-  for (long long first = 0; first < pool->m; first += chunk) {
-    long long count = pool->m - first < chunk ? pool->m - first : chunk;
-    const void *X = pool->X ? (const char *)pool->X + (size_t)first * pool->d * esz : nullptr;
-    rc = score_pass(ctx, gps, n_gp, pool, X, first, count, acq, precision, out_mu, out_var, out_acq, pool->m,
-                    best_dev, s);
-    if (rc) return rc;
+  if (prune_eligible(ctx, gps, n_gp, pool, acq, precision, out_mu, out_acq, best_dev, s)) {
+    bool done = false;
+    rc = score_pruned(ctx, gps, pool, acq, best_dev, s, &done);
+    if (rc || done) return rc;
   }
-  return OMBO_OK;
+  return score_passes(ctx, gps, n_gp, pool, acq, precision, out_mu, out_var, out_acq, best_dev, s);
 }
 
 int ombo_score_host(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
@@ -484,6 +656,28 @@ int ombo_profile_read(ombo_ctx *ctx, int64_t *n_launches, double *total_ms) {
   *total_ms = tot;
   ctx->prof_count = 0;
   return OMBO_OK;
+}
+
+// test hook (not part of the public header): mu and var of one GP with f8c planes over rows [0, m) of a pool, from
+// the BOUND launch (bound_chunks >= 1: var is the upper bound of the pruned arg-max) or the full one (0), with
+// gen_warps generator warps (8 / 16; 0: the context's choice)
+int ombo_debug_posterior_bound(ombo_ctx *ctx, const ombo_gp *gp, const ombo_pool *pool, int bound_chunks,
+                               int gen_warps, double *mu, double *var, void *stream) {
+  OMBO_CHECK(ctx && gp && gp->state && pool && mu && var, "debug_posterior_bound: NULL argument");
+  OMBO_CHECK(gp->reserved & OMBO_GP_F8C_PLANES, "debug_posterior_bound: the GP has no f8c planes");
+  OMBO_CHECK(gp->d == pool->d && pool->m >= 0, "debug_posterior_bound: bad pool");
+  OMBO_CHECK(bound_chunks >= 0 && bound_chunks <= 2 && (gen_warps == 0 || gen_warps == 8 || gen_warps == 16),
+             "debug_posterior_bound: bound_chunks 0..2, gen_warps 0 / 8 / 16");
+  OMBO_CUDA(cudaSetDevice(ctx->device));
+  PoolDev pd;
+  fill_pool_dev(pd, pool);
+  pd.X = pool->X;
+  const int keep = ctx->knobs.fast_gen_warps;
+  ctx->knobs.fast_gen_warps = gen_warps;
+  const int rc = ombo_posterior_fast(ctx, gp_dev_view(*gp), pd, pool->m, mu, var, true, (cudaStream_t)stream, nullptr,
+                                     nullptr, bound_chunks);
+  ctx->knobs.fast_gen_warps = keep;
+  return rc;
 }
 
 int64_t ombo_launch_count(ombo_ctx *ctx, int reset) {

@@ -47,7 +47,7 @@ struct ombo_knobs {
   int fast_dbg;           // OMBO_FAST_DBG: timing experiments (results are garbage)
   int fast_profile;       // OMBO_FAST_PROFILE: per-CTA wait-cycle counters printed to stderr
   int fast_notrim, fast_nocache, fast_zerocache, fast_mean_in_main;
-  int fast_gen_warps;     // OMBO_FAST_GEN_WARPS: 8 (default) or 16 K1 generator warps in the f8c kernel
+  int fast_gen_warps;     // OMBO_FAST_GEN_WARPS: 8 or 16 K1 generator warps in the f8c kernel (0: 8, bound launches 16)
   int f8_max_run;         // OMBO_F8_MAXRUN: most reload steps in a row between two generated blocks
   double f8_tg;           // OMBO_F8_TG: generator time per K-block in units of one 256-column MMA unit (schedule)
   int chunk_log2;         // OMBO_CHUNK_LOG2: device-pool candidates per pass = 2^chunk_log2
@@ -55,6 +55,10 @@ struct ombo_knobs {
   double f8c_kappa;       // OMBO_F8C_KAPPA: conditioning limit of that format
   int acq_fp64;           // OMBO_ACQ_FP64: keep the FP64 acquisition kernel in fast mode
   int no_fuse;            // OMBO_NO_FUSE: never fuse the 2-D EHVI + arg-max into the f8c kernel's epilogue
+  int no_prune;           // OMBO_NO_PRUNE: score every candidate in full even where a variance bound could skip most
+  int prune_depth;        // OMBO_PRUNE_DEPTH: 256-column chunks of V behind the variance bound (1 or 2)
+  long long prune_cap;    // OMBO_PRUNE_CAP: most survivors scored in full before falling back (0: max(2^16, m / 64))
+  int prune_log;          // OMBO_PRUNE_LOG: one stderr line per pruned call (survivors, bound, threshold)
 };
 
 struct ombo_ctx {
@@ -63,13 +67,14 @@ struct ombo_ctx {
   int64_t launches;
   ombo_knobs knobs;
   long long *prof_dev;    // per-CTA wait counters of the fast kernels (OMBO_FAST_PROFILE)
-  // step schedule of the f8c kernel (posterior_fast8.cu), rebuilt when n_pad changes
-  unsigned int *f8_sched; int f8_sched_np, f8_sched_len, f8_sched_cap;
+  // step schedules of the f8c kernel (posterior_fast8.cu), [0] full, [1] bound; rebuilt when n_pad or the depth changes
+  unsigned int *f8_sched[2]; int f8_sched_np[2], f8_sched_depth[2], f8_sched_len[2], f8_sched_cap[2];
   // workspaces (grown on demand, freed in ctx_destroy)
   void *ws_post;      size_t ws_post_bytes;      // posterior mu/var chunk buffers
   void *ws_scratch;   size_t ws_scratch_bytes;   // FP64 K* tiles (L2 resident) / fast-path scratch
   void *ws_partial;   size_t ws_partial_bytes;   // per-block arg-max partials
   void *ws_box;       size_t ws_box_bytes;       // EHVI_BOX boxes as packed 16-bit breakpoint indices
+  void *ws_prune;     size_t ws_prune_bytes;     // pruned scoring: per-candidate upper bounds, survivors, cub scratch
   void *ws_stage[2];  size_t ws_stage_bytes;     // host-entry H2D staging (double buffered)
   void *ws_best;                                  // 16 B device best for the host entry
   ombo_best *pinned_best;                         // pinned host landing zone
@@ -197,12 +202,16 @@ int ombo_posterior_fp64(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lon
 // fuse_req != NULL asks for the fused 2-D EHVI + arg-max epilogue; *fused reports whether the launch did it (only
 // the f8c kernel can, and only while the stripes fit beside its operand rings) -- if not, mu / var were written
 // and the caller runs K4 as usual
+// bound_chunks >= 1 (f8c planes only): var is the upper bound from the first bound_chunks 256-column chunks of V
+// (posterior_fast8.cu, BOUND schedule), mu and everything else as in a full launch
 int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, long long m,
                         double *mu, double *var, bool want_var, cudaStream_t s,
-                        const FuseAcq *fuse_req = nullptr, int *fused = nullptr);
+                        const FuseAcq *fuse_req = nullptr, int *fused = nullptr, int bound_chunks = 0);
 int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, long long m,
                          double *mu, double *var, cudaStream_t s,
-                         const FuseAcq *fuse_req = nullptr, int *fused = nullptr);
+                         const FuseAcq *fuse_req = nullptr, int *fused = nullptr, int bound_chunks = 0);
+// whether an f8c launch for this GP can carry the fused 2-D EHVI of a front of n_pf points (shared memory)
+bool ombo_f8_can_fuse(ombo_ctx *ctx, const GpDev &gp, int n_pf, int bound_chunks, cudaStream_t s);
 // merges n_partials per-block (value, index) pairs in ctx->ws_partial with the running best
 int ombo_argmax_merge(ombo_ctx *ctx, int n_partials, ombo_best *best_dev, cudaStream_t s);
 int ombo_fast_path_built();

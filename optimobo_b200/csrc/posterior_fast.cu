@@ -826,7 +826,7 @@ static int launch_fast(ombo_ctx *ctx, const CUtensorMap &map_hi, const CUtensorM
 }
 
 int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, long long m, double *mu, double *var,
-                        bool want_var, cudaStream_t s, const FuseAcq *fuse_req, int *fused) {
+                        bool want_var, cudaStream_t s, const FuseAcq *fuse_req, int *fused, int bound_chunks) {
   if (fused) *fused = 0;
   if (m <= 0) return OMBO_OK;
   if (gp.d > 24) {
@@ -865,7 +865,7 @@ int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lon
   // (k_posterior_fast_dc, d <= 12).
   bool pair = false, wide = true, dc = false;
   int cs = 1;
-  if (want_var && (gp.flags & OMBO_GP_F8C_PLANES)) return ombo_posterior_fast8(ctx, gp, pool, m, mu, var, s, fuse_req, fused);
+  if (want_var && (gp.flags & OMBO_GP_F8C_PLANES)) return ombo_posterior_fast8(ctx, gp, pool, m, mu, var, s, fuse_req, fused, bound_chunks);
   { const int mode = kn.fast_mode ? kn.fast_mode : 3;
     if (mode == 1) wide = false;
     else if (mode == 2) { wide = false; pair = true; }

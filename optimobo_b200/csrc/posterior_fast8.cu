@@ -116,12 +116,16 @@ __device__ __forceinline__ void sts64_at(uint32_t a, uint32_t x, uint32_t y) {
 #define SW_CHUNK(w, slot) ((int)(((w) >> (10 + 6 * (slot))) & 63u) - 1)   // chunk in TMEM slot 0 / 1, -1 = none
 #define SW_FIRST(w, slot) (((w) >> (22 + (slot))) & 1u)          // first block of that chunk (accumulator reset)
 #define SW_DONE(w, slot) (((w) >> (24 + (slot))) & 1u)           // last block of that chunk (epilogue may drain)
+#define SW_MEAN(w) (((w) >> 26) & 1u)                            // bound schedule: fresh block that feeds the mean only
 
 struct F8Maps {            // tensor maps of the three B planes (128-row and 32-row boxes) and of the K* cache
   CUtensorMap hi128, hi32, c1_128, c1_32, c2_128, c2_32, kc;
 };
 
-template <int DP, int R, int GW, bool MATERN>
+// BOUND: the kernel walks a bound schedule (f8_build_schedule, bound_chunks > 0).  Its MEAN steps generate k' and the
+// mean exactly as a full launch does and multiply nothing, so mu is the full launch's and var is the upper bound
+// sigma_f2 - (the first chunks' sum of V^2) >= var.  A separate instantiation: the full kernel carries no mean-step code.
+template <int DP, int R, int GW, bool MATERN, bool BOUND>
 __global__ void __launch_bounds__((8 + GW) * 32, 1)
 k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
   constexpr int NSTA = 3, NSTB = 3;
@@ -258,6 +262,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
         for (int si = 0; si < n_steps; ++si) {
           const uint32_t w = sched[si];
           const int kb = SW_KB(w);
+          if (BOUND && SW_MEAN(w)) continue;                // nothing to multiply, no stage
           F8_TRACE(1, 0x80 | (kb & 31));
           mbar_wait_prof(smem_u32(&a_full[sa]), pa, MMA_SLEEP_NS, w_afull, pon);
           F8_TRACE(1, 0xC0 | (kb & 31));
@@ -368,6 +373,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
         for (int si = 0; si < n_steps; ++si) {
           const uint32_t w = sched[si];
           const int kb = SW_KB(w);
+          if (BOUND && SW_MEAN(w)) { slice_next(); continue; }   // the block's slice only, no stage
           const uint32_t stage = smem_u32(sA + sa * STAGE_BYTES);
           if (SW_FRESH(w)) {
             slice_next();
@@ -539,6 +545,67 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&xc_empty[b]));                   // xc[b] may be refilled
+      // the K1 math of one K-block, shared by the full and the mean-only steps (the same operations in the same order,
+      // so both see the same k' and accumulate the same mean): squared distances of this lane's rows to the block's
+      // eight training points of column group g, k'(r) of one row, and that row's share of the mean
+      auto dist2 = [&](const float *xs, float2 (&r2)[ROWS][4]) {
+        {
+          const float4 n0 = *(const float4 *)(xs + (DP + 1) * FK);      // |b_i|^2
+          const float4 n1 = *(const float4 *)(xs + (DP + 1) * FK + 4);
+#pragma unroll
+          for (int rr = 0; rr < ROWS; ++rr) {
+            const float2 aa = make_float2(a2[rr], a2[rr]);
+            r2[rr][0] = __fadd2_rn(aa, make_float2(n0.x, n0.y));
+            r2[rr][1] = __fadd2_rn(aa, make_float2(n0.z, n0.w));
+            r2[rr][2] = __fadd2_rn(aa, make_float2(n1.x, n1.y));
+            r2[rr][3] = __fadd2_rn(aa, make_float2(n1.z, n1.w));
+          }
+        }
+#pragma unroll
+        for (int j = 0; j < DP; ++j) {
+          const float4 t0 = *(const float4 *)(xs + j * FK);
+          const float4 t1 = *(const float4 *)(xs + j * FK + 4);
+#pragma unroll
+          for (int rr = 0; rr < ROWS; ++rr) {
+            const float2 xx = make_float2(x[rr][j], x[rr][j]);            // -2 a_j
+            r2[rr][0] = __ffma2_rn(xx, make_float2(t0.x, t0.y), r2[rr][0]);
+            r2[rr][1] = __ffma2_rn(xx, make_float2(t0.z, t0.w), r2[rr][1]);
+            r2[rr][2] = __ffma2_rn(xx, make_float2(t1.x, t1.y), r2[rr][2]);
+            r2[rr][3] = __ffma2_rn(xx, make_float2(t1.z, t1.w), r2[rr][3]);
+          }
+        }
+      };
+      auto kval = [&](const float2 (&r2r)[4], float2 (&kv)[4]) {
+        if (MATERN) {
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            float2 rad, ex;
+            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad.x) : "f"(fabsf(r2r[e].x)));
+            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad.y) : "f"(fabsf(r2r[e].y)));
+            const float2 arg = __fmul2_rn(rad, make_float2(-3.2259955597f, -3.2259955597f));   // -sqrt5 log2(e)
+            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ex.x) : "f"(arg.x));
+            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ex.y) : "f"(arg.y));
+            const float2 poly = __ffma2_rn(rad, make_float2(2.2360679775f, 2.2360679775f),
+                                           __ffma2_rn(r2r[e], make_float2(1.6666666667f, 1.6666666667f),
+                                                      make_float2(1.0f, 1.0f)));
+            kv[e] = __fmul2_rn(poly, ex);
+          }
+        } else {
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float2 arg = __fmul2_rn(r2r[e], make_float2(-0.7213475204f, -0.7213475204f));  // -0.5 log2(e)
+            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(kv[e].x) : "f"(arg.x));
+            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(kv[e].y) : "f"(arg.y));
+          }
+        }
+      };
+      auto mean_add = [&](const float2 (&kv)[4], const float4 al0, const float4 al1, float &acc) {
+        float2 m2 = __fmul2_rn(kv[0], make_float2(al0.x, al0.y));
+        m2 = __ffma2_rn(kv[1], make_float2(al0.z, al0.w), m2);
+        m2 = __ffma2_rn(kv[2], make_float2(al1.x, al1.y), m2);
+        m2 = __ffma2_rn(kv[3], make_float2(al1.z, al1.w), m2);
+        acc += m2.x + m2.y;
+      };
       {
         for (int si = 0; si < n_steps; ++si) {
           const uint32_t w = sched[si];
@@ -551,6 +618,25 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
             if (++sa == NSTA) { sa = 0; pa ^= 1; }
             continue;
           }
+          if (BOUND && SW_MEAN(w)) {
+            // a block beyond the bound: k' and the mean only -- no operands, no stage, only the slice to release
+            if (!solo) mbar_wait_sleep(s_full_u + sl * 8, slph, 20);
+            const float *xs = xt + sl * XT_STRIDE + 8 * g;
+            float2 r2[ROWS][4];
+            dist2(xs, r2);
+            const float4 al0 = *(const float4 *)(xs + DP * FK);
+            const float4 al1 = *(const float4 *)(xs + DP * FK + 4);
+#pragma unroll
+            for (int rr = 0; rr < ROWS; ++rr) {
+              float2 kv[4];
+              kval(r2[rr], kv);
+              mean_add(kv, al0, al1, mu_acc[rr]);
+            }
+            __syncwarp();
+            if (lane == 0 && !solo) mbar_arrive(s_empty_u + sl * 8);
+            if (++sl == NSL) { sl = 0; slph ^= 1; }
+            continue;
+          }
           F8_TRACE_G(kb);
           if (!solo) mbar_wait_sleep(s_full_u + sl * 8, slph, 20);            // this block's train slice has landed
           F8_TRACE_G(0x40 | kb);
@@ -559,31 +645,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
           const uint32_t st_hi = st_u + off_hi0, st_c8 = st_u + off_c80;
           if (!(prm.dbg & 2)) {
             float2 r2[ROWS][4];
-            {
-              const float4 n0 = *(const float4 *)(xs + (DP + 1) * FK);      // |b_i|^2
-              const float4 n1 = *(const float4 *)(xs + (DP + 1) * FK + 4);
-#pragma unroll
-              for (int rr = 0; rr < ROWS; ++rr) {
-                const float2 aa = make_float2(a2[rr], a2[rr]);
-                r2[rr][0] = __fadd2_rn(aa, make_float2(n0.x, n0.y));
-                r2[rr][1] = __fadd2_rn(aa, make_float2(n0.z, n0.w));
-                r2[rr][2] = __fadd2_rn(aa, make_float2(n1.x, n1.y));
-                r2[rr][3] = __fadd2_rn(aa, make_float2(n1.z, n1.w));
-              }
-            }
-#pragma unroll
-            for (int j = 0; j < DP; ++j) {
-              const float4 t0 = *(const float4 *)(xs + j * FK);
-              const float4 t1 = *(const float4 *)(xs + j * FK + 4);
-#pragma unroll
-              for (int rr = 0; rr < ROWS; ++rr) {
-                const float2 xx = make_float2(x[rr][j], x[rr][j]);            // -2 a_j
-                r2[rr][0] = __ffma2_rn(xx, make_float2(t0.x, t0.y), r2[rr][0]);
-                r2[rr][1] = __ffma2_rn(xx, make_float2(t0.z, t0.w), r2[rr][1]);
-                r2[rr][2] = __ffma2_rn(xx, make_float2(t1.x, t1.y), r2[rr][2]);
-                r2[rr][3] = __ffma2_rn(xx, make_float2(t1.z, t1.w), r2[rr][3]);
-              }
-            }
+            dist2(xs, r2);
             const float4 al0 = *(const float4 *)(xs + DP * FK);
             const float4 al1 = *(const float4 *)(xs + DP * FK + 4);
             F8_TRACE_G(0x80 | kb);
@@ -592,35 +654,8 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
 #pragma unroll
             for (int rr = 0; rr < ROWS; ++rr) {
               float2 kv[4];
-              if (MATERN) {
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  float2 rad, ex;
-                  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad.x) : "f"(fabsf(r2[rr][e].x)));
-                  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad.y) : "f"(fabsf(r2[rr][e].y)));
-                  const float2 arg = __fmul2_rn(rad, make_float2(-3.2259955597f, -3.2259955597f));   // -sqrt5 log2(e)
-                  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ex.x) : "f"(arg.x));
-                  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ex.y) : "f"(arg.y));
-                  const float2 poly = __ffma2_rn(rad, make_float2(2.2360679775f, 2.2360679775f),
-                                                 __ffma2_rn(r2[rr][e], make_float2(1.6666666667f, 1.6666666667f),
-                                                            make_float2(1.0f, 1.0f)));
-                  kv[e] = __fmul2_rn(poly, ex);
-                }
-              } else {
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  const float2 arg = __fmul2_rn(r2[rr][e], make_float2(-0.7213475204f, -0.7213475204f));  // -0.5 log2(e)
-                  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(kv[e].x) : "f"(arg.x));
-                  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(kv[e].y) : "f"(arg.y));
-                }
-              }
-              {
-                float2 m2 = __fmul2_rn(kv[0], make_float2(al0.x, al0.y));
-                m2 = __ffma2_rn(kv[1], make_float2(al0.z, al0.w), m2);
-                m2 = __ffma2_rn(kv[2], make_float2(al1.x, al1.y), m2);
-                m2 = __ffma2_rn(kv[3], make_float2(al1.z, al1.w), m2);
-                mu_acc[rr] += m2.x + m2.y;
-              }
+              kval(r2[rr], kv);
+              mean_add(kv, al0, al1, mu_acc[rr]);
               uint32_t hi[4];
               uint32_t c1[2], c2[2];
 #pragma unroll
@@ -689,15 +724,35 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
 
 // ---- host side ------------------------------------------------------------------------------
 // Step schedule of one tile (see the header).  max_run <= 0: the PASS schedule (default, below).  max_run >= 1: the
-// ROLLING schedule (OMBO_F8_MAXRUN, experimental).  The generators deliver block f = 0 .. nkb-1 in order, one per `tg`
+// ROLLING schedule (OMBO_F8_MAXRUN, experimental).  bound_chunks >= 1: the BOUND schedule of the pass schedule (below).  The generators deliver block f = 0 .. nkb-1 in order, one per `tg`
 // units of MMA time (unit = one 256-column chunk x one 64-deep K-block x the three products).  Two TMEM slots; a
 // chunk opens in the slot that frees, with the already generated blocks it needs queued as reloads.  Reloads are
 // issued (a) when a chunk needs no further fresh block and only its queue keeps its slot busy, (b) in the MMA time
 // a fresh step leaves over (tg - its units, at most one unit banked; never more than max_run in a row), (c) at the end.  A reload that both open
 // chunks still need serves both (one stage fill, two units).
-void f8_build_schedule(int np, double tg, int max_run, std::vector<unsigned int> &steps) {
+void f8_build_schedule(int np, double tg, int max_run, std::vector<unsigned int> &steps, int bound_chunks) {
   const int nkb = np / FK, n_chunks = (np + 255) / 256;
   auto last_kb = [&](int c) { return std::min(4 * c + 3, nkb - 1); };
+  if (bound_chunks > 0) {
+    // BOUND schedule: chunks 0 .. bound_chunks - 1 (1 = chunk 0, 2 = both chunks of pass 0) take exactly the steps,
+    // N-shrink and order of the pass schedule, so their accumulators -- and the epilogue's partial sums of V^2 --
+    // are bit-identical to a full launch's.  The K-blocks beyond them are generated for the mean only (MEAN steps:
+    // fresh, no chunk).  Nothing is reloaded, so nothing is stored.
+    std::vector<unsigned int> full;
+    f8_build_schedule(np, tg, 0, full, 0);
+    const int nb = std::min(nkb, 4 * bound_chunks);
+    steps.clear();
+    for (unsigned int w : full) {
+      if (!((w >> 8) & 1u) || (int)(w & 0xFFu) >= nb) continue;      // pass 0 generates blocks 0 .. 7 in order
+      w &= ~(1u << 9);
+      for (int sl = 0; sl < 2; ++sl)
+        if ((int)((w >> (10 + 6 * sl)) & 63u) - 1 >= bound_chunks)
+          w &= ~((63u << (10 + 6 * sl)) | (1u << (22 + sl)) | (1u << (24 + sl)));
+      steps.push_back(w);
+    }
+    for (int kb = nb; kb < nkb; ++kb) steps.push_back((unsigned int)kb | (1u << 8) | (1u << 26));
+    return;
+  }
   if (max_run <= 0) {
     // PASS schedule (the default, measured faster on the three-stage A ring -- DESIGN.md section 4): chunks 2p and
     // 2p+1 share pass p; the blocks earlier passes generated come back as reloads that serve BOTH chunks (two units
@@ -808,7 +863,13 @@ void f8_build_schedule(int np, double tg, int max_run, std::vector<unsigned int>
 // debug / test hook (not part of the public header): the schedule for n_pad as the kernel will walk it
 extern "C" int ombo_debug_f8_schedule(int n_pad, double tg, int max_run, unsigned int *out, int cap) {
   std::vector<unsigned int> steps;
-  f8_build_schedule(n_pad, tg, max_run, steps);
+  f8_build_schedule(n_pad, tg, max_run, steps, 0);
+  for (int i = 0; i < (int)steps.size() && i < cap; ++i) out[i] = steps[i];
+  return (int)steps.size();
+}
+extern "C" int ombo_debug_f8_bound_schedule(int n_pad, int bound_chunks, unsigned int *out, int cap) {
+  std::vector<unsigned int> steps;
+  f8_build_schedule(n_pad, 3.0, 0, steps, bound_chunks < 1 ? 1 : bound_chunks);
   for (int i = 0; i < (int)steps.size() && i < cap; ++i) out[i] = steps[i];
   return (int)steps.size();
 }
@@ -835,14 +896,14 @@ static size_t f8_smem_base(int DP) {
          34 * 8 + 16 * 8 + 128 * 4 + 16 + 2 * 8 + 8 * 8 + 1024;
 }
 
-template <int DP, int R, int GW, bool MATERN>
+template <int DP, int R, int GW, bool MATERN, bool BOUND>
 static int launch_fast8(ombo_ctx *ctx, const F8Maps &maps, FastParams prm, int grid, cudaStream_t s) {
   // the fused stripes first, then the schedule if it still fits (the same order as the can-fuse test of the caller)
   size_t smem = f8_smem_base(DP) + (prm.fuse.on ? (size_t)2 * (prm.fuse.n_pf + 2) * 4 : 0);
   prm.sched_in_smem = smem + (size_t)prm.n_steps * 4 <= 227 * 1024 ? 1 : 0;
   if (prm.sched_in_smem) smem += (size_t)prm.n_steps * 4;
   // per device, not per process: the attribute belongs to the (function, device) pair
-  OMBO_CUDA(cudaFuncSetAttribute(k_posterior_fast8<DP, R, GW, MATERN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  OMBO_CUDA(cudaFuncSetAttribute(k_posterior_fast8<DP, R, GW, MATERN, BOUND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ProfScope prof(ctx, s);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
@@ -854,13 +915,46 @@ static int launch_fast8(ombo_ctx *ctx, const F8Maps &maps, FastParams prm, int g
   at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  OMBO_CUDA(cudaLaunchKernelEx(&cfg, k_posterior_fast8<DP, R, GW, MATERN>, maps, prm));
+  OMBO_CUDA(cudaLaunchKernelEx(&cfg, k_posterior_fast8<DP, R, GW, MATERN, BOUND>, maps, prm));
   return OMBO_OK;
+}
+
+// the step schedule of a tile for n_pad (full, or bound with bound_chunks chunks), built and uploaded once
+static int f8_schedule(ombo_ctx *ctx, int n_pad, int bound_chunks, cudaStream_t s) {
+  const int k = bound_chunks > 0 ? 1 : 0;
+  if (ctx->f8_sched_np[k] == n_pad && ctx->f8_sched_depth[k] == bound_chunks) return OMBO_OK;
+  std::vector<unsigned int> steps;
+  f8_build_schedule(n_pad, ctx->knobs.f8_tg, ctx->knobs.f8_max_run, steps, bound_chunks);
+  if ((int)steps.size() > ctx->f8_sched_cap[k]) {
+    if (ctx->f8_sched[k]) OMBO_CUDA(cudaFree(ctx->f8_sched[k]));
+    ctx->f8_sched[k] = nullptr;
+    OMBO_CUDA(cudaMalloc(&ctx->f8_sched[k], steps.size() * sizeof(unsigned int)));
+    ctx->f8_sched_cap[k] = (int)steps.size();
+  }
+  OMBO_CUDA(cudaStreamSynchronize(s));            // a launch in flight may still read the old table
+  OMBO_CUDA(cudaMemcpy(ctx->f8_sched[k], steps.data(), steps.size() * sizeof(unsigned int), cudaMemcpyHostToDevice));
+  ctx->f8_sched_np[k] = n_pad;
+  ctx->f8_sched_depth[k] = bound_chunks;
+  ctx->f8_sched_len[k] = (int)steps.size();
+  return OMBO_OK;
+}
+
+// shared memory of a fused launch: the stripes must fit beside the operand rings (the schedule may stay in global memory)
+static bool f8_fuse_fits(const GpDev &gp, int n_pf, int n_steps) {
+  const int dp = gp.d <= 2 ? 2 : (gp.d + 1) / 2 * 2;
+  size_t need = f8_smem_base(dp) + (size_t)2 * (n_pf + 2) * 4;
+  if (need + (size_t)n_steps * 4 <= 227 * 1024) need += (size_t)n_steps * 4;
+  return need <= 227 * 1024;
+}
+
+bool ombo_f8_can_fuse(ombo_ctx *ctx, const GpDev &gp, int n_pf, int bound_chunks, cudaStream_t s) {
+  if (f8_schedule(ctx, gp.n_pad, bound_chunks, s)) return false;
+  return f8_fuse_fits(gp, n_pf, ctx->f8_sched_len[bound_chunks > 0 ? 1 : 0]);
 }
 
 // mu / var of one GP whose planes are in the f8c format (gp.flags & OMBO_GP_F8C_PLANES), d <= 12
 int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, long long m, double *mu, double *var,
-                         cudaStream_t s, const FuseAcq *fuse_req, int *fused) {
+                         cudaStream_t s, const FuseAcq *fuse_req, int *fused, int bound_chunks) {
   if (fused) *fused = 0;
   const long long tiles = (m + FM - 1) / FM;
   F8Maps maps;
@@ -890,29 +984,15 @@ int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lo
   int grid = (int)(tiles < ctx->num_sms ? tiles : ctx->num_sms);
   grid = (grid + 1) / 2 * 2;                    // whole pairs; a surplus CTA runs a dummy tile
   if (grid > ctx->num_sms) grid = ctx->num_sms / 2 * 2;
-  if (ctx->f8_sched_np != gp.n_pad) {              // step schedule of a tile: a function of n_pad (and the knob) only
-    std::vector<unsigned int> steps;
-    f8_build_schedule(gp.n_pad, ctx->knobs.f8_tg, ctx->knobs.f8_max_run, steps);
-    if ((int)steps.size() > ctx->f8_sched_cap) {
-      if (ctx->f8_sched) OMBO_CUDA(cudaFree(ctx->f8_sched));
-      ctx->f8_sched = nullptr;
-      OMBO_CUDA(cudaMalloc(&ctx->f8_sched, steps.size() * sizeof(unsigned int)));
-      ctx->f8_sched_cap = (int)steps.size();
-    }
-    OMBO_CUDA(cudaStreamSynchronize(s));            // a launch in flight may still read the old table
-    OMBO_CUDA(cudaMemcpy(ctx->f8_sched, steps.data(), steps.size() * sizeof(unsigned int), cudaMemcpyHostToDevice));
-    ctx->f8_sched_np = gp.n_pad;
-    ctx->f8_sched_len = (int)steps.size();
-  }
-  prm.sched = ctx->f8_sched;
-  prm.n_steps = ctx->f8_sched_len;
+  // step schedule of a tile: a function of n_pad, the bound depth (and the knobs) only
+  const int sk = bound_chunks > 0 ? 1 : 0;
+  if ((rc = f8_schedule(ctx, gp.n_pad, bound_chunks, s))) return rc;
+  prm.sched = ctx->f8_sched[sk];
+  prm.n_steps = ctx->f8_sched_len[sk];
   prm.fuse.on = 0;
   if (fuse_req) {
     // fused 2-D EHVI + arg-max: only while the stripes fit beside everything else in shared memory
-    const int dp = gp.d <= 2 ? 2 : (gp.d + 1) / 2 * 2;
-    size_t need = f8_smem_base(dp) + (size_t)2 * (fuse_req->n_pf + 2) * 4;
-    if (need + (size_t)prm.n_steps * 4 <= 227 * 1024) need += (size_t)prm.n_steps * 4;
-    if (need <= 227 * 1024) {
+    if (f8_fuse_fits(gp, fuse_req->n_pf, prm.n_steps)) {
       rc = ombo_ws_reserve(&ctx->ws_partial, &ctx->ws_partial_bytes, (size_t)grid * sizeof(ombo_best));
       if (rc) return rc;
       prm.fuse = *fuse_req;
@@ -921,7 +1001,7 @@ int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lo
       if (fused) *fused = grid;
     }
   }
-  if (gp.n_pad > 512) {                          // more than two chunks: generated K* blocks are cached in L2 for later chunks
+  if (gp.n_pad > 512 && !bound_chunks) {         // more than two chunks: generated K* blocks are cached in L2 for later chunks
     rc = ombo_ws_reserve(&ctx->ws_scratch, &ctx->ws_scratch_bytes, (size_t)grid * (gp.n_pad / FK) * STAGE_BYTES);
     if (rc) return rc;
     prm.kcache = (unsigned char *)ctx->ws_scratch;
@@ -929,11 +1009,16 @@ int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lo
     if (rc) return rc;
   }
   const int d = gp.d;
-  const bool gw16 = ctx->knobs.fast_gen_warps == 16;
+  // the bound schedule leaves the generators alone on the critical path, below the power cap: 16 warps (measured,
+  // DESIGN.md section 4); the full schedule keeps 8 unless OMBO_FAST_GEN_WARPS says otherwise
+  const int gw_knob = ctx->knobs.fast_gen_warps;
+  const bool gw16 = gw_knob ? gw_knob == 16 : bound_chunks > 0;
   const bool mat = gp.kernel == OMBO_KERNEL_MATERN52;
-#define F8_DISPATCH(DPV)                                                                     \
-  rc = gw16 ? (mat ? launch_fast8<DPV, 2, 16, true>(ctx, maps, prm, grid, s) : launch_fast8<DPV, 2, 16, false>(ctx, maps, prm, grid, s)) \
-            : (mat ? launch_fast8<DPV, 4, 8, true>(ctx, maps, prm, grid, s) : launch_fast8<DPV, 4, 8, false>(ctx, maps, prm, grid, s))
+#define F8_LAUNCH(DPV, RV, GWV, BV)                                                                                  \
+  (mat ? launch_fast8<DPV, RV, GWV, true, BV>(ctx, maps, prm, grid, s) : launch_fast8<DPV, RV, GWV, false, BV>(ctx, maps, prm, grid, s))
+#define F8_DISPATCH(DPV)                                                                                             \
+  rc = bound_chunks ? (gw16 ? F8_LAUNCH(DPV, 2, 16, true) : F8_LAUNCH(DPV, 4, 8, true))                               \
+                    : (gw16 ? F8_LAUNCH(DPV, 2, 16, false) : F8_LAUNCH(DPV, 4, 8, false))
   if (d <= 2) { F8_DISPATCH(2); }
   else if (d <= 4) { F8_DISPATCH(4); }
   else if (d <= 6) { F8_DISPATCH(6); }
@@ -941,6 +1026,7 @@ int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lo
   else if (d <= 10) { F8_DISPATCH(10); }
   else { F8_DISPATCH(12); }
 #undef F8_DISPATCH
+#undef F8_LAUNCH
   if (rc) return rc;
   ctx->launches += 1;
   OMBO_CUDA(cudaGetLastError());

@@ -66,6 +66,21 @@ def ehvi_stripes(PF, ref_point):
     return np.stack([y1, y2])
 
 
+def front_is_staircase(PF, ref_point):
+    """True when the 2-objective front is a valid staircase for the stripes of ehvi_stripes: finite, inside the
+    reference point and mutually non-dominated without duplicates (sorted by objective 2, objective 1 strictly
+    decreases while objective 2 strictly increases).  Over such a front the exact EHVI never decreases in either
+    sigma, which is what lets ombo_score prune candidates by a variance bound."""
+    PF = np.atleast_2d(np.asarray(PF, dtype=np.float64))
+    r = np.asarray(ref_point, dtype=np.float64).reshape(-1)
+    if PF.shape[1] != 2 or len(PF) == 0 or r.shape != (2,) or not np.all(np.isfinite(PF)) or not np.all(np.isfinite(r)):
+        return False
+    if not np.all(PF <= r):
+        return False
+    S = PF[np.argsort(PF[:, 1], kind="stable")]
+    return bool(np.all(np.diff(S[:, 0]) < 0) and np.all(np.diff(S[:, 1]) > 0))
+
+
 def ehvi_boxes(PF, ref_point):
     """Disjoint boxes tiling {z <= r : no front point dominates z} (minimisation), for the exact EHVI of
     2 <= k <= 4 objectives.  Points not <= r are dropped and the first front is taken; the region is sliced on the
