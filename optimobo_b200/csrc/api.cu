@@ -67,14 +67,8 @@ int ombo_ctx_create(int device, ombo_ctx **out) {
   {   // environment knobs: read here, once, never on the launch path
     auto geti = [](const char *name, int dflt) { const char *e = getenv(name); return e ? atoi(e) : dflt; };
     ombo_knobs &k = c->knobs;
-    k.fast_mode = geti("OMBO_FAST_MODE", 0);
-    k.fast_cluster = geti("OMBO_FAST_CLUSTER", 1);
     k.fast_dbg = geti("OMBO_FAST_DBG", 0);
     k.fast_profile = geti("OMBO_FAST_PROFILE", 0);
-    k.fast_notrim = getenv("OMBO_FAST_NOTRIM") != nullptr;
-    k.fast_nocache = getenv("OMBO_FAST_NOCACHE") != nullptr;
-    k.fast_zerocache = getenv("OMBO_FAST_ZEROCACHE") != nullptr;
-    k.fast_mean_in_main = getenv("OMBO_FAST_MEAN_IN_MAIN") != nullptr;
     k.fast_gen_warps = geti("OMBO_FAST_GEN_WARPS", 0);
     k.f8_max_run = geti("OMBO_F8_MAXRUN", 0);
     { const char *e = getenv("OMBO_F8_TG"); k.f8_tg = e ? atof(e) : 3.0; }

@@ -42,11 +42,8 @@ void ombo_set_error(const char *fmt, ...);
 
 // environment knobs, read ONCE when the context is created (never on the launch path)
 struct ombo_knobs {
-  int fast_mode;          // OMBO_FAST_MODE: 0 = default; 1 / 2 / 4 = experimental variants of the 16-bit x3 kernels
-  int fast_cluster;       // OMBO_FAST_CLUSTER (mode 1 only)
   int fast_dbg;           // OMBO_FAST_DBG: timing experiments (results are garbage)
   int fast_profile;       // OMBO_FAST_PROFILE: per-CTA wait-cycle counters printed to stderr
-  int fast_notrim, fast_nocache, fast_zerocache, fast_mean_in_main;
   int fast_gen_warps;     // OMBO_FAST_GEN_WARPS: 8 or 16 K1 generator warps in the f8c kernel (0: 8, bound launches 16)
   int f8_max_run;         // OMBO_F8_MAXRUN: most reload steps in a row between two generated blocks
   double f8_tg;           // OMBO_F8_TG: generator time per K-block in units of one 256-column MMA unit (schedule)

@@ -7,9 +7,10 @@
 //   V ~= A_hi B_hi^T + A_lo B_hi^T + A_hi B_lo^T      (three kind::f16 MMAs, FP32 accumulate in TMEM)
 //   var = sigma_f2 - sum_j V_j^2 (V = L^-1 k*),  mu = sum_i k'_i (sigma_f2 alpha_i) on the CUDA cores.
 //
-// One persistent CTA per SM owns a tile of 128 candidates (UMMA M = 128, cta_group::1).  Default variant
-// (MODE 2, 256-column accumulator chunks):
-//   warp 0      TMA producer: 256x64 bf16 planes of B (SWIZZLE_128B), hi then lo, into a 3-entry ring
+// One persistent CTA per SM owns a tile of 128 candidates (UMMA M = 128, cta_group::1), 256-column accumulator chunks:
+//   warp 0      TMA producer: 256x64 16-bit planes of B (SWIZZLE_128B) into a 3-entry ring, one plane per entry
+//               (hi, then lo: the lo plane of a unit can still be in flight while its hi plane is multiplied);
+//               on the diagonal K-blocks only the rows of the band are fetched
 //   warp 1      MMA issuer (one elected lane): 12 tcgen05.mma (4 k-steps x 3 products) per (chunk, K-block),
 //               N shrinking 256/192/128/64 on the diagonal K-blocks
 //   warp 2      TMEM allocator (512 columns = 2 accumulator chunks of 256 columns)
@@ -23,54 +24,39 @@
 // load in the later passes: every K* block is generated exactly once per tile.
 // Within a pass the loop is K-outer, so a chunk's accumulator completes as soon as the K loop crosses
 // its diagonal and the epilogue drains it while the tensor core continues on the later chunks.
-// PTX wrappers and the parameter block: umma.cuh.  Decoupled cta_group::2 variant: posterior_fast_dc.cu.
+// The UMMA runs at its N/2-cycle floor (scripts/umma_bench.cu); what limits this kernel is shared-memory traffic
+// per MAC (the A tile is re-read by every MMA: 32 B/clk at N = 256, on top of 64 B/clk of B reads and the TMA / K1
+// writes) and, at the power cap, issued work -- hence 256-column chunks on one CTA, with N shrinking on the diagonal
+// (a cta_group::2 pair halves the B traffic but cannot shrink N and was slower at the cap: DESIGN.md section 4).
+// PTX wrappers and the parameter block: umma.cuh.
 #include "umma.cuh"
 
 
-// DP   = input dimension padded to the instantiated size (padding coordinates are zero on both sides)
-// R    = candidate rows held in registers per generator thread (4 when DP <= 12, else 2)
-// PAIR = cta_group::2: two CTAs of a cluster form one UMMA M = 256 x N = 256 tile pair.  Each CTA generates
-//        the K* rows of its own 128 candidates and TMA-loads only ITS half of the B tile; the leader CTA
-//        issues the MMAs for both tensor cores.  Per MAC this halves the B traffic through shared memory.
-// The UMMA itself runs at its N/2-cycle floor in every mode (scripts/umma_bench.cu); what separates the
-// modes is shared-memory traffic per MAC (the A tile is re-read by every MMA: 64 B/clk at N = 128, 32 B/clk
-// at N = 256, on top of 64 B/clk of B reads and the TMA / K1 writes) and, at the power cap, issued work.
-// MODE = 0: single CTA, 128-column chunks
-//        1: cta_group::2 pair (see above; N cannot shrink on the diagonal K-blocks)
-//        2: single CTA, 256-column chunks (half the A re-reads per MAC; the diagonal K-blocks shrink N to
-//           192 / 128 / 64), B ring entries are single planes so the lo plane of a unit can still be in
-//           flight while its hi plane is being multiplied -- the default
-template <int DP, int R, int MODE, int GW, bool F16>
-__global__ void __launch_bounds__((8 + GW) * 32, 1)
+// DP  = input dimension padded to the instantiated size (padding coordinates are zero on both sides)
+// R   = candidate rows held in registers per generator thread (4 when DP <= 12, else 2)
+// F16 = fp16 planes (ill-conditioned GP): fp16 hi/lo split of K* and direct distances
+template <int DP, int R, bool F16>
+__global__ void __launch_bounds__(16 * 32, 1)
 k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo,
                  const __grid_constant__ CUtensorMap map_kc, const FastParams prm) {
-  constexpr bool PAIR = (MODE == 1), WIDE = (MODE == 2);
-#ifndef WIDE_NSTA
-#define WIDE_NSTA 3
-#endif
-  constexpr int NSTA = WIDE ? WIDE_NSTA : 3, NSTB = 6 - NSTA;  // ring depths (32 KB entries, 192 KB in all modes)
-  constexpr int GEN_WARPS = GW, GEN_THREADS = GW * 32;
-  constexpr int CW = (PAIR || WIDE) ? 256 : 128; // accumulator chunk width = widest UMMA N
+  constexpr int NSTA = 3, NSTB = 3;               // ring depths (32 KB entries, 192 KB in all)
+  constexpr int GEN_WARPS = 8, GEN_THREADS = GEN_WARPS * 32;
+  constexpr int CW = 256;                        // accumulator chunk width = widest UMMA N
   constexpr int NSLOT = 512 / CW;                // TMEM accumulator slots
-  constexpr int KSH = (PAIR || WIDE) ? 2 : 1;    // chunk c needs K-blocks kb < (c + 1) << KSH
-  constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(CW >> 3) << 17) |
-                             ((uint32_t)((PAIR ? 256 : 128) >> 4) << 24);
+  constexpr int KSH = 2;                         // chunk c needs K-blocks kb < (c + 1) << KSH
+  constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(CW >> 3) << 17) | ((uint32_t)(FM >> 4) << 24);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int d = prm.gp.d, np = prm.gp.n_pad;
   const int nkb = np / FK;
   const int n_chunks = (np + CW - 1) / CW;
   const int n_pass = (n_chunks + NSLOT - 1) / NSLOT;
   const long long n_tiles = (prm.m + FM - 1) / FM;
-  // every CTA of a cluster walks the same (tile, chunk, K-block) sequence
   const long long n_iter = (n_tiles + gridDim.x - 1) / gridDim.x;
-  const uint32_t cs = cluster_size(), crank = cluster_rank();
-  const uint16_t cmask = (uint16_t)((1u << cs) - 1u);
-  const bool leader = !PAIR || crank == 0;
   auto last_kb = [&](int c) { return min(((c + 1) << KSH) - 1, nkb - 1); };
 
-  // ---- shared memory carve-up (identical in every CTA: the pair's UMMA descriptors rely on it) ----
+  // ---- shared memory carve-up ----
   unsigned char *sA = fast_smem + ((1024u - (smem_u32(fast_smem) & 1023u)) & 1023u);   // SWIZZLE_128B: 1024-B aligned
-  unsigned char *sB = sA + NSTA * STAGE_BYTES;                 // NSTB x (hi 16 KB, lo 16 KB)
+  unsigned char *sB = sA + NSTA * STAGE_BYTES;                 // NSTB x one plane of a 256-row B tile (32 KB)
   float *xc = (float *)(sB + NSTB * STAGE_BYTES);              // [DP][128] scaled candidate coords
   float *xt = xc + (size_t)DP * FM;                            // [2][(DP+2)][64] train slice (+ alpha, |b|^2 rows)
   float *mu_sm = xt + 2 * (size_t)(DP + 2) * FK;               // [8][128]
@@ -84,35 +70,28 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
   if (tid == 0) {
     for (int j = 0; j < DP; ++j) inv_ell[j] = j < d ? 1.0 / prm.gp.ell[j] : 0.0;
     for (int s = 0; s < NSTA; ++s) {
-      mbar_init(smem_u32(&a_full[s]), PAIR ? 2 * GEN_WARPS : GEN_WARPS);
+      mbar_init(smem_u32(&a_full[s]), GEN_WARPS);
       mbar_init(smem_u32(&a_empty[s]), 1);
     }
     for (int s = 0; s < NSTB; ++s) {
       mbar_init(smem_u32(&b_full[s]), 1);
-      mbar_init(smem_u32(&b_empty[s]), PAIR ? 1 : cs);
+      mbar_init(smem_u32(&b_empty[s]), 1);
     }
-    for (int s = 0; s < 4; ++s) { mbar_init(smem_u32(&t_full[s]), 1); mbar_init(smem_u32(&t_empty[s]), PAIR ? 8 : 4); }
+    for (int s = 0; s < 4; ++s) { mbar_init(smem_u32(&t_full[s]), 1); mbar_init(smem_u32(&t_empty[s]), 4); }
     fence_mbar_init();
   }
   if (warp == 2) {
-    if (PAIR) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(smem_u32(tmem_slot)), "r"(512u));
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;\n" ::);
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(smem_u32(tmem_slot)), "r"(512u));
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::);
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(smem_u32(tmem_slot)), "r"(512u));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::);
   }
   tc_fence_before();
   __syncthreads();
-  if (cs > 1) cluster_sync_all();          // peers arrive on / write into this CTA's barriers and smem
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  const bool mo = prm.mean_only != 0;
   if (warp == 0) {
     // =============================== TMA producer (B tiles) ===============================
-    if (!mo && elect_one()) {
+    if (elect_one()) {
       uint32_t st = 0, ph = 0;
       long long w_bempty = 0; const bool pon = prm.prof != nullptr; const long long t_start = clock64();
       for (long long it = 0; it < n_iter; ++it) {
@@ -121,51 +100,26 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
           const int kb_end = last_kb(c_last) + 1;
           for (int kb = 0; kb < kb_end; ++kb) {
             for (int c = max(c_first, kb >> KSH); c <= c_last; ++c) {
-              if (WIDE) {                    // two ring entries per unit: the hi plane, then the lo plane
-                // rows of the chunk above the diagonal band are never multiplied (the UMMA's N shrinks):
-                // on the diagonal K-blocks only the 64-row boxes from r0 on are fetched
-                // (a ragged last chunk keeps the per-plane maps: their out-of-bounds rows are zero-filled)
-                const int r0 = (prm.trim_b && (c + 1) * CW <= np) ? max(0, kb - 4 * c) * 64 : 0;
+              // two ring entries per unit: the hi plane, then the lo plane.  Rows of the chunk above the diagonal
+              // band are never multiplied (the UMMA's N shrinks): on the diagonal K-blocks only the 64-row boxes
+              // from r0 on are fetched (a ragged last chunk keeps the per-plane maps: their out-of-bounds rows are
+              // zero-filled)
+              const int r0 = ((c + 1) * CW <= np) ? max(0, kb - 4 * c) * 64 : 0;
 #pragma unroll
-                for (int pl = 0; pl < 2; ++pl) {
-                  mbar_wait_prof(smem_u32(&b_empty[st]), ph ^ 1, 64, w_bempty, pon);
-                  const uint32_t full = smem_u32(&b_full[st]);
-                  const uint32_t dst = smem_u32(sB + st * STAGE_BYTES);
-                  if (r0 == 0) {
-                    mbar_expect_tx(full, STAGE_BYTES);
-                    tma_load_2d(dst, pl == 0 ? &map_hi : &map_lo, full, kb * FK, c * CW);
-                  } else {
-                    mbar_expect_tx(full, (uint32_t)((CW - r0) * 128));
-                    for (int rr = r0; rr < CW; rr += 64)       // map_kc: both planes as one (2 n_pad, n_pad) matrix, 64-row boxes
-                      tma_load_2d(dst + (uint32_t)(rr * 128), &map_kc, full, kb * FK, pl * np + c * CW + rr);
-                  }
-                  if (++st == NSTB) { st = 0; ph ^= 1; }
-                }
-                continue;
-              }
-              mbar_wait_prof(smem_u32(&b_empty[st]), ph ^ 1, 64, w_bempty, pon);
-              const uint32_t dst = smem_u32(sB + st * STAGE_BYTES);
-              if (PAIR) {                    // this CTA's half of the 256-row B tile; bytes counted on the leader
-                // the leader alone arms its barrier, with the bytes of BOTH halves (a remote expect_tx with
-                // release.cluster semantics costs the peer's producer ~1 us per stage and throttles the ring)
-                const uint32_t full = mapa_rank(smem_u32(&b_full[st]), 0);
-                if (crank == 0) mbar_expect_tx(smem_u32(&b_full[st]), 2 * STAGE_BYTES);
-                tma_load_2d_2sm(dst, &map_hi, full, kb * FK, c * CW + (int)crank * 128);
-                tma_load_2d_2sm(dst + PLANE_BYTES, &map_lo, full, kb * FK, c * CW + (int)crank * 128);
-              } else {
+              for (int pl = 0; pl < 2; ++pl) {
+                mbar_wait_prof(smem_u32(&b_empty[st]), ph ^ 1, 64, w_bempty, pon);
                 const uint32_t full = smem_u32(&b_full[st]);
-                mbar_expect_tx(full, STAGE_BYTES);
-                if (cs == 1) {
-                  tma_load_2d(dst, &map_hi, full, kb * FK, c * CW);
-                  tma_load_2d(dst + PLANE_BYTES, &map_lo, full, kb * FK, c * CW);
-                } else {                     // this CTA fetches rows [crank, crank+1) * 128/cs and multicasts them
-                  const int rows = 128 / (int)cs;
-                  const uint32_t sl = (uint32_t)(crank * rows * 128);
-                  tma_load_2d_mc(dst + sl, &map_hi, full, kb * FK, c * CW + (int)crank * rows, cmask);
-                  tma_load_2d_mc(dst + PLANE_BYTES + sl, &map_lo, full, kb * FK, c * CW + (int)crank * rows, cmask);
+                const uint32_t dst = smem_u32(sB + st * STAGE_BYTES);
+                if (r0 == 0) {
+                  mbar_expect_tx(full, STAGE_BYTES);
+                  tma_load_2d(dst, pl == 0 ? &map_hi : &map_lo, full, kb * FK, c * CW);
+                } else {
+                  mbar_expect_tx(full, (uint32_t)((CW - r0) * 128));
+                  for (int rr = r0; rr < CW; rr += 64)       // map_kc: both planes as one (2 n_pad, n_pad) matrix, 64-row boxes
+                    tma_load_2d(dst + (uint32_t)(rr * 128), &map_kc, full, kb * FK, pl * np + c * CW + rr);
                 }
+                if (++st == NSTB) { st = 0; ph ^= 1; }
               }
-              if (++st == NSTB) { st = 0; ph ^= 1; }
             }
           }
         }
@@ -173,8 +127,8 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
       if (pon) { prm.prof[blockIdx.x * 16 + 0] = w_bempty; prm.prof[blockIdx.x * 16 + 1] = clock64() - t_start; }
     }
   } else if (warp == 1) {
-    // =============================== MMA issuer (leader CTA only in PAIR mode) ============
-    if (!mo && leader && elect_one()) {
+    // =============================== MMA issuer ===========================================
+    if (elect_one()) {
       uint32_t sa = 0, pa = 0, sb = 0, pb = 0, tph = 0;   // tph: per-slot phase bits of t_empty
       // operand format chosen by K3 on the device (bscale[3]): bf16 planes for well-conditioned GPs, fp16 otherwise
       constexpr uint32_t IDESC_RT = IDESC | (F16 ? 0u : ((1u << 7) | (1u << 10)));
@@ -194,78 +148,34 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
                 tph ^= (1u << slot);
                 tc_fence_after();
               }
-              if (WIDE) {
-                // rows of the chunk above the diagonal band are zero: skip them (N = 256, 192, 128 or 64)
-                const int r0 = max(0, kb - 4 * c) * 64;
-                const uint32_t dcolw = tmem_base + (uint32_t)(slot * CW + r0);
-                const uint32_t idw = (IDESC_RT & ~(0x3Fu << 17)) | ((uint32_t)((CW - r0) >> 3) << 17);
-                // hi plane: A_hi.B_hi and A_lo.B_hi
-                mbar_wait_prof(smem_u32(&b_full[sb]), pb, MMA_SLEEP_NS, w_bfull, pon);
-                tc_fence_after();
-                uint32_t bp = smem_u32(sB + sb * STAGE_BYTES) + (uint32_t)(r0 * 128);
-                if (!(prm.dbg & 1)) {
-#pragma unroll
-                  for (int ks = 0; ks < FK / 16; ++ks) {
-                    const uint64_t dbh = make_sdesc(bp + ks * 32);
-                    umma_bf16(dcolw, make_sdesc(a_hi + ks * 32), dbh, idw, (kb > 0 || ks > 0) ? 1u : 0u);
-                    umma_bf16(dcolw, make_sdesc(a_lo + ks * 32), dbh, idw, 1u);
-                  }
-                }
-                umma_commit(smem_u32(&b_empty[sb]));
-                if (++sb == NSTB) { sb = 0; pb ^= 1; }
-                // lo plane: A_hi.B_lo
-                mbar_wait_prof(smem_u32(&b_full[sb]), pb, MMA_SLEEP_NS, w_bfull, pon);
-                tc_fence_after();
-                bp = smem_u32(sB + sb * STAGE_BYTES) + (uint32_t)(r0 * 128);
-                if (!(prm.dbg & 1)) {
-#pragma unroll
-                  for (int ks = 0; ks < FK / 16; ++ks)
-                    umma_bf16(dcolw, make_sdesc(a_hi + ks * 32), make_sdesc(bp + ks * 32), idw, 1u);
-                }
-                umma_commit(smem_u32(&b_empty[sb]));
-                if (++sb == NSTB) { sb = 0; pb ^= 1; }
-                if (kb == last_kb(c)) umma_commit(smem_u32(&t_full[slot]));      // chunk complete
-                continue;
-              }
+              // rows of the chunk above the diagonal band are zero: skip them (N = 256, 192, 128 or 64)
+              const int r0 = max(0, kb - 4 * c) * 64;
+              const uint32_t dcolw = tmem_base + (uint32_t)(slot * CW + r0);
+              const uint32_t idw = (IDESC_RT & ~(0x3Fu << 17)) | ((uint32_t)((CW - r0) >> 3) << 17);
+              // hi plane: A_hi.B_hi and A_lo.B_hi
               mbar_wait_prof(smem_u32(&b_full[sb]), pb, MMA_SLEEP_NS, w_bfull, pon);
               tc_fence_after();
-              uint32_t b_hi = smem_u32(sB + sb * STAGE_BYTES), b_lo = b_hi + PLANE_BYTES;
-              uint32_t dcol = tmem_base + (uint32_t)(slot * CW);
-              uint32_t idesc = IDESC_RT;
-              if (!PAIR && kb == 2 * c + 1) {
-                // second K-block of the diagonal 128x128 block: rows 0..63 of the chunk lie above the
-                // diagonal (zero), so only the lower 64 accumulator columns are touched: N = 64 UMMA
-                b_hi += 64 * 128; b_lo += 64 * 128; dcol += 64;
-                idesc = (IDESC_RT & ~(0x3Fu << 17)) | ((uint32_t)(64 >> 3) << 17);
-              }
-              if (!(prm.dbg & 1)) {
+              uint32_t bp = smem_u32(sB + sb * STAGE_BYTES) + (uint32_t)(r0 * 128);
 #pragma unroll
-                for (int ks = 0; ks < FK / 16; ++ks) {
-                  const uint64_t dah = make_sdesc(a_hi + ks * 32), dal = make_sdesc(a_lo + ks * 32);
-                  const uint64_t dbh = make_sdesc(b_hi + ks * 32), dbl = make_sdesc(b_lo + ks * 32);
-                  const uint32_t acc0 = (kb > 0 || ks > 0) ? 1u : 0u;
-                  if (PAIR) {
-                    umma_bf16_2sm(dcol, dah, dbh, idesc, acc0);
-                    umma_bf16_2sm(dcol, dal, dbh, idesc, 1u);
-                    umma_bf16_2sm(dcol, dah, dbl, idesc, 1u);
-                  } else {
-                    // All MMAs of a chunk accumulate into the SAME TMEM tile back to back: measured 2x faster
-                    // than alternating between two accumulators (the accumulator stays in the tensor core).
-                    umma_bf16_keep(dcol, dah, dbh, idesc, acc0);        // A_hi read once from smem ...
-                    umma_bf16_reuse_last(dcol, dah, dbl, idesc, 1u);   // ... and reused from the collector
-                    umma_bf16(dcol, dal, dbh, idesc, 1u);
-                  }
-                }
+              for (int ks = 0; ks < FK / 16; ++ks) {
+                const uint64_t dbh = make_sdesc(bp + ks * 32);
+                umma_bf16(dcolw, make_sdesc(a_hi + ks * 32), dbh, idw, (kb > 0 || ks > 0) ? 1u : 0u);
+                umma_bf16(dcolw, make_sdesc(a_lo + ks * 32), dbh, idw, 1u);
               }
-              if (PAIR) umma_commit_2sm(smem_u32(&b_empty[sb]));
-              else if (cs == 1) umma_commit(smem_u32(&b_empty[sb]));
-              else umma_commit_mc(smem_u32(&b_empty[sb]), cmask);
-              if (kb == last_kb(c)) {                                       // chunk complete
-                if (PAIR) umma_commit_2sm(smem_u32(&t_full[slot])); else umma_commit(smem_u32(&t_full[slot]));
-              }
+              umma_commit(smem_u32(&b_empty[sb]));
               if (++sb == NSTB) { sb = 0; pb ^= 1; }
+              // lo plane: A_hi.B_lo
+              mbar_wait_prof(smem_u32(&b_full[sb]), pb, MMA_SLEEP_NS, w_bfull, pon);
+              tc_fence_after();
+              bp = smem_u32(sB + sb * STAGE_BYTES) + (uint32_t)(r0 * 128);
+#pragma unroll
+              for (int ks = 0; ks < FK / 16; ++ks)
+                umma_bf16(dcolw, make_sdesc(a_hi + ks * 32), make_sdesc(bp + ks * 32), idw, 1u);
+              umma_commit(smem_u32(&b_empty[sb]));
+              if (++sb == NSTB) { sb = 0; pb ^= 1; }
+              if (kb == last_kb(c)) umma_commit(smem_u32(&t_full[slot]));      // chunk complete
             }
-            if (PAIR) umma_commit_2sm(smem_u32(&a_empty[sa])); else umma_commit(smem_u32(&a_empty[sa]));
+            umma_commit(smem_u32(&a_empty[sa]));
             if (++sa == NSTA) { sa = 0; pa ^= 1; }
           }
         }
@@ -277,7 +187,7 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
     const int quad = warp - 4;
     const int row = quad * 32 + lane;
     uint32_t fph = 0;                                        // per-slot phase bits of t_full
-    for (long long it = 0; it < (mo ? 0 : n_iter); ++it) {
+    for (long long it = 0; it < n_iter; ++it) {
       const long long tile = blockIdx.x + it * gridDim.x;
       double ss = 0.0;
       for (int c = 0; c < n_chunks; ++c) {
@@ -296,10 +206,7 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
         }
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) {
-          if (PAIR) mbar_arrive_cluster(mapa_rank(smem_u32(&t_empty[slot]), 0));
-          else mbar_arrive(smem_u32(&t_empty[slot]));
-        }
+        if (lane == 0) mbar_arrive(smem_u32(&t_empty[slot]));
         ss += (double)((part[0] + part[1]) + (part[2] + part[3]));
       }
       const long long cg = tile * FM + row;
@@ -316,13 +223,11 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
     // shared-memory reads in the inner loop are two broadcast LDS.128 of (negated) training
     // coordinates per dimension: the LSU traffic that competes with the UMMA operand fetch is
     // 1/R of a row-per-thread mapping.
-    const int gt = tid - 8 * 32;                 // 0 .. 32 GW - 1
-    const int q = (gt >> 5) & 7;                 // operand chunk 0..7 of this warp
-    const int rh = gt >> 8;                      // row half (GW = 16 only)
+    const int gt = tid - 8 * 32;                 // 0 .. 255
+    const int q = gt >> 5;                       // operand chunk 0..7 of this warp
     const bool matern = (prm.gp.kernel == OMBO_KERNEL_MATERN52);
     constexpr bool f16 = F16, direct = F16;         // fp16 planes (ill-conditioned GP): fp16 split + direct distances
-    constexpr int RB = 128 / (32 * R * (GW / 8));   // row batches per K-block
-    constexpr int ROW0 = R * RB;                  // rows (in units of 32) owned by one row half
+    constexpr int RB = 128 / (32 * R);              // row batches per K-block
     constexpr int XT_STRIDE = (DP + 2) * FK;
     uint32_t sa = 0, pa = 0;
     int xbuf = 0;
@@ -367,23 +272,23 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
         for (int rr = 0; rr < R; ++rr) {
           float acc = 0.f;
 #pragma unroll
-          for (int j = 0; j < DP; ++j) { x[rr][j] = xc[j * FM + lane + 32 * (ROW0 * rh + rr)]; acc = fmaf(x[rr][j], x[rr][j], acc); }
+          for (int j = 0; j < DP; ++j) { x[rr][j] = xc[j * FM + lane + 32 * rr]; acc = fmaf(x[rr][j], x[rr][j], acc); }
           a2[rr] = 0.25f * acc;
         }
       }
-      for (int p = 0; p < (mo ? 1 : n_pass); ++p) {
+      for (int p = 0; p < n_pass; ++p) {
         const int c_last = min(NSLOT * p + NSLOT - 1, n_chunks - 1);
-        const int kb_end = mo ? nkb : last_kb(c_last) + 1;
+        const int kb_end = last_kb(c_last) + 1;
         // K* blocks generated by an earlier pass of this tile are not recomputed: they were copied to a
         // per-CTA cache in L2 (bulk store of the 32 KB operand stage) and are streamed back by a bulk load
         // that completes the stage's full barrier.  Every K* block is generated exactly once per tile.
-        const bool use_cache = !mo && prm.kcache != nullptr;
-        const int kb_cached = (use_cache && p > 0 && !(prm.dbg & 16)) ? last_kb(min(NSLOT * (p - 1) + NSLOT - 1, n_chunks - 1)) + 1 : 0;
+        const bool use_cache = prm.kcache != nullptr;
+        const int kb_cached = (use_cache && p > 0) ? last_kb(min(NSLOT * (p - 1) + NSLOT - 1, n_chunks - 1)) + 1 : 0;
         const bool store_cache = use_cache && (p + 1 < n_pass);
         unsigned char *kc = prm.kcache + (size_t)blockIdx.x * nkb * STAGE_BYTES;
         if (kb_cached > 0 && gt == 0) asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory");   // stores landed
         for (int kb = 0; kb < kb_end; ++kb) {
-          const bool do_mu = mo || !use_cache ? (mo || p == n_pass - 1) : true;
+          const bool do_mu = use_cache || p == n_pass - 1;     // without the cache every pass regenerates K*
           const int kb_next = (kb + 1 < kb_end) ? kb + 1 : 0;
           prefetch_slice(xt + (xbuf ^ 1) * XT_STRIDE, kb_next);          // lands while this K-block is computed
           if (kb < kb_cached) {
@@ -392,18 +297,9 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
               // released: the other warps do not wait on a_empty here, so an arrival of their own could land
               // in the still-open phase of two K-blocks ago (its bulk load may not have completed yet)
               mbar_wait_prof(smem_u32(&a_empty[sa]), pa ^ 1, 32, w_aempty, pon);
-              if (PAIR) {
-                // the stage lands in THIS CTA's shared memory, its bytes are counted on the leader's barrier
-                // (2-SM tensor load through a linear map of the cache: 256 rows of 128 B = one stage)
-                const uint32_t full = mapa_rank(smem_u32(&a_full[sa]), 0);
-                mbar_expect_tx_cluster(full, STAGE_BYTES);
-                mbar_arrive_n_cluster(full, GEN_WARPS - 1);
-                tma_load_2d_2sm(smem_u32(sA + sa * STAGE_BYTES), &map_kc, full, 0, (int)((blockIdx.x * nkb + kb) * 256));
-              } else {
-                mbar_expect_tx(smem_u32(&a_full[sa]), STAGE_BYTES);
-                mbar_arrive_n(smem_u32(&a_full[sa]), GEN_WARPS - 1);
-                bulk_load(smem_u32(sA + sa * STAGE_BYTES), kc + (size_t)kb * STAGE_BYTES, STAGE_BYTES, smem_u32(&a_full[sa]));
-              }
+              mbar_expect_tx(smem_u32(&a_full[sa]), STAGE_BYTES);
+              mbar_arrive_n(smem_u32(&a_full[sa]), GEN_WARPS - 1);
+              bulk_load(smem_u32(sA + sa * STAGE_BYTES), kc + (size_t)kb * STAGE_BYTES, STAGE_BYTES, smem_u32(&a_full[sa]));
             }
             if (++sa == NSTA) { sa = 0; pa ^= 1; }
             asm volatile("cp.async.wait_group 0;\n" ::: "memory");
@@ -413,16 +309,15 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
           }
           const float *xs = xt + xbuf * XT_STRIDE + 8 * q;
           unsigned char *st_hi = sA + sa * STAGE_BYTES, *st_lo = st_hi + PLANE_BYTES;
-          if (prm.dbg & 2) mbar_wait_sleep(smem_u32(&a_empty[sa]), pa ^ 1, 32);
 #pragma unroll 1
-          for (int rb = 0; rb < ((prm.dbg & 2) ? 0 : RB); ++rb) {
+          for (int rb = 0; rb < RB; ++rb) {
             if (RB > 1) {
 #pragma unroll
               for (int rr = 0; rr < R; ++rr) {
                 float acc = 0.f;
 #pragma unroll
                 for (int j = 0; j < DP; ++j) {
-                  x[rr][j] = xc[j * FM + lane + 32 * (ROW0 * rh + R * rb + rr)];
+                  x[rr][j] = xc[j * FM + lane + 32 * (R * rb + rr)];
                   acc = fmaf(x[rr][j], x[rr][j], acc);
                 }
                 a2[rr] = 0.25f * acc;
@@ -479,7 +374,7 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
             }
             const float4 al0 = *(const float4 *)(xs + DP * FK);
             const float4 al1 = *(const float4 *)(xs + DP * FK + 4);
-            if (rb == 0 && !mo) mbar_wait_prof(smem_u32(&a_empty[sa]), pa ^ 1, 32, w_aempty, pon);   // stage released by the MMA
+            if (rb == 0) mbar_wait_prof(smem_u32(&a_empty[sa]), pa ^ 1, 32, w_aempty, pon);   // stage released by the MMA
 #pragma unroll
             for (int rr = 0; rr < R; ++rr) {
               float2 kv[4];
@@ -513,7 +408,6 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
                 m2 = __ffma2_rn(kv[3], make_float2(al1.z, al1.w), m2);
                 mu_acc[R * rb + rr] += m2.x + m2.y;
               }
-              if (!mo) {
               uint32_t hi[4], lo[4];
               if (f16) {
 #pragma unroll
@@ -534,19 +428,15 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
                   lo[e] = *reinterpret_cast<uint32_t *>(&l);
                 }
               }
-              const int row = lane + 32 * (ROW0 * rh + R * rb + rr);
+              const int row = lane + 32 * (R * rb + rr);
               const uint32_t off = (uint32_t)((row >> 3) * 1024 + (row & 7) * 128 + (((q ^ (row & 7)) & 7) << 4));
               *(uint4 *)(st_hi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
               *(uint4 *)(st_lo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-              }
             }
           }
-          if (!mo) fence_proxy_async_smem();
+          fence_proxy_async_smem();
           __syncwarp();
-          if (lane == 0 && !mo) {
-            if (PAIR) mbar_arrive_cluster(mapa_rank(smem_u32(&a_full[sa]), 0));   // the leader's MMA consumes both halves
-            else mbar_arrive(smem_u32(&a_full[sa]));
-          }
+          if (lane == 0) mbar_arrive(smem_u32(&a_full[sa]));
           const uint32_t stage_just_written = smem_u32(sA + sa * STAGE_BYTES);
           if (++sa == NSTA) { sa = 0; pa ^= 1; }
           asm volatile("cp.async.wait_group 0;\n" ::: "memory");          // next slice has landed
@@ -555,14 +445,14 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
           { long long t0 = pon ? clock64() : 0;
             asm volatile("bar.sync 1, %0;\n" ::"n"(GEN_THREADS));
             if (pon) w_bar += clock64() - t0; }
-          if (store_cache && gt == 0 && !(prm.dbg & 8)) bulk_store(kc + (size_t)kb * STAGE_BYTES, stage_just_written, STAGE_BYTES);
+          if (store_cache && gt == 0) bulk_store(kc + (size_t)kb * STAGE_BYTES, stage_just_written, STAGE_BYTES);
           xbuf ^= 1;
         }
       }
       if (pon && lane == 0) { prm.prof[blockIdx.x * 16 + 5 + 0] = w_aempty; if (q == 0) prm.prof[blockIdx.x * 16 + 6] = w_bar; if (q == 7) prm.prof[blockIdx.x * 16 + 7] = w_bar; }
       // mean: one partial sum per (chunk warp, row)
 #pragma unroll
-      for (int r4 = 0; r4 < ROW0; ++r4) mu_sm[q * FM + lane + 32 * (ROW0 * rh + r4)] = mu_acc[r4];
+      for (int r4 = 0; r4 < 4; ++r4) mu_sm[q * FM + lane + 32 * r4] = mu_acc[r4];
       asm volatile("bar.sync 1, %0;\n" ::"n"(GEN_THREADS));
       if (gt < FM) {
         const long long cg = tile * FM + gt;
@@ -571,7 +461,6 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
 #pragma unroll
           for (int w = 0; w < 8; ++w) acc += mu_sm[w * FM + gt];
           prm.mu_out[cg] = (double)acc;
-          if (mo) prm.var_out[cg] = nan("");
         }
       }
     }
@@ -580,11 +469,7 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
   // ---- teardown ----
   tc_fence_before();
   __syncthreads();
-  if (cs > 1) cluster_sync_all();          // nobody exits while a peer may still signal / multicast to it
-  if (warp == 2) {
-    if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;\n" ::"r"(tmem_base), "r"(512u));
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem_base), "r"(512u));
-  }
+  if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem_base), "r"(512u));
 }
 
 
@@ -593,7 +478,8 @@ k_posterior_fast(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
 // reference's semantics, the Pareto-label GP of KEEP).  No tensor core, no operand ring: K1 + the dot product with
 // sigma_f2 alpha.  The generator code of the main kernel would leave half of the SM idle here (8 of its 16 warps),
 // so this is a separate 256-thread kernel with a few KB of shared memory: two CTAs per SM, 16 K1 warps.
-// Warp q owns training points 8q..8q+7 of every 64-block, lane l the candidate rows l + 32 rr (as in the main kernel).
+// Warp q owns training points 8q..8q+7 of every 64-block, lane l the candidate rows l + 32 rr, with the main kernel's
+// distance form, k' arithmetic and summation order: mu is bit-identical to that of a variance launch.
 // =================================================================================================
 template <int DP, int R, bool DIRECT>
 __global__ void __launch_bounds__(256, 2)
@@ -655,7 +541,12 @@ k_posterior_mean_fast(const FastParams prm) {
       const float *xs = xt + xbuf * XT_STRIDE + 8 * q;
 #pragma unroll 1
       for (int rb = 0; rb < RB; ++rb) {
-        if (RB > 1) load_rows(rb);
+        if (RB > 1) {
+          // compiler barrier: the training-slice loads below do not depend on rb, and hoisted out of this loop
+          // they would hold 8 x DP values per lane (spills at DP = 16 / 24)
+          asm volatile("" ::: "memory");
+          load_rows(rb);
+        }
         float2 r2[R][4];
         if (DIRECT) {
 #pragma unroll
@@ -803,25 +694,15 @@ int ombo_make_linear_map(CUtensorMap *map, const void *base, size_t rows) {
 
 int ombo_fast_path_built() { return 1; }
 
-template <int DP, int R, int MODE, int GW, bool F16>
+template <int DP, int R, bool F16>
 static int launch_fast(ombo_ctx *ctx, const CUtensorMap &map_hi, const CUtensorMap &map_lo, const CUtensorMap &map_kc, const FastParams &prm,
-                       int grid, int cs, cudaStream_t s) {
+                       int grid, cudaStream_t s) {
   const size_t smem = (size_t)6 * STAGE_BYTES + (size_t)DP * FM * 4 + 2 * (size_t)(DP + 2) * FK * 4 +
                       8 * FM * 4 + 16 + 24 * 8 + 24 * 8 + 1024;   // barriers + TMEM slot, 1/lengthscale, alignment slack
   // set on every launch: the attribute belongs to the (function, device) pair, and one process may drive several devices
-  OMBO_CUDA(cudaFuncSetAttribute(k_posterior_fast<DP, R, MODE, GW, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  OMBO_CUDA(cudaFuncSetAttribute(k_posterior_fast<DP, R, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ProfScope prof(ctx, s);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3((8 + GW) * 32);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  OMBO_CUDA(cudaLaunchKernelEx(&cfg, k_posterior_fast<DP, R, MODE, GW, F16>, map_hi, map_lo, map_kc, prm));
+  k_posterior_fast<DP, R, F16><<<grid, 16 * 32, smem, s>>>(map_hi, map_lo, map_kc, prm);
   return OMBO_OK;
 }
 
@@ -835,12 +716,10 @@ int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lon
   }
   long long tiles = (m + FM - 1) / FM;
   const ombo_knobs &kn = ctx->knobs;
-  if (!want_var && gp.d <= 12 && !kn.fast_mean_in_main) {
-    // mean-only: the dedicated K1 kernel (two CTAs per SM; d <= 12 keeps 4 rows x d coordinates in registers)
-    FastParams prm;
-    prm.gp = gp; prm.pool = pool; prm.m = m; prm.mu_out = mu; prm.var_out = var; prm.mean_only = 1;
-    prm.kcache = nullptr; prm.prof = nullptr; prm.dbg = 0; prm.trim_b = 0;
-    const long long tiles = (m + FM - 1) / FM;
+  if (!want_var) {
+    // mean-only: the dedicated K1 kernel (two CTAs per SM; rows per lane and dimension padding as in the main kernel)
+    FastParams prm = {};
+    prm.gp = gp; prm.pool = pool; prm.m = m; prm.mu_out = mu; prm.var_out = var;
     const int grid = (int)(tiles < 2LL * ctx->num_sms ? tiles : 2LL * ctx->num_sms);
     const bool direct = (gp.flags & OMBO_GP_FP16_PLANES) != 0;
     ProfScope prof(ctx, s);
@@ -849,76 +728,43 @@ int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lon
       if (direct) k_posterior_mean_fast<DPV, RV, true><<<grid, 256, 0, s>>>(prm);                       \
       else k_posterior_mean_fast<DPV, RV, false><<<grid, 256, 0, s>>>(prm);                             \
     } else
-    MEAN_CASE(2, 4) MEAN_CASE(4, 4) MEAN_CASE(6, 4) MEAN_CASE(8, 4) MEAN_CASE(10, 4)
-    { if (direct) k_posterior_mean_fast<12, 4, true><<<grid, 256, 0, s>>>(prm);
-      else k_posterior_mean_fast<12, 4, false><<<grid, 256, 0, s>>>(prm); }
+    MEAN_CASE(2, 4) MEAN_CASE(4, 4) MEAN_CASE(6, 4) MEAN_CASE(8, 4) MEAN_CASE(10, 4) MEAN_CASE(12, 4) MEAN_CASE(16, 2)
+    { if (direct) k_posterior_mean_fast<24, 2, true><<<grid, 256, 0, s>>>(prm);
+      else k_posterior_mean_fast<24, 2, false><<<grid, 256, 0, s>>>(prm); }
 #undef MEAN_CASE
     ctx->launches += 1;
     OMBO_CUDA(cudaGetLastError());
     return OMBO_OK;
   }
-  // default: single-CTA UMMA with 256-column chunks (mode 3).  The B200s of this pool run the kernel at their 1 kW
-  // power cap (SM clock ~1.6 GHz), where time follows energy, i.e. issued tensor work: the single-CTA variant can
-  // shrink N on the diagonal K-blocks, the cta_group::2 variants cannot (N is split across the pair) and issue 17 %
-  // more MMAs.  Kept selectable (verified by the GPU tests): OMBO_FAST_MODE=1 the 128-column variant
-  // (OMBO_FAST_CLUSTER its multicast cluster size), 2 the coupled cta_group::2 pair, 4 the decoupled pair
-  // (k_posterior_fast_dc, d <= 12).
-  bool pair = false, wide = true, dc = false;
-  int cs = 1;
-  if (want_var && (gp.flags & OMBO_GP_F8C_PLANES)) return ombo_posterior_fast8(ctx, gp, pool, m, mu, var, s, fuse_req, fused, bound_chunks);
-  { const int mode = kn.fast_mode ? kn.fast_mode : 3;
-    if (mode == 1) wide = false;
-    else if (mode == 2) { wide = false; pair = true; }
-    else if (mode == 4 && gp.d <= 12) { wide = false; pair = true; dc = true; } }
-  if (!pair && !wide) { cs = kn.fast_cluster; if (cs != 1 && cs != 2 && cs != 4) cs = 1; if (tiles < cs) cs = 1; }
-  if (pair) cs = 2;
-  CUtensorMap map_hi, map_lo;
-  const int box_rows = wide ? 256 : (pair ? 128 : 128 / cs);
-  int rc = make_b_map(&map_hi, gp.bhi, gp.n_pad, box_rows);
+  if (gp.flags & OMBO_GP_F8C_PLANES) return ombo_posterior_fast8(ctx, gp, pool, m, mu, var, s, fuse_req, fused, bound_chunks);
+  CUtensorMap map_hi, map_lo, map_kc;
+  int rc = make_b_map(&map_hi, gp.bhi, gp.n_pad, 256);
   if (rc) return rc;
-  rc = make_b_map(&map_lo, gp.blo, gp.n_pad, box_rows);
+  rc = make_b_map(&map_lo, gp.blo, gp.n_pad, 256);
   if (rc) return rc;
-  FastParams prm;
-  prm.gp = gp; prm.pool = pool; prm.m = m; prm.mu_out = mu; prm.var_out = var; prm.mean_only = want_var ? 0 : 1;
-  prm.dbg = kn.fast_dbg;
+  FastParams prm = {};
+  prm.gp = gp; prm.pool = pool; prm.m = m; prm.mu_out = mu; prm.var_out = var;
   const bool want_prof = kn.fast_profile != 0;
   if (want_prof && !ctx->prof_dev) OMBO_CUDA(cudaMalloc(&ctx->prof_dev, 16 * 256 * sizeof(long long)));
   long long *prof_dev = ctx->prof_dev;
   prm.prof = want_prof ? prof_dev : nullptr;
   if (want_prof) OMBO_CUDA(cudaMemsetAsync(prof_dev, 0, 16 * 256 * sizeof(long long), s));
-  int grid = (int)(tiles < ctx->num_sms ? tiles : ctx->num_sms);
-  grid = (grid + cs - 1) / cs * cs;            // whole clusters; surplus CTAs run a dummy tile
-  if (grid > ctx->num_sms) grid = ctx->num_sms / cs * cs;
-  prm.kcache = nullptr;
-  CUtensorMap map_kc = map_hi;                 // pair variants: linear map of the K* cache; wide: 64-row boxes of B
-  prm.trim_b = 0;
-  if (wide && (const unsigned char *)gp.blo == (const unsigned char *)gp.bhi + (size_t)gp.n_pad * gp.n_pad * 2 &&
-      !kn.fast_notrim) {
-    // the two bf16 planes are adjacent in the state blob: one map over (2 n_pad, n_pad) serves both
-    rc = make_b_map(&map_kc, gp.bhi, gp.n_pad, 64, 2 * gp.n_pad);
-    if (rc) return rc;
-    prm.trim_b = 1;
-  }
-  if (want_var && (dc || (gp.n_pad > 512 && !kn.fast_nocache))) {   // dc: always; else only with > 1 TMEM pass
+  const int grid = (int)(tiles < ctx->num_sms ? tiles : ctx->num_sms);
+  // the two planes are adjacent in the state blob (gp_layout): one map of 64-row boxes over (2 n_pad, n_pad) serves both
+  rc = make_b_map(&map_kc, gp.bhi, gp.n_pad, 64, 2 * gp.n_pad);
+  if (rc) return rc;
+  if (gp.n_pad > 512) {            // more than one TMEM pass: generated K* blocks are cached in L2
     rc = ombo_ws_reserve(&ctx->ws_scratch, &ctx->ws_scratch_bytes, (size_t)grid * (gp.n_pad / FK) * STAGE_BYTES);
     if (rc) return rc;
     prm.kcache = (unsigned char *)ctx->ws_scratch;
-    if (kn.fast_zerocache) OMBO_CUDA(cudaMemsetAsync(prm.kcache, 0, (size_t)grid * (gp.n_pad / FK) * STAGE_BYTES, s));
-    if (pair) {
-      rc = ombo_make_linear_map(&map_kc, prm.kcache, (size_t)grid * (gp.n_pad / FK) * 256);
-      if (rc) return rc;
-    }
   }
   const int d = gp.d;
   // (16 generator warps with 2 rows per lane were measured too: the same number of independent chains per
   // scheduler, no gain -- the instantiations were dropped to keep the build short)
   const bool f16 = (gp.flags & OMBO_GP_FP16_PLANES) != 0;     // format of the planes, as reported by the refresh
-#define FAST_DISPATCH_F(DPV, RV, FV)                                                                  \
-  rc = dc ? ombo_launch_fast_dc(ctx, map_hi, map_lo, map_kc, prm, grid, s)                              \
-     : pair ? launch_fast<DPV, RV, 1, 8, FV>(ctx, map_hi, map_lo, map_kc, prm, grid, cs, s)             \
-     : wide ? launch_fast<DPV, RV, 2, 8, FV>(ctx, map_hi, map_lo, map_kc, prm, grid, cs, s)             \
-            : launch_fast<DPV, RV, 0, 8, FV>(ctx, map_hi, map_lo, map_kc, prm, grid, cs, s)
-#define FAST_DISPATCH(DPV, RV) do { if (f16) { FAST_DISPATCH_F(DPV, RV, true); } else { FAST_DISPATCH_F(DPV, RV, false); } } while (0)
+#define FAST_DISPATCH(DPV, RV)                                                                                \
+  rc = f16 ? launch_fast<DPV, RV, true>(ctx, map_hi, map_lo, map_kc, prm, grid, s)                            \
+           : launch_fast<DPV, RV, false>(ctx, map_hi, map_lo, map_kc, prm, grid, s)
   if (d <= 2) { FAST_DISPATCH(2, 4); }
   else if (d <= 4) { FAST_DISPATCH(4, 4); }
   else if (d <= 6) { FAST_DISPATCH(6, 4); }
@@ -928,7 +774,6 @@ int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lon
   else if (d <= 16) { FAST_DISPATCH(16, 2); }
   else { FAST_DISPATCH(24, 2); }
 #undef FAST_DISPATCH
-#undef FAST_DISPATCH_F
   if (rc) return rc;
   ctx->launches += 1;
   OMBO_CUDA(cudaGetLastError());
@@ -936,12 +781,11 @@ int ombo_posterior_fast(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lon
     static long long h[16 * 256];
     OMBO_CUDA(cudaStreamSynchronize(s));
     OMBO_CUDA(cudaMemcpy(h, prof_dev, sizeof(h), cudaMemcpyDeviceToHost));
-    double a[10] = {0};
-    for (int b = 0; b < grid; ++b) for (int k = 0; k < 10; ++k) a[k] += (double)h[b * 16 + k] / grid;
+    double a[8] = {0};
+    for (int b = 0; b < grid; ++b) for (int k = 0; k < 8; ++k) a[k] += (double)h[b * 16 + k] / grid;
     fprintf(stderr, "[fast prof] per-CTA cycles: tma.wait_b_empty %.0f / tma.total %.0f | mma.wait_a_full %.0f wait_b_full %.0f "
             "wait_t_empty %.0f | gen.wait_a_empty %.0f gen.bar(w0) %.0f gen.bar(w7) %.0f  (tiles/CTA %.1f)\n",
             a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], (double)tiles / grid);
-    if (dc) fprintf(stderr, "[fast prof] feeder: wait_produced %.0f wait_a_empty %.0f | gen.wait_slot %.0f\n", a[8], a[9], a[5]);
   }
   return OMBO_OK;
 }

@@ -968,8 +968,8 @@ int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lo
   if ((rc = make_plane_map(&maps.c2_32, c2, gp.n_pad, 1, 32))) return rc;
   maps.kc = maps.hi128;
   FastParams prm;
-  prm.gp = gp; prm.pool = pool; prm.m = m; prm.mu_out = mu; prm.var_out = var; prm.mean_only = 0;
-  prm.dbg = ctx->knobs.fast_dbg; prm.trim_b = 1; prm.kcache = nullptr;
+  prm.gp = gp; prm.pool = pool; prm.m = m; prm.mu_out = mu; prm.var_out = var;
+  prm.dbg = ctx->knobs.fast_dbg; prm.kcache = nullptr;
   const bool want_prof = ctx->knobs.fast_profile != 0;
   if (want_prof && !ctx->prof_dev) OMBO_CUDA(cudaMalloc(&ctx->prof_dev, 16 * 256 * sizeof(long long)));
   prm.prof = want_prof ? ctx->prof_dev : nullptr;

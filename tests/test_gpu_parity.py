@@ -2,6 +2,10 @@
 seeded inputs, against the committed golden fixtures minted from the reference's own code, and
 through size-independent properties.  Tolerances: FP64 mode rtol 1e-6 (north_star) with the
 atol the SURVEY derives (section 7, "variance cancellation"): atol = 1e-7 * sigma_f on sigma."""
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 
@@ -16,6 +20,7 @@ from optimobo_b200 import _cabi  # noqa: E402
 from oracle import oracle as O  # noqa: E402
 
 DEV = "cuda:0"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def zdt1(X):
@@ -403,28 +408,69 @@ def test_posterior_fast_vs_oracle(n, d, m):
         assert torch.equal(mu_b[0].cpu(), torch.as_tensor(mu)) and torch.equal(var_b[0].cpu(), torch.as_tensor(var))
 
 
-@pytest.mark.parametrize("mode", ["1", "2", "4"])
-def test_posterior_fast_kernel_variants(mode, monkeypatch):
-    """The variants kept selectable next to the default kernel (128-column single CTA, coupled
-    cta_group::2 pair, decoupled pair) answer within the same tolerance -- ragged m, one to three
-    TMEM passes, n_pad = 128 (two K-blocks: shorter than the operand ring)."""
+def _in_fresh_process(call, **env):
+    """Runs `call` (source text calling a function of this module) in a new interpreter with `env` added to the
+    environment: the library reads its knobs once per process, when it creates the device context."""
+    code = f"import sys\nsys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'tests')!r}]\nimport test_gpu_parity as T\nT.{call}\n"
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, **env), capture_output=True, text=True,
+                         timeout=600)
+    assert out.returncode == 0, out.stderr[-3000:]
+
+
+def _posterior_16bit_vs_oracle(n, d, m):
+    X, Y, ells, sf2 = make_problem(n, d)
+    gp = ob.GPModel(X, Y[:, 0], ells[0], sf2[0], device=DEV)
+    assert gp.plane_format in ("bf16x3", "fp16x3"), gp.plane_format      # k_posterior_fast, not the f8c kernel
+    st = O.gp_fit_state(X, Y[:, 0], ells[0], sf2[0])
+    Xc = np.random.default_rng(n + d).random((m, d))
+    sel = np.random.default_rng(1).integers(0, m, min(m, 3000))
+    mu_o, var_o = O.gp_posterior(st, Xc[sel])
+    mu, var = ob.posterior([gp], Xc, precision="fast")
+    mu, var = mu[0].cpu().numpy(), var[0].cpu().numpy()
+    np.testing.assert_allclose(mu[sel], mu_o, rtol=1e-3, atol=1e-3 * np.abs(mu_o).max())
+    np.testing.assert_allclose(np.sqrt(var[sel]), np.sqrt(var_o), rtol=1e-3, atol=1e-3 * np.sqrt(sf2[0]))
+    mu_b, var_b = ob.posterior([gp], Xc, precision="fast")
+    assert torch.equal(mu_b[0].cpu(), torch.as_tensor(mu)) and torch.equal(var_b[0].cpu(), torch.as_tensor(var))
+
+
+@pytest.mark.parametrize("n,d,m", [(100, 4, 129), (512, 12, 3000), (1024, 10, 148 * 128 * 2 + 77), (1536, 7, 2048)])
+def test_posterior_fast_16bit_kernel(n, d, m):
+    """The 16-bit x3 kernel on the shapes the f8c kernel would otherwise take (OMBO_NO_F8C, in a fresh process):
+    ragged m, one to three TMEM passes, n_pad = 128 (two K-blocks: shorter than the operand ring)."""
     if not _cabi.fast_path_available():
         pytest.skip("fast path not built")
-    monkeypatch.setenv("OMBO_FAST_MODE", mode)
-    for n, d, m in ((100, 4, 129), (512, 12, 3000), (1024, 10, 148 * 128 * 2 + 77), (1536, 7, 2048)):
-        X, Y, ells, sf2 = make_problem(n, d)
-        gp = ob.GPModel(X, Y[:, 0], ells[0], sf2[0], device=DEV)
-        st = O.gp_fit_state(X, Y[:, 0], ells[0], sf2[0])
-        Xc = np.random.default_rng(n + d).random((m, d))
-        sel = np.random.default_rng(1).integers(0, m, min(m, 3000))
-        mu_o, var_o = O.gp_posterior(st, Xc[sel])
-        mu, var = ob.posterior([gp], Xc, precision="fast")
-        mu, var = mu[0].cpu().numpy(), var[0].cpu().numpy()
-        np.testing.assert_allclose(mu[sel], mu_o, rtol=1e-3, atol=1e-3 * np.abs(mu_o).max())
-        np.testing.assert_allclose(np.sqrt(var[sel]), np.sqrt(var_o), rtol=1e-3, atol=1e-3 * np.sqrt(sf2[0]))
-        mu_b, var_b = ob.posterior([gp], Xc, precision="fast")
-        assert torch.equal(mu_b[0].cpu(), torch.as_tensor(mu)) and torch.equal(var_b[0].cpu(), torch.as_tensor(var))
-    # mean-only launches (the acquisition never reads this model's variance) and d > 12 (mode 4 falls back)
+    _in_fresh_process(f"_posterior_16bit_vs_oracle({n}, {d}, {m})", OMBO_NO_F8C="1")
+
+
+def _mean_only_matches_variance_launch(d, ell_bf16, ell_fp16):
+    X = np.random.default_rng(d).random((300, d))
+    Y = zdt1(X)
+    spec = ob.spec_ehvi(Y.max(0), ob.host_prep.calc_pf(Y), ob.host_prep.cached_samples(2, 5, seed=0), "reference")
+    pool = ob.CandidatePool.counter(5000, np.zeros(d), np.ones(d), seed=d)
+    for ell, fmt in ((ell_bf16, "bf16x3"), (ell_fp16, "fp16x3")):
+        models = [ob.GPModel(X, Y[:, i], ell * np.ones(d), 1.0 + i, device=DEV) for i in range(2)]
+        assert models[1].plane_format == fmt, (models[1].plane_format, models[1].conditioning)
+        # reference semantics never reads model 1's variance: without the posterior requested, model 1 runs the
+        # mean-only kernel; with it, k_posterior_fast computes its mean next to the variance
+        mean_only = ob.score(models, spec, pool, precision="fast", want_acq=True)
+        both = ob.score(models, spec, pool, precision="fast", want_acq=True, want_posterior=True)
+        assert torch.equal(mean_only.acq, both.acq)
+
+
+@pytest.mark.parametrize("d,ell_bf16,ell_fp16", [(6, 0.5, 1.0), (13, 1.0, 3.0), (16, 1.0, 3.0), (24, 1.0, 6.0)])
+def test_fast_mean_only_launch_is_bit_identical(d, ell_bf16, ell_fp16):
+    """Mean-only launches (k_posterior_mean_fast) give the mean of a variance launch bit for bit, on bf16 and fp16
+    planes, with 4 (d <= 12) and 2 (d > 12) candidate rows per generator lane."""
+    if not _cabi.fast_path_available():
+        pytest.skip("fast path not built")
+    _in_fresh_process(f"_mean_only_matches_variance_launch({d}, {ell_bf16}, {ell_fp16})", OMBO_NO_F8C="1")
+
+
+def test_fast_mode_d16_and_reference_semantics():
+    """d > 12 (bf16 x3 planes, 2 rows per generator lane) against the oracle, and the reference-semantics EHVI in fast
+    mode (model 1 mean-only) against FP64."""
+    if not _cabi.fast_path_available():
+        pytest.skip("fast path not built")
     X, Y, ells, sf2 = make_problem(300, 16)
     gp = ob.GPModel(X, Y[:, 0], ells[0] * 2.0, sf2[0], device=DEV)
     st = O.gp_fit_state(X, Y[:, 0], ells[0] * 2.0, sf2[0])
@@ -432,7 +478,6 @@ def test_posterior_fast_kernel_variants(mode, monkeypatch):
     mu_o, var_o = O.gp_posterior(st, Xc)
     mu, var = ob.posterior([gp], Xc, precision="fast")
     np.testing.assert_allclose(np.sqrt(var[0].cpu().numpy()), np.sqrt(var_o), rtol=2e-3, atol=2e-3 * np.sqrt(sf2[0]))
-    # reference semantics never reads model 1's variance: that GP runs the kernel's mean-only path
     X, Y, ells, sf2 = make_problem(640, 6)
     models = [ob.GPModel(X, Y[:, i], ells[i], sf2[i], device=DEV) for i in range(2)]
     spec = ob.spec_ehvi(Y.max(0), ob.host_prep.calc_pf(Y), ob.host_prep.cached_samples(2, 5, seed=0), "reference")
