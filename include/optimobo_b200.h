@@ -13,6 +13,7 @@
  *                        :118,:366; cparego.py:94,:544; emo.py:240; the EA loops
  *                        parego.py:242-270, keep.py:260-292       (rows a1-a12 / K1,K2,K4,K5)
  *   ombo_score_host   <- same, with the candidate pool in HOST memory (end-to-end entry)
+ *   ombo_score_topk   <- same, keeping the k best candidates (batch proposals; no reference counterpart)
  *   acquisition kinds <- util_functions.py:136 (EHVI), :170 (EHVI_3D), :285
  *                        (expected_decomposition), optimisers.py:325 / parego.py:126 /
  *                        keep.py:118 / cparego.py:450 (EI), cparego.py:486 (consraint_ei),
@@ -206,6 +207,14 @@ int ombo_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *poo
                const ombo_acq *acq, int precision, double *out_mu, double *out_var,
                double *out_acq, ombo_best *best_dev, void *stream);
 
+/* The k best candidates of the pool: topk_dev DEVICE (k,) ombo_best sorted by value descending, ties -> lowest
+ * global index, NaN treated as -inf (a stable descending sort of the values ombo_score would write to out_acq; -0
+ * ranks and is reported as +0).  Slots beyond pool->m hold (-inf, -1).  1 <= k <= OMBO_TOPK_MAX.  Every pass is
+ * scored unpruned.  Workspace O(k + 2^OMBO_CHUNK_LOG2), never O(m).  Asynchronous on `stream`. */
+#define OMBO_TOPK_MAX 65536
+int ombo_score_topk(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
+                    int precision, int k, ombo_best *topk_dev, void *stream);
+
 /* End-to-end twin: pool->X is a HOST buffer (pinned for full speed); chunks are copied
  * host->device on a side stream overlapped with scoring; `best_host` is read back and the
  * call returns after the result is on the host. */
@@ -227,6 +236,13 @@ int ombo_acquire_posterior(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const d
 /* regenerates rows [index, index+count) of a counter-generated pool into DEVICE out (count,d) f64 */
 int ombo_pool_rows(ombo_ctx *ctx, const ombo_pool *pool, int64_t index, int64_t count,
                    double *out, void *stream);
+
+/* rows of the listed global indices of a pool (index_dev DEVICE (count,) int64, each in [index_base, index_base + m))
+ * into DEVICE out (count, d) f64, exactly as the scoring kernels read them: the f32 values of an f32 pool (exact in
+ * f64), the f64 coordinates of an f64 or counter-generated pool.  Scoring those rows as an explicit pool of the
+ * pool's dtype reproduces the values of the full pool (batch shortlists). */
+int ombo_pool_gather(ombo_ctx *ctx, const ombo_pool *pool, const int64_t *index_dev, int64_t count, double *out,
+                     void *stream);
 
 /* C1 support: packs the 16-byte best into ONE order-preserving signed 64-bit key for a single
  * NCCL all-reduce(MAX): high 32 bits = order-preserving image of (float)value, low 32 bits =

@@ -22,6 +22,7 @@ SEM_REFERENCE, SEM_EXACT = 0, 1
 ACQ_EHVI_BOX = 8
 ACQ_FRONT_VALID = 1   # ombo_acq.reserved bit: the EHVI2D stripes form a valid staircase (OMBO_ACQ_FRONT_VALID)
 EHVI_BOX_MAX_BREAKS, EHVI_BOX_MAX_BOXES = 514, 1 << 20
+TOPK_MAX = 65536
 (FIELD_L, FIELD_LINV, FIELD_ALPHA, FIELD_XS, FIELD_STATUS, FIELD_BHI, FIELD_BLO, FIELD_XS32,
  FIELD_ALPHA32) = range(9)
 
@@ -31,6 +32,7 @@ EXPORTS = [
     "ombo_score_host", "ombo_acquire_posterior", "ombo_pool_rows", "ombo_launch_count",
     "ombo_pack_key", "ombo_profile_enable", "ombo_profile_read",
     "ombo_pareto_mask", "ombo_hypervolume", "ombo_cells_2d", "ombo_posterior_joint_samples", "ombo_scalarise",
+    "ombo_score_topk", "ombo_pool_gather",
 ]
 
 
@@ -104,6 +106,9 @@ def lib():
                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ombo_score_host.argtypes = [C.c_void_p, C.POINTER(Gp), C.c_int, C.POINTER(Pool), C.POINTER(Acq),
                                   C.c_int, C.POINTER(Best), C.c_void_p]
+    L.ombo_score_topk.argtypes = [C.c_void_p, C.POINTER(Gp), C.c_int, C.POINTER(Pool), C.POINTER(Acq), C.c_int,
+                                  C.c_int, C.c_void_p, C.c_void_p]
+    L.ombo_pool_gather.argtypes = [C.c_void_p, C.POINTER(Pool), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     L.ombo_acquire_posterior.argtypes = [C.c_void_p, C.POINTER(Acq), C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
                                          C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ombo_scalarise.argtypes = [C.c_void_p, C.POINTER(Acq), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]

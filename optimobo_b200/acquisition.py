@@ -280,9 +280,7 @@ def _models_list(models):
     return [models] if isinstance(models, GPModel) else list(models)
 
 
-def score(models, spec, pool, precision="fp64", want_posterior=False, want_acq=False, want_best=True,
-          var_floor=1e-15, sync=True):
-    """One pass of the hot path over `pool` (K1+K2 per model, K4, K5)."""
+def _checked_models(models, pool):
     models = _models_list(models)
     dev = models[0].device
     for mdl in models:
@@ -292,6 +290,13 @@ def score(models, spec, pool, precision="fp64", want_posterior=False, want_acq=F
             raise ValueError("all models must live on the same device")
     if pool.X is not None and pool.X.device != dev:
         raise ValueError("pool and models are on different devices")
+    return models, dev
+
+
+def score(models, spec, pool, precision="fp64", want_posterior=False, want_acq=False, want_best=True,
+          var_floor=1e-15, sync=True):
+    """One pass of the hot path over `pool` (K1+K2 per model, K4, K5)."""
+    models, dev = _checked_models(models, pool)
     precision = resolve_precision(models, precision)
     G = len(models)
     gps = (_cabi.Gp * G)(*[m.c_struct(var_floor) for m in models])
@@ -429,20 +434,57 @@ def polish(models, spec, starts, lo, hi, max_iter=30, fd_step=1e-5, precision="f
     return best_x, best_v, np.asarray(vals)
 
 
+def score_topk(models, spec, pool, k, precision="fp64", var_floor=1e-15):
+    """The k best candidates of the whole pool by one unpruned scoring pass (`ombo_score_topk`): (values (k,),
+    global indices (k,)) as numpy arrays, values descending, ties to the lowest index, NaN ranked as -inf.  The values
+    are the ones `score(..., want_acq=True)` writes.  Slots beyond pool.m hold (-inf, -1)."""
+    models, dev = _checked_models(models, pool)
+    k = int(k)
+    if not 1 <= k <= _cabi.TOPK_MAX:
+        raise ValueError(f"k must be in 1..{_cabi.TOPK_MAX} (got {k})")
+    if spec.n_models > len(models):
+        raise ValueError(f"acquisition needs {spec.n_models} models, got {len(models)}")
+    precision = resolve_precision(models, precision)
+    G = len(models)
+    gps = (_cabi.Gp * G)(*[m.c_struct(var_floor) for m in models])
+    p = pool.c_struct()
+    a = spec.c_struct(dev)
+    out = torch.empty((k, 2), dtype=torch.int64, device=dev)
+    ctx = _cabi.Context.get(dev.index)
+    with torch.cuda.device(dev):
+        _cabi.check(_cabi.lib().ombo_score_topk(ctx.handle, gps, G, C.byref(p), C.byref(a), _PREC[precision], k,
+                                                C.c_void_p(out.data_ptr()), current_stream_ptr(dev)))
+    host = out.cpu()
+    return host[:, 0].contiguous().view(torch.float64).numpy(), host[:, 1].numpy()
+
+
+def gather_rows(pool, indices, device=None):
+    """Rows of the listed global indices as an explicit pool of the pool's dtype (`ombo_pool_gather`): scoring it
+    reproduces the full pool's values at those indices bit for bit."""
+    dev = pool.X.device if pool.X is not None else _as_device(device)
+    idx = torch.as_tensor(np.asarray(indices, dtype=np.int64), device=dev)
+    out = torch.empty((len(idx), pool.d), dtype=torch.float64, device=dev)
+    ctx = _cabi.Context.get(dev.index)
+    p = pool.c_struct()
+    with torch.cuda.device(dev):
+        _cabi.check(_cabi.lib().ombo_pool_gather(ctx.handle, C.byref(p), C.c_void_p(idx.data_ptr()), len(idx),
+                                                 C.c_void_p(out.data_ptr()), current_stream_ptr(dev)))
+    if pool.X is not None and pool.X.dtype == torch.float32:
+        out = out.to(torch.float32)                      # f32 values, exact in f64 and back
+    return CandidatePool.explicit(out)
+
+
 def top_candidates(models, spec, pool, k, precision="fp64", head=1 << 18):
-    """The k best candidates among the first `head` rows of `pool` (acquisition values materialised for that head only)
-    as (X (k, d) ndarray, values (k,)).  Used to seed `polish` next to the pool winner."""
+    """The k best candidates among the first `head` rows of `pool` (head=None: the whole pool) as (X (k, d) ndarray,
+    values (k,)), by `score_topk`.  Used to seed `polish` next to the pool winner."""
     models = _models_list(models)
     dev = models[0].device
-    m = min(pool.m, head)
-    sub = pool.shard(0, 1)
+    m = pool.m if head is None else min(pool.m, head)
     sub = CandidatePool(m=m, d=pool.d, X=None if pool.X is None else pool.X[:m], lo=pool.lo, hi=pool.hi, seed=pool.seed,
                         index_base=pool.index_base)
-    r = score(models, spec, sub, precision=precision, want_acq=True, want_best=False)
-    acq = torch.nan_to_num(r.acq, nan=-float("inf"))
-    vals, idx = torch.topk(acq, min(k, m))
-    rows = torch.stack([sub.rows(int(i) + pool.index_base, 1, device=dev)[0] for i in idx.cpu()])
-    return rows.cpu().numpy(), vals.cpu().numpy()
+    vals, idx = score_topk(models, spec, sub, min(k, m), precision=precision)
+    rows = torch.stack([sub.rows(int(i), 1, device=dev)[0] for i in idx])
+    return rows.cpu().numpy(), vals
 
 
 def propose(models, spec, pool, precision="fp64", refine_rounds=0, refine_candidates=1 << 14, refine_shrink=0.125,
@@ -484,6 +526,93 @@ def propose(models, spec, pool, precision="fp64", refine_rounds=0, refine_candid
         if vp > float(evaluate(models, spec, x[None, :], precision="fp64")[0]):
             x, best, index = xp, vp, -1
     return x, -best, index
+
+
+# Kriging believer: after believing y = mu(x) at the picked x, no candidate's value rises for these kinds (the mean is
+# unchanged, every variance can only fall, the front / incumbent can only improve and the value is non-decreasing in
+# every sigma), so the top of the last full pass certifies later picks (DESIGN.md section 4, "Batch proposals")
+_CERT_TAU = {"fast": 2e-3, "fp64": 2e-6}      # twice the acquisition contract of each precision mode
+BATCH_SHORTLIST = 4096
+
+
+def _certifiable(spec):
+    return (spec.kind in (_cabi.ACQ_EI, _cabi.ACQ_EHVI_BOX)
+            or (spec.kind == _cabi.ACQ_EHVI2D and spec.semantics == "exact"))
+
+
+def _best_new(vals, idx):
+    """(value, position) of the largest value, NaN as -inf, ties to the lowest global index."""
+    v = np.where(np.isnan(vals), -np.inf, vals)
+    top = v.max()
+    pos = np.flatnonzero(v == top)
+    return top, int(pos[np.argmin(idx[pos])])
+
+
+def propose_batch(models, spec_for, pool, q, precision="fp64", shortlist=BATCH_SHORTLIST):
+    """q proposals from one pool by the Kriging believer: step j believes y = mu(x_{j-1}) (the FP64 mean of the current
+    models), conditions every model on it (`GPModel.with_observations`) and picks the best candidate not selected yet.
+
+    `spec_for(Y_believed)` maps the believed objective rows so far, (j, n_models), to the AcquisitionSpec of step j;
+    `spec_for(empty)` is the ordinary spec.  Step 0 is one `score_topk` pass with k = shortlist.  For EI, exact 2-D EHVI
+    and box EHVI a later step first rescores only that shortlist; its best value certifies the pick when it is at
+    least v_K + tau * v_1 (v_1, v_K: first and K-th values of the last full pass, tau twice the precision mode's
+    acquisition contract), because no value outside the shortlist can have risen above v_K.  Otherwise, and for every
+    other kind, the step runs a full pass with the fantasy models, whose top becomes the new shortlist.  The result
+    is the brute-force Kriging-believer selection either way.
+
+    Returns (X (q, d) ndarray, neg_values (q,), global indices (q,), certified (q,) bool); certified[j] is True when
+    step j was decided by the shortlist alone (never for step 0).  Every point is a pool row."""
+    models = _models_list(models)
+    precision = resolve_precision(models, precision)
+    dev = models[0].device
+    q, K = int(q), int(shortlist)
+    if not 1 <= q <= min(pool.m, _cabi.TOPK_MAX - 1):
+        raise ValueError(f"q must be in 1..min(pool.m, {_cabi.TOPK_MAX - 1}) (got {q}, pool.m={pool.m})")
+    if not 1 <= K <= _cabi.TOPK_MAX:
+        raise ValueError(f"shortlist must be in 1..{_cabi.TOPK_MAX} (got {K})")
+    tau = _CERT_TAU[precision]
+    Y_bel = np.empty((0, len(models)))
+    spec = spec_for(Y_bel)
+    picked, values, certified = [], [], []
+
+    def full_pass():
+        vals, idx = score_topk(models, spec, pool, min(K + len(picked), _cabi.TOPK_MAX), precision=precision)
+        keep = (idx >= 0) & ~np.isin(idx, picked)
+        # every candidate outside the list ranks at or below its last entry (-inf once the list covers the pool)
+        v_last = vals[-1] if idx[-1] >= 0 else -np.inf
+        return vals[keep], idx[keep], vals[0], v_last
+
+    short_v, short_i, v1, vK = full_pass()
+    for j in range(q):
+        if j > 0:
+            x_prev = pool.rows(picked[-1], 1, device=dev)
+            mu, _ = posterior(models, x_prev, precision="fp64")
+            y = mu[:, 0].cpu().numpy()
+            Y_bel = np.vstack([Y_bel, y[None, :]])
+            models = [mdl.with_observations(x_prev, y[g:g + 1]) for g, mdl in enumerate(models)]
+            spec = spec_for(Y_bel)
+            ok = False
+            if _certifiable(spec):
+                live = ~np.isin(short_i, picked)
+                if live.any():
+                    cand = short_i[live]
+                    new = score(models, spec, gather_rows(pool, cand, dev), precision=precision, want_acq=True,
+                                want_best=False).acq.cpu().numpy()
+                    best, pos = _best_new(new, cand)
+                    ok = bool(best >= vK + tau * abs(v1))
+            if ok:
+                pick, value = int(cand[pos]), float(best)
+            else:
+                short_v, short_i, v1, vK = full_pass()
+                pick, value = int(short_i[0]), float(short_v[0])
+        else:
+            ok = False
+            pick, value = int(short_i[0]), float(short_v[0])
+        picked.append(pick)
+        values.append(value)
+        certified.append(ok)
+    X = np.vstack([pool.rows(i, 1, device=dev).cpu().numpy() for i in picked])
+    return X, -np.asarray(values), np.asarray(picked, dtype=np.int64), np.asarray(certified)
 
 
 def propose_host(models, spec, X_host, precision="fp64", index_base=0):

@@ -19,7 +19,7 @@ import numpy as np
 import torch
 
 from .. import device_prep, host_prep
-from ..acquisition import CandidatePool, propose
+from ..acquisition import CandidatePool, propose, propose_batch
 from ..fit import fit_hyperparameters, fit_hyperparameters_device
 from ..gp import GPModel
 
@@ -146,6 +146,24 @@ class PoolOptimiserBase:
                                  score_s=time.perf_counter() - t0, n_candidates=self.n_candidates))
         self._t_fit = self._t_refresh = 0.0
         return x, neg_value
+
+    def _propose_batch(self, models, spec_for, q):
+        """q pool rows by the Kriging believer (acquisition.propose_batch); one timing record for the batch."""
+        t0 = time.perf_counter()
+        pool = CandidatePool.counter(self.n_candidates, self.test_problem.xl, self.test_problem.xu,
+                                     seed=int(self.rng.integers(1, 2 ** 62)))
+        X, neg_values, _, certified = propose_batch(models, spec_for, pool, q, precision=self._precision_for(models))
+        self.timings.append(dict(fit_s=getattr(self, "_t_fit", 0.0), refresh_s=getattr(self, "_t_refresh", 0.0),
+                                 score_s=time.perf_counter() - t0, n_candidates=self.n_candidates, batch=q,
+                                 certified=int(certified.sum())))
+        self._t_fit = self._t_refresh = 0.0
+        return X, neg_values
+
+    @staticmethod
+    def _check_batch_size(batch_size):
+        if int(batch_size) != batch_size or batch_size < 1:
+            raise ValueError(f"batch_size must be a positive integer (got {batch_size!r})")
+        return int(batch_size)
 
     # ---- result ------------------------------------------------------------------------------------
     @staticmethod

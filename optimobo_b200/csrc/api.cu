@@ -112,6 +112,7 @@ int ombo_ctx_destroy(ombo_ctx *c) {
   if (c->prof_dev) cudaFree(c->prof_dev);
   for (int i = 0; i < 2; ++i) if (c->f8_sched[i]) cudaFree(c->f8_sched[i]);
   if (c->ws_prune) cudaFree(c->ws_prune);
+  if (c->ws_topk) cudaFree(c->ws_topk);
   if (c->ws_best) cudaFree(c->ws_best);
   if (c->pinned_best) cudaFreeHost(c->pinned_best);
   cudaStreamDestroy(c->copy_stream);
@@ -172,8 +173,10 @@ int ombo_gp_nlml_grad(ombo_ctx *ctx, const ombo_gp_spec *sp, void *state, double
   return ombo_nlml_grad_impl(ctx, sp, state, out_host, (cudaStream_t)stream);
 }
 
-static int validate_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
-                          int precision) {
+}  // extern "C"
+
+int ombo_validate_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
+                        int precision) {
   OMBO_CHECK(ctx && gps && pool && acq, "score: NULL argument");
   OMBO_CHECK(n_gp >= 1 && n_gp <= OMBO_MAX_GP, "score: n_gp=%d out of range (1..%d)", n_gp, OMBO_MAX_GP);
   OMBO_CHECK(precision == OMBO_PREC_FP64 || precision == OMBO_PREC_FAST, "score: unknown precision %d", precision);
@@ -227,11 +230,10 @@ static void fill_pool_dev(PoolDev &pd, const ombo_pool *pool) {
   }
 }
 
-// scores rows [first, first+count) of the pool; X_dev points at row `first` (or NULL -> generator)
-static int score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const void *X_dev,
-                      long long first, long long count, const ombo_acq *acq, int precision, double *out_mu,
-                      double *out_var, double *out_acq, long long out_ld, ombo_best *best_dev, cudaStream_t s,
-                      int bound_chunks = 0) {
+int ombo_score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const void *X_dev,
+                    long long first, long long count, const ombo_acq *acq, int precision, double *out_mu,
+                    double *out_var, double *out_acq, long long out_ld, ombo_best *best_dev, cudaStream_t s,
+                    int bound_chunks) {
   PoolDev pd;
   fill_pool_dev(pd, pool);
   pd.X = X_dev;
@@ -311,7 +313,7 @@ static int score_passes(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_
   for (long long first = 0; first < pool->m; first += chunk) {
     long long count = pool->m - first < chunk ? pool->m - first : chunk;
     const void *X = pool->X ? (const char *)pool->X + (size_t)first * pool->d * esz : nullptr;
-    int rc = score_pass(ctx, gps, n_gp, pool, X, first, count, acq, precision, out_mu, out_var, out_acq, pool->m,
+    int rc = ombo_score_pass(ctx, gps, n_gp, pool, X, first, count, acq, precision, out_mu, out_var, out_acq, pool->m,
                         best_dev, s, bound_chunks);
     if (rc) return rc;
   }
@@ -468,10 +470,12 @@ static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool
   return OMBO_OK;
 }
 
+extern "C" {
+
 int ombo_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
                int precision, double *out_mu, double *out_var, double *out_acq, ombo_best *best_dev,
                void *stream) {
-  int rc = validate_score(ctx, gps, n_gp, pool, acq, precision);
+  int rc = ombo_validate_score(ctx, gps, n_gp, pool, acq, precision);
   if (rc) return rc;
   OMBO_CHECK((out_mu == nullptr) == (out_var == nullptr), "score: out_mu and out_var must both be given or both NULL");
   OMBO_CUDA(cudaSetDevice(ctx->device));
@@ -487,7 +491,7 @@ int ombo_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *poo
 
 int ombo_score_host(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
                     int precision, ombo_best *best_host, void *stream) {
-  int rc = validate_score(ctx, gps, n_gp, pool, acq, precision);
+  int rc = ombo_validate_score(ctx, gps, n_gp, pool, acq, precision);
   if (rc) return rc;
   OMBO_CHECK(best_host != nullptr, "score_host: best_host is NULL");
   OMBO_CHECK(acq->kind != OMBO_ACQ_NONE, "score_host: needs an acquisition");
@@ -524,7 +528,7 @@ int ombo_score_host(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool
       OMBO_CUDA(cudaStreamWaitEvent(s, ctx->ev_copied[b], 0));
       X = ctx->ws_stage[b];
     }
-    rc = score_pass(ctx, gps, n_gp, pool, X, first, count, acq, precision, nullptr, nullptr, nullptr, 0, best_dev, s);
+    rc = ombo_score_pass(ctx, gps, n_gp, pool, X, first, count, acq, precision, nullptr, nullptr, nullptr, 0, best_dev, s);
     if (rc) return rc;
     if (pool->X) OMBO_CUDA(cudaEventRecord(ctx->ev_consumed[it & 1], s));
   }
@@ -544,7 +548,7 @@ int ombo_acquire_posterior(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const d
   fake.d = 1; fake.m = m;
   ombo_gp gp_ok[OMBO_MAX_GP];
   for (int g = 0; g < n_gp; ++g) { gp_ok[g].state = (const void *)mu; gp_ok[g].d = 1; gp_ok[g].n = 1; }
-  int rc = validate_score(ctx, gp_ok, n_gp, &fake, acq, OMBO_PREC_FP64);
+  int rc = ombo_validate_score(ctx, gp_ok, n_gp, &fake, acq, OMBO_PREC_FP64);
   if (rc) return rc;
   OMBO_CHECK(acq->kind != OMBO_ACQ_NONE, "acquire_posterior: needs an acquisition kind");
   OMBO_CUDA(cudaSetDevice(ctx->device));
@@ -581,6 +585,32 @@ int ombo_pool_rows(ombo_ctx *ctx, const ombo_pool *pool, int64_t index, int64_t 
   pd.X = pool->X;
   long long total = count * pool->d;
   k_pool_rows<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(pd, index - pool->index_base, count, out);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  return OMBO_OK;
+}
+
+__global__ void k_pool_gather(PoolDev pool, const long long *__restrict__ idx, long long count,
+                              double *__restrict__ out) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= count * pool.d) return;
+  out[e] = ombo_pool_coord(pool, idx[e / pool.d] - pool.index_base, (int)(e % pool.d));
+}
+
+int ombo_pool_gather(ombo_ctx *ctx, const ombo_pool *pool, const int64_t *index_dev, int64_t count, double *out,
+                     void *stream) {
+  OMBO_CHECK(ctx && pool && out && (index_dev || count == 0), "pool_gather: NULL argument");
+  OMBO_CHECK(pool->d >= 1 && pool->d <= OMBO_MAX_DIM, "pool_gather: d out of range");
+  OMBO_CHECK(pool->dtype == 0 || pool->dtype == 1, "pool_gather: pool dtype must be 0 (f64) or 1 (f32)");
+  OMBO_CHECK(count >= 0, "pool_gather: negative count");
+  if (count == 0) return OMBO_OK;
+  OMBO_CUDA(cudaSetDevice(ctx->device));
+  PoolDev pd;
+  fill_pool_dev(pd, pool);
+  pd.X = pool->X;
+  const long long total = count * pool->d;
+  k_pool_gather<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(pd, (const long long *)index_dev,
+                                                                                   count, out);
   ctx->launches += 1;
   OMBO_CUDA(cudaGetLastError());
   return OMBO_OK;

@@ -72,6 +72,7 @@ struct ombo_ctx {
   void *ws_partial;   size_t ws_partial_bytes;   // per-block arg-max partials
   void *ws_box;       size_t ws_box_bytes;       // EHVI_BOX boxes as packed 16-bit breakpoint indices
   void *ws_prune;     size_t ws_prune_bytes;     // pruned scoring: per-candidate upper bounds, survivors, cub scratch
+  void *ws_topk;      size_t ws_topk_bytes;      // top-k: one pass's keys, the running k-list, selections, cub scratch
   void *ws_stage[2];  size_t ws_stage_bytes;     // host-entry H2D staging (double buffered)
   void *ws_best;                                  // 16 B device best for the host entry
   ombo_best *pinned_best;                         // pinned host landing zone
@@ -192,6 +193,14 @@ struct FuseAcq {
 };
 
 // ---- internal entry points (one per .cu) ------------------------------------------------
+// api.cu: the argument checks of every scoring entry, and one pass of it: rows [first, first + count) of the pool,
+// X_dev pointing at row `first` (NULL: generator); out_mu / out_var / out_acq are offset by `first`
+int ombo_validate_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const ombo_acq *acq,
+                        int precision);
+int ombo_score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool *pool, const void *X_dev,
+                    long long first, long long count, const ombo_acq *acq, int precision, double *out_mu,
+                    double *out_var, double *out_acq, long long out_ld, ombo_best *best_dev, cudaStream_t s,
+                    int bound_chunks = 0);
 int ombo_refresh_impl(ombo_ctx *ctx, const ombo_gp_spec *spec, void *state, cudaStream_t s);
 int ombo_nlml_grad_impl(ombo_ctx *ctx, const ombo_gp_spec *spec, void *state, double *out_host, cudaStream_t s);
 int ombo_posterior_fp64(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, long long m,

@@ -101,6 +101,16 @@ class GPModel:
         self._flags = (0, 2, 4)[int(st[1])]           # OMBO_GP_FP16_PLANES / OMBO_GP_F8C_PLANES
         return self
 
+    def with_observations(self, X_new, y_new):
+        """A new model with the rows (X_new, y_new) appended: the same hyper-parameters, kernel, noise and jitter
+        policy, refreshed by K3.  This model's X / y are not mutated (Kriging-believer batches condition on
+        y_new = mu(X_new))."""
+        Xn = torch.as_tensor(X_new, dtype=torch.float64).to(self.device).reshape(-1, self.d)
+        yn = torch.as_tensor(y_new, dtype=torch.float64).to(self.device).reshape(-1)
+        return GPModel(torch.cat([self.X, Xn]), torch.cat([self.y, yn]), self.lengthscale, self.variance,
+                       noise=self.noise, jitter=self.jitter, kernel=self.kernel_name, device=self.device,
+                       max_jitter_tries=self.max_jitter_tries)
+
     # fast precision mode keeps sigma within 1e-3 sigma_f while `conditioning` stays below this (measured,
     # scripts/cond_study.py: the error grows from 4e-5 sigma_f at 15 to 2.4e-4 at 4e2, 1e-3 at 4e3-8e3, 1.5e-2 at 4e7)
     FAST_MODE_CONDITIONING_LIMIT = 2.0e3
