@@ -18,7 +18,8 @@
  *                        (expected_decomposition), optimisers.py:325 / parego.py:126 /
  *                        keep.py:118 / cparego.py:450 (EI), cparego.py:486 (consraint_ei),
  *                        keep.py:142 (pareto_expected_improvement), emo.py:192
- *                        (hypervolume_based_PoI)
+ *                        (hypervolume_based_PoI); EHVI_BOX and EHVI_BOX_FEAS have no
+ *                        reference counterpart
  *   scalarisation ids <- optimobo/scalarisations.py:37,53,76,113,153,177,201,222,242,277,314,355
  *
  * Conventions: every function returns an int status (0 = ok, negative = error; the message
@@ -64,7 +65,8 @@ enum {
   OMBO_ACQ_CONSTRAINED_EI = 5,  /* cparego.py:486-496                                     */
   OMBO_ACQ_PARETO_EI = 6,       /* keep.py:142-150 (gp 0 = pareto model, gp 1 = scalar)   */
   OMBO_ACQ_HV_POI = 7,          /* emo.py:192-228                                         */
-  OMBO_ACQ_EHVI_BOX = 8         /* exact EHVI, 2 <= n_obj <= 4, by box decomposition      */
+  OMBO_ACQ_EHVI_BOX = 8,        /* exact EHVI, 2 <= n_obj <= 4, by box decomposition      */
+  OMBO_ACQ_EHVI_BOX_FEAS = 9    /* EHVI_BOX x probability of feasibility (constraint GPs) */
 };
 
 /* OMBO_ACQ_EHVI_BOX: the exact expected hypervolume improvement for k = n_obj independent Gaussian objectives,
@@ -78,7 +80,15 @@ enum {
  *   cells   = DEVICE (n_cells, 2, k) f64 holding integer breakpoint indices: [c][0] upper, [c][1] lower corner,
  *             index 0 = -inf
  * Each model's own variance is used (semantics is ignored).  Limits: 2 <= B <= OMBO_EHVI_BOX_MAX_BREAKS,
- * 1 <= n_cells <= OMBO_EHVI_BOX_MAX_BOXES; indices outside [0, B) are clamped. */
+ * 1 <= n_cells <= OMBO_EHVI_BOX_MAX_BOXES; indices outside [0, B) are clamped.
+ *
+ * OMBO_ACQ_EHVI_BOX_FEAS: constrained EHVI.  Every field as for OMBO_ACQ_EHVI_BOX; in addition GPs 0..k-1 are the
+ * objectives and GPs k..n_gp-1 the c = n_gp - k >= 1 constraint models (a point is feasible when every constraint
+ * is <= 0), and var_eps[k + j] is added to the variance of constraint j:
+ *   EHVI_box(mu_0..k-1, sigma_0..k-1) * prod_j Phi(-mu_{k+j} / sqrt(var_{k+j} + var_eps[k+j])),
+ * the product taken in j order and in FP64 (also in the fast precision mode, so that a pool far on the infeasible
+ * side keeps values below FLT_MIN).  Limits: those of OMBO_ACQ_EHVI_BOX and k + 1 <= n_gp <= OMBO_MAX_GP.  The
+ * scoring entries compute every model's variance for this kind, and never prune or fuse it. */
 #define OMBO_EHVI_BOX_MAX_BREAKS 514        /* a front of up to 512 points */
 #define OMBO_EHVI_BOX_MAX_BOXES  (1 << 20)
 

@@ -171,8 +171,8 @@ class AcquisitionSpec:
 
         if self.stripes is not None:
             a.stripes = up("stripes", self.stripes)
-            # EHVI2D: stripes are (2, P + 2); EHVI_BOX: the (k, B) breakpoint table
-            a.n_pf = self.stripes.shape[1] - (0 if self.kind == _cabi.ACQ_EHVI_BOX else 2)
+            # EHVI2D: stripes are (2, P + 2); EHVI_BOX(_FEAS): the (k, B) breakpoint table
+            a.n_pf = self.stripes.shape[1] - (0 if self.kind in (_cabi.ACQ_EHVI_BOX, _cabi.ACQ_EHVI_BOX_FEAS) else 2)
         if self.cells is not None:
             a.cells = up("cells", self.cells)
             a.n_cells = self.cells.shape[0]
@@ -211,6 +211,25 @@ def spec_ehvi_box(max_point, PF):
     k = len(r)
     return AcquisitionSpec(kind=_cabi.ACQ_EHVI_BOX, n_obj=k, ref=tuple(r), stripes=table,
                            cells=boxes.astype(np.float64), n_models=k)
+
+
+def spec_ehvi_box_feasible(max_point, PF, n_constraints, var_eps=1e-5):
+    """Constrained box EHVI: spec_ehvi_box(max_point, PF) times the probability that every constraint holds,
+    prod_j Phi(-mu_j / sqrt(var_j + var_eps)), with models = k objective GPs followed by `n_constraints` constraint GPs
+    (feasible: every constraint <= 0).  PF is the front of the feasible samples; an empty front scores against the
+    single box [-inf, r].  var_eps defaults to the 1e-5 of the constrained EI's feasibility factor (cparego.py:486-496);
+    0 is allowed.  Not a reference acquisition; `semantics` does not apply."""
+    r = np.asarray(max_point, dtype=np.float64).reshape(-1)
+    k, c = len(r), int(n_constraints)
+    if c != n_constraints or not 1 <= c <= _cabi.MAX_GP - k:
+        raise ValueError(f"n_constraints must be an integer in 1..{_cabi.MAX_GP - k} for {k} objectives "
+                         f"(got {n_constraints!r})")
+    if not var_eps >= 0:
+        raise ValueError(f"var_eps must be >= 0 (got {var_eps!r})")
+    table, boxes = host_prep.ehvi_boxes(np.asarray(PF, dtype=np.float64).reshape(-1, k), r)
+    return AcquisitionSpec(kind=_cabi.ACQ_EHVI_BOX_FEAS, n_obj=k, ref=tuple(r), stripes=table,
+                           cells=boxes.astype(np.float64), var_eps=(0.0,) * k + (float(var_eps),) * c,
+                           n_models=k + c)
 
 
 def spec_expected_decomposition(weights, agg_func, agg_function_min, cache, semantics="reference"):
@@ -535,6 +554,7 @@ _CERT_TAU = {"fast": 2e-3, "fp64": 2e-6}      # twice the acquisition contract o
 BATCH_SHORTLIST = 4096
 
 
+# EHVI_BOX_FEAS is not: the probability of feasibility rises where a constraint's sigma falls with its mean above 0
 def _certifiable(spec):
     return (spec.kind in (_cabi.ACQ_EI, _cabi.ACQ_EHVI_BOX)
             or (spec.kind == _cabi.ACQ_EHVI2D and spec.semantics == "exact"))
@@ -662,6 +682,12 @@ def EHVI_3D(X, models, max_point, PF, cache, semantics="reference", precision="f
 
 def EHVI_box(X, models, max_point, PF, precision="fp64"):
     return evaluate(models, spec_ehvi_box(max_point, PF), X, precision)
+
+
+def EHVI_box_feasible(X, models, constraint_models, max_point, PF, precision="fp64"):
+    models = list(_models_list(models)) + list(constraint_models)
+    k = len(np.asarray(max_point).reshape(-1))
+    return evaluate(models, spec_ehvi_box_feasible(max_point, PF, len(models) - k), X, precision)
 
 
 def expected_decomposition(X, models, weights, agg_func, agg_function_min, cache, semantics="reference",

@@ -5,7 +5,8 @@ from __future__ import annotations
 import numpy as np
 
 from .. import host_prep, result
-from ..acquisition import spec_ehvi, spec_ehvi3d, spec_ehvi_box, spec_ei, spec_expected_decomposition
+from ..acquisition import (spec_ehvi, spec_ehvi3d, spec_ehvi_box, spec_ehvi_box_feasible, spec_ei,
+                           spec_expected_decomposition)
 from .base import PoolOptimiserBase
 
 
@@ -19,11 +20,32 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
 
     Additive knob `batch_size` (default 1: one point per iteration, the reference's loop): q > 1 proposes q pool
     rows per iteration by the Kriging believer (`propose_batch`) and evaluates them all; `budget` then counts the
-    evaluations after the initial design."""
+    evaluations after the initial design.
 
-    def __init__(self, test_problem, *args, ehvi="reference", batch_size=1, **kwargs):
+    Additive knob `constrained` (default False: the objectives alone, as above): True optimises a problem with
+    inequality constraints (feasible: every constraint <= 0).  One GP per objective and per constraint is fitted, and
+    the acquisition is the box EHVI over the front of the feasible samples times the probability that every
+    constraint holds (`spec_ehvi_box_feasible`); with no feasible sample yet the front is empty.  It needs
+    ehvi="box", no `acquisition_func`, no equality constraints and n_obj + n_ieq_constr <= 8.  The hypervolume
+    history counts the feasible samples only (0 while there are none), and `solve` returns a `Constrained_Res` with
+    the constraint values in `gsample`."""
+
+    def __init__(self, test_problem, *args, ehvi="reference", batch_size=1, constrained=False, **kwargs):
         if ehvi not in ("reference", "box"):
             raise ValueError(f"ehvi must be 'reference' or 'box' (got {ehvi!r})")
+        self.constrained = bool(constrained)
+        if self.constrained:
+            n_ieq = int(getattr(test_problem, "n_ieq_constr", 0))
+            if ehvi != "box":
+                raise ValueError("constrained=True scores with the constrained box EHVI: pass ehvi='box'")
+            if int(getattr(test_problem, "n_eq_constr", 0)) != 0:
+                raise ValueError("constrained=True takes inequality constraints only (the problem has "
+                                 f"n_eq_constr={test_problem.n_eq_constr})")
+            if n_ieq < 1:
+                raise ValueError("constrained=True needs a problem with at least one inequality constraint")
+            if test_problem.n_obj + n_ieq > 8:
+                raise ValueError(f"constrained=True supports n_obj + n_ieq_constr <= 8 models (got "
+                                 f"{test_problem.n_obj} + {n_ieq})")
         super().__init__(test_problem, *args, **kwargs)
         self.ehvi = ehvi
         self.batch_size = self._check_batch_size(batch_size)
@@ -32,6 +54,10 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
         return host_prep.cached_samples(dimensions, sample_exponent, seed=int(self.rng.integers(0, 2 ** 31)))
 
     def solve(self, budget=100, n_init_samples=5, sample_exponent=5, acquisition_func=None):
+        if self.constrained:
+            if acquisition_func is not None:
+                raise ValueError("constrained=True scores with the constrained box EHVI; acquisition_func must be None")
+            return self._solve_constrained(budget, n_init_samples)
         if self.batch_size > 1:
             return self._solve_batched(budget, n_init_samples, sample_exponent, acquisition_func)
         problem = self.test_problem
@@ -115,6 +141,60 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
         mask = self._pareto_members(ysample)
         res = result.Res(ysample[mask], Xsample[mask], ysample, Xsample, hypervolume_convergence, problem.n_obj,
                          n_init_samples)
+        res.timings = self.timings
+        return res
+
+
+    def _constrained_spec_for(self, pf):
+        """spec_for(Y_believed) of one constrained batch: a believed row (objectives, then constraints) joins the
+        feasible front only when every believed constraint is <= 0 and its objectives are inside max_point."""
+        max_point = np.array(self.max_point, dtype=float)
+        k, c = self.n_obj, self.test_problem.n_ieq_constr
+
+        def spec_for(Y_bel):
+            Y = np.asarray(Y_bel, dtype=float).reshape(-1, k + c)
+            ok = Y[np.all(Y[:, k:] <= 0, axis=1) & np.all(Y[:, :k] <= max_point, axis=1), :k]
+            front = self._calc_pf(np.vstack([pf, ok])) if len(ok) else pf
+            return spec_ehvi_box_feasible(max_point, front, c)
+
+        return spec_for
+
+    def _solve_constrained(self, budget, n_init_samples):
+        problem = self.test_problem
+        k, c = problem.n_obj, problem.n_ieq_constr
+        Xsample, ysample = self._initial_design(n_init_samples)
+        gsample = np.asarray([self._constraint_function(problem, x) for x in Xsample]).reshape(-1, c)
+        hypervolume_convergence = []
+        done = 0
+        while done < budget:
+            q = min(self.batch_size, budget - done)
+            self._update_bounds(ysample)
+            y_feasible = ysample[np.all(gsample <= 0, axis=1)]
+            hypervolume_convergence.append(self._hypervolume(y_feasible) if len(y_feasible) else 0.0)
+            models = self._fit_models(Xsample, [ysample[:, i] for i in range(k)] + [gsample[:, j] for j in range(c)])
+            pf = self._calc_pf(y_feasible) if len(y_feasible) else np.empty((0, k))
+            if self.batch_size == 1:
+                X_next, _ = self._propose(models, spec_ehvi_box_feasible(self.max_point, pf, c))
+                X_next = np.atleast_2d(X_next)
+            else:
+                X_next, _ = self._propose_batch(models, self._constrained_spec_for(pf), q)
+            y_next = np.asarray([self._objective_function(problem, x) for x in X_next]).reshape(q, k)
+            g_next = np.asarray([self._constraint_function(problem, x) for x in X_next]).reshape(q, c)
+            ysample = np.vstack((ysample, y_next))
+            Xsample = np.vstack((Xsample, X_next))
+            gsample = np.vstack((gsample, g_next))
+            done += q
+        infeasible = np.any(gsample > 0, axis=1)
+        y_feasible, y_infeasible = ysample[~infeasible], ysample[infeasible]
+        X_feasible, X_infeasible = Xsample[~infeasible], Xsample[infeasible]
+        if len(y_feasible):
+            mask = self._pareto_members(y_feasible)
+            pf_approx, pf_inputs = y_feasible[mask], X_feasible[mask]
+        else:
+            pf_approx, pf_inputs = y_feasible, X_feasible
+        res = result.Constrained_Res(y_infeasible, y_feasible, X_infeasible, X_feasible, pf_approx, pf_inputs, ysample,
+                                     Xsample, hypervolume_convergence, k, n_init_samples)
+        res.gsample = gsample
         res.timings = self.timings
         return res
 

@@ -11,6 +11,7 @@
 //   PARETO_EI         keep.py:142-150
 //   HV_POI            emo.py:176-228
 //   EHVI_BOX          not in the reference: the exact k-objective EHVI over a box decomposition (k_acquire_box)
+//   EHVI_BOX_FEAS     not in the reference: EHVI_BOX times the probability of feasibility of CONSTRAINED_EI
 // Arg-max replaces the inner optimiser call sites (differential_evolution at optimisers.py:87,
 // :118,:366; cparego.py:94,:544; emo.py:240; EA loops parego.py:242-270, keep.py:260-292):
 // warp shuffle -> block (smem) -> per-block partial -> one final block; ties resolve to the
@@ -348,20 +349,25 @@ __device__ __forceinline__ float shortfall_tail(float s, float az, float) { retu
 // odd candidate stride of V (in elements): the groups of one warp read the same box from different banks
 __host__ __device__ inline int box_cand_stride(int k, int B) { return (k * B) | 1; }
 
+// feas: OMBO_ACQ_EHVI_BOX_FEAS adds the (tile,) f64 feasibility products
 template <typename T>
-__host__ __device__ inline size_t box_smem_bytes(int k, int B, int tile) {
+__host__ __device__ inline size_t box_smem_bytes(int k, int B, int tile, bool feas = false) {
   return (size_t)BOX_CHUNK * 16 + (size_t)k * B * sizeof(T) + (size_t)tile * k * (3 * sizeof(T) + 4) +
-         (size_t)tile * box_cand_stride(k, B) * sizeof(T);
+         (size_t)tile * box_cand_stride(k, B) * sizeof(T) + (feas ? (size_t)tile * 8 : 0);
 }
 
-template <typename T, int K>
+// FEAS (OMBO_ACQ_EHVI_BOX_FEAS): GPs K..n_gp-1 are constraint models, and the value is the box sum times the
+// probability of feasibility prod_j Phi(-mu_j / sqrt(var_j + var_eps[j])), formed in FP64 exactly as the
+// constrained EI forms it (k_acquire), once per candidate in the prologue
+template <typename T, int K, bool FEAS>
 __global__ void __launch_bounds__(ACQ_THREADS)
 k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double *__restrict__ var, long long m,
               long long ld, long long index_base, const uint4 *__restrict__ boxes, double *__restrict__ out_acq,
-              ombo_best *__restrict__ partials) {
+              ombo_best *__restrict__ partials, int n_gp) {
   const int B = a.n_pf, n_boxes = a.n_cells, G = ACQ_THREADS / tile, cs = box_cand_stride(K, B);
   uint4 *bx = reinterpret_cast<uint4 *>(acq_smem);                  // BOX_CHUNK staged boxes
-  T *V = reinterpret_cast<T *>(bx + BOX_CHUNK);                     // (tile, cs)
+  double *pof = reinterpret_cast<double *>(bx + BOX_CHUNK);         // FEAS: (tile,) feasibility products
+  T *V = reinterpret_cast<T *>(pof + (FEAS ? tile : 0));            // (tile, cs)
   T *tr = V + tile * cs;                                            // (K, B) breakpoints t - r
   T *sd = tr + K * B;                                               // (tile, K) sigma
   T *rsd = sd + tile * K;                                           // (tile, K) 1 / sigma
@@ -381,6 +387,15 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
     shift[e] = (T)(a.stripes[i * B + B - 1] - mv);
     split[e] = B;                                                   // mu above every breakpoint
   }
+  if (FEAS)
+    for (int j = threadIdx.x; j < tile; j += ACQ_THREADS) {
+      const long long c = c0 + j;
+      double p = 1;           // a mostly infeasible pool is a product of small probabilities: accumulated in FP64
+      if (c < m)
+        for (int g = K; g < n_gp; ++g)
+          p *= Phi_wide(((T)0 - (T)mu[g * ld + c]) / sqrt_t((T)var[g * ld + c] + (T)a.var_eps[g]));
+      pof[j] = p;
+    }
   __syncthreads();
   // phase 1: the V table
   for (int e = threadIdx.x; e < tile * K * B; e += ACQ_THREADS) {
@@ -438,8 +453,14 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
   if (owner) {
     T sum = 0;
     for (int g = 0; g < G; ++g) sum += red[g * tile + threadIdx.x];
-    if (out_acq) out_acq[c0 + threadIdx.x] = (double)sum;
-    val = isnan(sum) ? -INFINITY : (double)sum;
+    if (FEAS) {
+      const double v = (double)sum * pof[threadIdx.x];
+      if (out_acq) out_acq[c0 + threadIdx.x] = v;
+      val = isnan(v) ? -INFINITY : v;
+    } else {
+      if (out_acq) out_acq[c0 + threadIdx.x] = (double)sum;
+      val = isnan(sum) ? -INFINITY : (double)sum;
+    }
   }
   // ---- K5: block arg-max ----
   BestPair bb;
@@ -461,31 +482,45 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
 
 // the largest tile whose shared memory leaves room for two CTAs per SM, else the largest that fits at all
 template <typename T>
-static int box_tile(int k, int B) {
-  for (int t = 32; t >= 8; t >>= 1) if (box_smem_bytes<T>(k, B, t) <= 110 * 1024) return t;
-  return box_smem_bytes<T>(k, B, 8) <= 220 * 1024 ? 8 : 0;          // + the static arg-max slots, under 227 KB
+static int box_tile(int k, int B, bool feas) {
+  for (int t = 32; t >= 8; t >>= 1) if (box_smem_bytes<T>(k, B, t, feas) <= 110 * 1024) return t;
+  return box_smem_bytes<T>(k, B, 8, feas) <= 220 * 1024 ? 8 : 0;    // + the static arg-max slots, under 227 KB
 }
 
-template <typename T, int K>
-static int launch_box(ombo_ctx *ctx, const ombo_acq *acq, const double *mu, const double *var, long long m,
+template <typename T, int K, bool FEAS>
+static int launch_box(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var, long long m,
                       long long ld, long long index_base, double *out_acq, cudaStream_t s) {
-  const int tile = box_tile<T>(K, acq->n_pf);
+  const int tile = box_tile<T>(K, acq->n_pf, FEAS);
   OMBO_CHECK(tile > 0, "EHVI_BOX: %d breakpoints x %d objectives do not fit in shared memory", acq->n_pf, K);
-  const size_t smem = box_smem_bytes<T>(K, acq->n_pf, tile);
+  const size_t smem = box_smem_bytes<T>(K, acq->n_pf, tile, FEAS);
   if (smem > 48 * 1024)
-    OMBO_CUDA(cudaFuncSetAttribute(k_acquire_box<T, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    OMBO_CUDA(cudaFuncSetAttribute(k_acquire_box<T, K, FEAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long blocks = (m + tile - 1) / tile;
   int rc = ombo_ws_reserve(&ctx->ws_partial, &ctx->ws_partial_bytes, (size_t)blocks * sizeof(ombo_best));
   if (rc) return rc;
-  k_acquire_box<T, K><<<(unsigned)blocks, ACQ_THREADS, smem, s>>>(*acq, tile, mu, var, m, ld, index_base,
-                                                                  (const uint4 *)ctx->ws_box, out_acq,
-                                                                  (ombo_best *)ctx->ws_partial);
+  k_acquire_box<T, K, FEAS><<<(unsigned)blocks, ACQ_THREADS, smem, s>>>(*acq, tile, mu, var, m, ld, index_base,
+                                                                        (const uint4 *)ctx->ws_box, out_acq,
+                                                                        (ombo_best *)ctx->ws_partial, n_gp);
   ctx->launches += 1;
   return (int)blocks;
 }
 
-static int ombo_acquire_box(ombo_ctx *ctx, const ombo_acq *acq, const double *mu, const double *var, long long m,
-                            long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
+template <bool FEAS>
+static int launch_box_k(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var,
+                        long long m, long long ld, long long index_base, double *out_acq, cudaStream_t s, bool fp32) {
+  switch (acq->n_obj) {
+    case 2: return fp32 ? launch_box<float, 2, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
+                        : launch_box<double, 2, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
+    case 3: return fp32 ? launch_box<float, 3, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
+                        : launch_box<double, 3, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
+    default: return fp32 ? launch_box<float, 4, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
+                         : launch_box<double, 4, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
+  }
+}
+
+// OMBO_ACQ_EHVI_BOX and OMBO_ACQ_EHVI_BOX_FEAS
+static int ombo_acquire_box(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var,
+                            long long m, long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
                             cudaStream_t s, bool fp32) {
   const int k = acq->n_obj;
   int rc = ombo_ws_reserve(&ctx->ws_box, &ctx->ws_box_bytes, (size_t)acq->n_cells * sizeof(uint4));
@@ -494,13 +529,9 @@ static int ombo_acquire_box(ombo_ctx *ctx, const ombo_acq *acq, const double *mu
                                                           (uint4 *)ctx->ws_box);
   ctx->launches += 1;
   fp32 = fp32 && !ctx->knobs.acq_fp64;
-  int blocks;
-  if (k == 2) blocks = fp32 ? launch_box<float, 2>(ctx, acq, mu, var, m, ld, index_base, out_acq, s)
-                            : launch_box<double, 2>(ctx, acq, mu, var, m, ld, index_base, out_acq, s);
-  else if (k == 3) blocks = fp32 ? launch_box<float, 3>(ctx, acq, mu, var, m, ld, index_base, out_acq, s)
-                                 : launch_box<double, 3>(ctx, acq, mu, var, m, ld, index_base, out_acq, s);
-  else blocks = fp32 ? launch_box<float, 4>(ctx, acq, mu, var, m, ld, index_base, out_acq, s)
-                     : launch_box<double, 4>(ctx, acq, mu, var, m, ld, index_base, out_acq, s);
+  const int blocks = acq->kind == OMBO_ACQ_EHVI_BOX_FEAS
+                         ? launch_box_k<true>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32)
+                         : launch_box_k<false>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32);
   if (blocks < 0) return blocks;
   if (best_dev) {
     k_argmax_final<<<1, 1024, 0, s>>>((const ombo_best *)ctx->ws_partial, blocks, best_dev);
@@ -514,8 +545,8 @@ int ombo_acquire(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu,
                  long long m, long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
                  cudaStream_t s, bool fp32) {
   if (m <= 0) return OMBO_OK;
-  if (acq->kind == OMBO_ACQ_EHVI_BOX)
-    return ombo_acquire_box(ctx, acq, mu, var, m, ld, index_base, out_acq, best_dev, s, fp32);
+  if (acq->kind == OMBO_ACQ_EHVI_BOX || acq->kind == OMBO_ACQ_EHVI_BOX_FEAS)
+    return ombo_acquire_box(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, best_dev, s, fp32);
   int n_stage = 0;
   if (acq->kind == OMBO_ACQ_EHVI2D) n_stage = 2 * (acq->n_pf + 2);
   else if (acq->kind == OMBO_ACQ_HV_POI) n_stage = acq->n_cells * 2 * acq->n_obj;
