@@ -44,6 +44,7 @@ extern "C" {
 #define OMBO_ERR_NOT_PD      -2   /* K + (sigma_n2 + jitter) I not positive definite */
 #define OMBO_ERR_CUDA        -3
 #define OMBO_ERR_UNSUPPORTED -4
+#define OMBO_ERR_SPACE       -5   /* an output buffer is too small; the call reported the size it needs */
 
 #define OMBO_MAX_GP   8
 #define OMBO_MAX_OBJ  4
@@ -276,6 +277,22 @@ int ombo_hypervolume(ombo_ctx *ctx, const double *P, int p, int k, const double 
                      void *stream);
 int ombo_cells_2d(ombo_ctx *ctx, const double *PF, int p, const double *ideal, const double *maxp,
                   double *cells, void *stream);
+
+/* ombo_ehvi_boxes: the breakpoint table and boxes OMBO_ACQ_EHVI_BOX / OMBO_ACQ_EHVI_BOX_FEAS score against, defined by
+ *   host_prep.ehvi_boxes (optimobo_b200/host_prep.py) and equal to it element for element and in its order, so a spec
+ *   built from either scores bit-identically.  Rows of PF (p, k) that are not <= ref (NaN rows included) are dropped,
+ *   the first front is taken and duplicate rows are removed.
+ *   PF     DEVICE (p, k) f64, 0 <= p <= 16384, 2 <= k <= 4;  ref HOST k finite doubles
+ *   table  DEVICE room for k * (p + 2) doubles: written as the contiguous (k, B) table (the spec's `stripes`)
+ *   boxes  DEVICE room for boxes_cap * 2 * k doubles: written as (n_boxes, 2, k) breakpoint indices (the spec's `cells`)
+ *   B_out, n_boxes_out  HOST: B and n_boxes, reported whenever the front is accepted.
+ * Synchronises `stream` once.  Returns OMBO_ERR_SPACE, writing neither table nor boxes, when n_boxes > boxes_cap (call
+ * again with a buffer of n_boxes_out); OMBO_ERR_UNSUPPORTED when the front has more than
+ * OMBO_EHVI_BOX_MAX_BREAKS - 2 = 512 distinct points inside ref; OMBO_ERR_INVALID when a row inside ref has a -inf
+ * coordinate, or when B > OMBO_EHVI_BOX_MAX_BREAKS or n_boxes > OMBO_EHVI_BOX_MAX_BOXES (what ombo_score would
+ * reject). */
+int ombo_ehvi_boxes(ombo_ctx *ctx, const double *PF, int p, int k, const double *ref, double *table, double *boxes,
+                    int64_t boxes_cap, int *B_out, int64_t *n_boxes_out, void *stream);
 
 /* ---- joint posterior samples (SURVEY.md section 8f rank 4) --------------------------------------------
  * The device side of TuRBO's Thompson sampling, `GP.posterior_samples(X_cand, size=batch_size)`

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "liboptimobo_b200.so")
 
-OK, ERR_INVALID, ERR_NOT_PD, ERR_CUDA, ERR_UNSUPPORTED = 0, -1, -2, -3, -4
+OK, ERR_INVALID, ERR_NOT_PD, ERR_CUDA, ERR_UNSUPPORTED, ERR_SPACE = 0, -1, -2, -3, -4, -5
 MAX_GP, MAX_OBJ, MAX_DIM, MAX_TRAIN = 8, 4, 32, 8192
 
 KERNEL_MATERN52, KERNEL_RBF = 0, 1
@@ -33,7 +33,7 @@ EXPORTS = [
     "ombo_score_host", "ombo_acquire_posterior", "ombo_pool_rows", "ombo_launch_count",
     "ombo_pack_key", "ombo_profile_enable", "ombo_profile_read",
     "ombo_pareto_mask", "ombo_hypervolume", "ombo_cells_2d", "ombo_posterior_joint_samples", "ombo_scalarise",
-    "ombo_score_topk", "ombo_pool_gather",
+    "ombo_score_topk", "ombo_pool_gather", "ombo_ehvi_boxes",
 ]
 
 
@@ -120,6 +120,8 @@ def lib():
                                    C.c_void_p]
     L.ombo_cells_2d.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                 C.c_void_p, C.c_void_p]
+    L.ombo_ehvi_boxes.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_double), C.c_void_p,
+                                  C.c_void_p, C.c_int64, C.POINTER(C.c_int), C.POINTER(C.c_int64), C.c_void_p]
     L.ombo_posterior_joint_samples.argtypes = [C.c_void_p, C.POINTER(Gp), C.c_void_p, C.c_int, C.c_void_p, C.c_int,
                                                C.c_double, C.c_void_p, C.c_void_p]
     L.ombo_profile_enable.argtypes = [C.c_void_p, C.c_int]

@@ -164,9 +164,13 @@ class AcquisitionSpec:
         a.reserved = self.reserved
 
         def up(name, arr):
+            if (torch.is_tensor(arr) and arr.device == torch.device(device) and arr.dtype == torch.float64
+                    and arr.is_contiguous()):
+                return arr.data_ptr()                   # already where the kernels read it: no copy
             key = (name, str(device))
             if key not in self._dev:
-                self._dev[key] = torch.as_tensor(np.ascontiguousarray(arr, dtype=np.float64)).to(device)
+                self._dev[key] = (arr.to(device=device, dtype=torch.float64).contiguous() if torch.is_tensor(arr) else
+                                  torch.as_tensor(np.ascontiguousarray(arr, dtype=np.float64)).to(device))
             return self._dev[key].data_ptr()
 
         if self.stripes is not None:
@@ -202,23 +206,33 @@ def spec_ehvi3d(max_point, PF, cache, semantics="reference"):
                            best=host_prep.hypervolume(PF, max_point), cache=cache, n_models=k)
 
 
-def spec_ehvi_box(max_point, PF):
+def _box_tables(PF, r, device):
+    """(table, boxes as float64) of the box decomposition: host_prep.ehvi_boxes as numpy arrays, or with a device its
+    device twin (device_prep.ehvi_boxes, equal element for element) as tensors on that device."""
+    if device is not None:
+        from . import device_prep
+        return device_prep.ehvi_boxes(PF, r, device)
+    table, boxes = host_prep.ehvi_boxes(PF, r)
+    return table, boxes.astype(np.float64)
+
+
+def spec_ehvi_box(max_point, PF, device=None):
     """Exact expected hypervolume improvement for 2 <= k <= 4 objectives: sum over the disjoint boxes of the region
     no front point dominates (host_prep.ehvi_boxes) of prod_i (H_i(u_i) - H_i(l_i)), H_i(t) = E[(t - y_i)^+], with each
-    model's own mean and variance.  Not a reference acquisition; `semantics` does not apply."""
+    model's own mean and variance.  Not a reference acquisition; `semantics` does not apply.  With `device`, the
+    decomposition is built there (device_prep.ehvi_boxes) and the spec holds its device tensors."""
     r = np.asarray(max_point, dtype=np.float64).reshape(-1)
-    table, boxes = host_prep.ehvi_boxes(PF, r)
+    table, boxes = _box_tables(PF, r, device)
     k = len(r)
-    return AcquisitionSpec(kind=_cabi.ACQ_EHVI_BOX, n_obj=k, ref=tuple(r), stripes=table,
-                           cells=boxes.astype(np.float64), n_models=k)
+    return AcquisitionSpec(kind=_cabi.ACQ_EHVI_BOX, n_obj=k, ref=tuple(r), stripes=table, cells=boxes, n_models=k)
 
 
-def spec_ehvi_box_feasible(max_point, PF, n_constraints, var_eps=1e-5):
+def spec_ehvi_box_feasible(max_point, PF, n_constraints, var_eps=1e-5, device=None):
     """Constrained box EHVI: spec_ehvi_box(max_point, PF) times the probability that every constraint holds,
     prod_j Phi(-mu_j / sqrt(var_j + var_eps)), with models = k objective GPs followed by `n_constraints` constraint GPs
     (feasible: every constraint <= 0).  PF is the front of the feasible samples; an empty front scores against the
     single box [-inf, r].  var_eps defaults to the 1e-5 of the constrained EI's feasibility factor (cparego.py:486-496);
-    0 is allowed.  Not a reference acquisition; `semantics` does not apply."""
+    0 is allowed.  Not a reference acquisition; `semantics` does not apply.  `device` as for spec_ehvi_box."""
     r = np.asarray(max_point, dtype=np.float64).reshape(-1)
     k, c = len(r), int(n_constraints)
     if c != n_constraints or not 1 <= c <= _cabi.MAX_GP - k:
@@ -226,9 +240,9 @@ def spec_ehvi_box_feasible(max_point, PF, n_constraints, var_eps=1e-5):
                          f"(got {n_constraints!r})")
     if not var_eps >= 0:
         raise ValueError(f"var_eps must be >= 0 (got {var_eps!r})")
-    table, boxes = host_prep.ehvi_boxes(np.asarray(PF, dtype=np.float64).reshape(-1, k), r)
+    table, boxes = _box_tables(np.asarray(PF, dtype=np.float64).reshape(-1, k), r, device)
     return AcquisitionSpec(kind=_cabi.ACQ_EHVI_BOX_FEAS, n_obj=k, ref=tuple(r), stripes=table,
-                           cells=boxes.astype(np.float64), var_eps=(0.0,) * k + (float(var_eps),) * c,
+                           cells=boxes, var_eps=(0.0,) * k + (float(var_eps),) * c,
                            n_models=k + c)
 
 

@@ -48,7 +48,8 @@ class PoolOptimiserBase:
         self.fit_on_device = fit_on_device       # likelihood + gradient on the GPU (ombo_gp_nlml_grad)
         self.refine_rounds = refine_rounds       # zoom rounds around the pool winner (DE's polish step)
         # first front / hypervolume / cells on the device (bit-identical to host_prep; "auto": once the sample
-        # holds >= 512 rows, where the O(n^2) host versions start to show next to a ~100 ms scoring pass)
+        # holds >= 512 rows, where the O(n^2) host versions start to show next to a ~100 ms scoring pass); the box
+        # decomposition of ehvi="box" follows its own rule (MultiSurrogateOptimiser._box_device)
         self.prep_on_device = prep_on_device
         self.timings = []
 

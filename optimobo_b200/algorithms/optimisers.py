@@ -10,13 +10,20 @@ from ..acquisition import (spec_ehvi, spec_ehvi3d, spec_ehvi_box, spec_ehvi_box_
 from .base import PoolOptimiserBase
 
 
+# "auto" builds the box decomposition on the device from this front size on: on the B200 the device is faster at every
+# front size measured, and from 16 points the host takes 4.6x (k = 3) to 24x (k = 4) its time (DESIGN.md section 4)
+BOX_DEVICE_MIN_FRONT = 16
+BOX_DEVICE_MAX_FRONT = 512      # ombo_ehvi_boxes takes fronts of up to 512 distinct points
+
+
 class MultiSurrogateOptimiser(PoolOptimiserBase):
     """One GP per objective; default acquisition 2-D EHVI (crude 3-D EHVI for 3 objectives), or the
     expected improvement over a scalarisation when `acquisition_func` is given
     (optimisers.py:144-277).
 
     Additive knob `ehvi`: "reference" (default) keeps the reference's EHVI / crude 3-D EHVI above; "box" scores
-    every 2 to 4 objective problem with the exact EHVI over the box decomposition (`spec_ehvi_box`).
+    every 2 to 4 objective problem with the exact EHVI over the box decomposition (`spec_ehvi_box`), built on the
+    device or the host as `prep_on_device` selects (`_box_device`); both give the same boxes.
 
     Additive knob `batch_size` (default 1: one point per iteration, the reference's loop): q > 1 proposes q pool
     rows per iteration by the Kriging believer (`propose_batch`) and evaluates them all; `budget` then counts the
@@ -50,6 +57,21 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
         self.ehvi = ehvi
         self.batch_size = self._check_batch_size(batch_size)
 
+    def _box_device(self, front):
+        """Where the box decomposition of `front` is built: self.device when prep_on_device is True (or "auto" and the
+        front has at least BOX_DEVICE_MIN_FRONT rows) and the front is finite and within the device limit, else None
+        (the host)."""
+        front = np.asarray(front, dtype=float)
+        n = len(front)
+        if self.prep_on_device is True:
+            wanted = True
+        elif self.prep_on_device == "auto":
+            wanted = n >= BOX_DEVICE_MIN_FRONT
+        else:
+            wanted = False
+        ok = n <= BOX_DEVICE_MAX_FRONT and bool(np.all(np.isfinite(front)))
+        return self.device if wanted and ok else None
+
     def _get_cached_samples(self, dimensions, sample_exponent):
         return host_prep.cached_samples(dimensions, sample_exponent, seed=int(self.rng.integers(0, 2 ** 31)))
 
@@ -73,7 +95,7 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
             if acquisition_func is None:
                 pf = self._calc_pf(ysample)
                 if self.ehvi == "box":
-                    spec = spec_ehvi_box(self.max_point, pf)
+                    spec = spec_ehvi_box(self.max_point, pf, device=self._box_device(pf))
                 elif problem.n_obj == 2:
                     spec = spec_ehvi(self.max_point, pf, cached_samples, self.semantics)
                 else:
@@ -108,7 +130,7 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
             inside = inside[np.all(inside <= max_point, axis=1)]
             front = self._calc_pf(np.vstack([pf, inside])) if len(inside) else pf
             if self.ehvi == "box":
-                return spec_ehvi_box(max_point, front)
+                return spec_ehvi_box(max_point, front, device=self._box_device(front))
             if self.n_obj == 2:
                 return spec_ehvi(max_point, front, cached_samples, self.semantics)
             return spec_ehvi3d(max_point, front, cached_samples, self.semantics)
@@ -155,7 +177,7 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
             Y = np.asarray(Y_bel, dtype=float).reshape(-1, k + c)
             ok = Y[np.all(Y[:, k:] <= 0, axis=1) & np.all(Y[:, :k] <= max_point, axis=1), :k]
             front = self._calc_pf(np.vstack([pf, ok])) if len(ok) else pf
-            return spec_ehvi_box_feasible(max_point, front, c)
+            return spec_ehvi_box_feasible(max_point, front, c, device=self._box_device(front))
 
         return spec_for
 
@@ -174,7 +196,8 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
             models = self._fit_models(Xsample, [ysample[:, i] for i in range(k)] + [gsample[:, j] for j in range(c)])
             pf = self._calc_pf(y_feasible) if len(y_feasible) else np.empty((0, k))
             if self.batch_size == 1:
-                X_next, _ = self._propose(models, spec_ehvi_box_feasible(self.max_point, pf, c))
+                X_next, _ = self._propose(models, spec_ehvi_box_feasible(self.max_point, pf, c,
+                                                                         device=self._box_device(pf)))
                 X_next = np.atleast_2d(X_next)
             else:
                 X_next, _ = self._propose_batch(models, self._constrained_spec_for(pf), q)

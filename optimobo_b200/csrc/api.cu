@@ -113,6 +113,7 @@ int ombo_ctx_destroy(ombo_ctx *c) {
   for (int i = 0; i < 2; ++i) if (c->f8_sched[i]) cudaFree(c->f8_sched[i]);
   if (c->ws_prune) cudaFree(c->ws_prune);
   if (c->ws_topk) cudaFree(c->ws_topk);
+  if (c->ws_boxprep) cudaFree(c->ws_boxprep);
   if (c->ws_best) cudaFree(c->ws_best);
   if (c->pinned_best) cudaFreeHost(c->pinned_best);
   cudaStreamDestroy(c->copy_stream);
@@ -647,6 +648,21 @@ int ombo_cells_2d(ombo_ctx *ctx, const double *PF, int p, const double *ideal, c
   OMBO_CHECK(p >= 1 && p <= 16384, "cells_2d: 1 <= p <= 16384 (got %d)", p);
   OMBO_CUDA(cudaSetDevice(ctx->device));
   return ombo_cells_2d_impl(ctx, PF, p, ideal, maxp, cells, (cudaStream_t)stream);
+}
+
+int ombo_ehvi_boxes(ombo_ctx *ctx, const double *PF, int p, int k, const double *ref, double *table, double *boxes,
+                    int64_t boxes_cap, int *B_out, int64_t *n_boxes_out, void *stream) {
+  OMBO_CHECK(ctx && ref && table && B_out && n_boxes_out && (PF || p == 0) && (boxes || boxes_cap == 0),
+             "ehvi_boxes: NULL argument");
+  OMBO_CHECK(k >= 2 && k <= OMBO_MAX_OBJ, "ehvi_boxes: 2 to %d objectives (got %d)", OMBO_MAX_OBJ, k);
+  OMBO_CHECK(p >= 0 && p <= 16384, "ehvi_boxes: 0 <= p <= 16384 (got %d)", p);
+  OMBO_CHECK(boxes_cap >= 0, "ehvi_boxes: negative boxes_cap");
+  for (int c = 0; c < k; ++c) OMBO_CHECK(isfinite(ref[c]), "ehvi_boxes: ref[%d] is not finite", c);
+  OMBO_CUDA(cudaSetDevice(ctx->device));
+  long long nb = 0;
+  const int rc = ombo_ehvi_boxes_impl(ctx, PF, p, k, ref, table, boxes, boxes_cap, B_out, &nb, (cudaStream_t)stream);
+  *n_boxes_out = nb;
+  return rc;
 }
 
 int ombo_posterior_joint_samples(ombo_ctx *ctx, const ombo_gp *gp, const double *Xc, int m, const double *Z,

@@ -73,6 +73,7 @@ struct ombo_ctx {
   void *ws_box;       size_t ws_box_bytes;       // EHVI_BOX boxes as packed 16-bit breakpoint indices
   void *ws_prune;     size_t ws_prune_bytes;     // pruned scoring: per-candidate upper bounds, survivors, cub scratch
   void *ws_topk;      size_t ws_topk_bytes;      // top-k: one pass's keys, the running k-list, selections, cub scratch
+  void *ws_boxprep;   size_t ws_boxprep_bytes;   // ombo_ehvi_boxes: flags, ranks, slice lists, tuples, counts, table
   void *ws_stage[2];  size_t ws_stage_bytes;     // host-entry H2D staging (double buffered)
   void *ws_best;                                  // 16 B device best for the host entry
   ombo_best *pinned_best;                         // pinned host landing zone
@@ -236,5 +237,8 @@ int ombo_pareto_mask_impl(ombo_ctx *ctx, const double *Y, int n, int k, unsigned
 int ombo_hypervolume_impl(ombo_ctx *ctx, const double *P, int p, int k, const double *ref, double *out, cudaStream_t s);
 int ombo_cells_2d_impl(ombo_ctx *ctx, const double *PF, int p, const double *ideal, const double *maxp, double *cells,
                        cudaStream_t s);
+// box_prep.cu: the box decomposition of host_prep.ehvi_boxes (one synchronise)
+int ombo_ehvi_boxes_impl(ombo_ctx *ctx, const double *PF, int p, int k, const double *ref, double *table,
+                         double *boxes, long long boxes_cap, int *B_out, long long *n_boxes_out, cudaStream_t s);
 int ombo_pool_rows_impl(ombo_ctx *ctx, const PoolDev &pool, long long first, long long count,
                         double *out, cudaStream_t s);
