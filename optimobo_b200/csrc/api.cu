@@ -83,6 +83,8 @@ int ombo_ctx_create(int device, ombo_ctx **out) {
     k.prune_depth = geti("OMBO_PRUNE_DEPTH", 1) >= 2 ? 2 : 1;
     { const char *e = getenv("OMBO_PRUNE_CAP"); k.prune_cap = e ? atoll(e) : 0; }
     k.prune_log = getenv("OMBO_PRUNE_LOG") != nullptr;
+    k.prune_stage1 = geti("OMBO_PRUNE_STAGE1", 1) != 0;
+    { const char *e = getenv("OMBO_PRUNE_STAGE1_CAP"); k.prune_cap1 = e ? atoll(e) : 0; }
   }
   OMBO_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; ++i) {
@@ -112,6 +114,7 @@ int ombo_ctx_destroy(ombo_ctx *c) {
   if (c->prof_dev) cudaFree(c->prof_dev);
   for (int i = 0; i < 2; ++i) if (c->f8_sched[i]) cudaFree(c->f8_sched[i]);
   if (c->ws_prune) cudaFree(c->ws_prune);
+  if (c->ws_prune1) cudaFree(c->ws_prune1);
   if (c->ws_topk) cudaFree(c->ws_topk);
   if (c->ws_boxprep) cudaFree(c->ws_boxprep);
   if (c->ws_best) cudaFree(c->ws_best);
@@ -404,7 +407,9 @@ static bool prune_eligible(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const om
   return ombo_f8_can_fuse(ctx, g1, acq->n_pf, ctx->knobs.prune_depth, s) && ombo_f8_can_fuse(ctx, g1, acq->n_pf, 0, s);
 }
 
-static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, const ombo_acq *acq,
+// the depth-1 path: the BOUND pass over the pool, its threshold and survivors; *done = false: nothing was merged
+// into best_dev and the caller scores the pool in full
+static int prune_depth1(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, const ombo_acq *acq,
                         ombo_best *best_dev, cudaStream_t s, bool *done) {
   *done = false;
   const long long m = pool->m;
@@ -469,6 +474,127 @@ static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool
     if (rc) return rc;
   }
   k_prune_merge<<<1, 1, 0, s>>>(h, sel, pool->index_base, best_dev);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  *done = true;
+  return OMBO_OK;
+}
+
+// ---- stage 1 of the pruned arg-max: the mean-only bound (posterior_mean8.cu) ---------------------------------------
+// UB1 (both means exact, each variance replaced by its prior bound) is computed for every candidate in one launch.
+// The threshold v0 is the largest full score among the per-CTA maxima of UB1 (one candidate per CTA of the launch,
+// the global maximum among them); candidates with UB1 >= v0 - tau UB1_max (or NaN) survive, by the argument above
+// with UB1 in place of UB.  The survivors are gathered into an explicit pool and go through the depth-1 path
+// unchanged; a gathered subset reproduces mu, var and the values bit for bit, so the winner and its value are the
+// unpruned call's.  Too many survivors (or no positive threshold): the depth-1 path takes the whole pool.
+
+// rows of the per-CTA maxima (partials of the stage-1 launch) into an explicit pool, and their local indices
+__global__ void k_prune1_top(PoolDev pool, long long m, const ombo_best *__restrict__ partials, int n,
+                             long long *__restrict__ top_idx, void *__restrict__ out, int out_f32) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n * pool.d) return;
+  const int r = e / pool.d, j = e % pool.d;
+  long long c = partials[r].index - pool.index_base;
+  if (c < 0 || c >= m) c = 0;                     // a CTA without candidates: row 0 stands in (a real candidate)
+  if (j == 0) top_idx[r] = c;
+  const double x = ombo_pool_coord(pool, c, j);
+  if (out_f32) ((float *)out)[e] = (float)x;
+  else ((double *)out)[e] = x;
+}
+
+// the best threshold candidate and the best survivor of stage 2, mapped to global indices, into the running best
+__global__ void k_prune1_merge(const PruneHdr *__restrict__ h, const long long *__restrict__ top_idx,
+                               const long long *__restrict__ sel, long long base, ombo_best *__restrict__ best) {
+  BestPair b;
+  b.v = -INFINITY; b.i = -1;
+  if (h->v0.index >= 0) { b.v = h->v0.value; b.i = base + top_idx[h->v0.index]; }
+  if (h->loc.index >= 0) {
+    const long long gi = base + sel[h->loc.index];
+    if (b.i < 0 || better(h->loc.value, gi, b.v, b.i)) { b.v = h->loc.value; b.i = gi; }
+  }
+  if (b.i >= 0 && (best->index < 0 || better(b.v, b.i, best->value, best->index))) {
+    best->value = b.v; best->index = b.i;
+  }
+}
+
+static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, const ombo_acq *acq,
+                        ombo_best *best_dev, cudaStream_t s, bool *done) {
+  *done = false;
+  const GpDev gd[2] = {gp_dev_view(gps[0]), gp_dev_view(gps[1])};
+  if (!ctx->knobs.prune_stage1 || !ombo_mean8_covers(gd, acq->n_pf))
+    return prune_depth1(ctx, gps, pool, acq, best_dev, s, done);
+  const long long m = pool->m;
+  const long long cap = ctx->knobs.prune_cap1 > 0 ? ctx->knobs.prune_cap1 : std::max(1LL << 16, m / 8);
+  const int n_top = ctx->num_sms;                 // the most CTAs stage 1 launches: one threshold row each
+  const int out_f32 = pool->X && pool->dtype == 1;
+  const size_t resz = out_f32 ? 4 : 8;
+  auto up = [](size_t b) { return (b + 255) / 256 * 256; };
+  const cub::CountingInputIterator<long long> ids(0);
+  size_t cub_bytes = 0;
+  OMBO_CUDA(cub::DeviceSelect::If(nullptr, cub_bytes, ids, (long long *)nullptr, (long long *)nullptr, m,
+                                  PruneKeep{nullptr, nullptr}, s));
+  const size_t o_top = up(sizeof(PruneHdr)), o_trows = o_top + up((size_t)n_top * 8),
+               o_ub = o_trows + up((size_t)n_top * pool->d * resz), o_sel = o_ub + up((size_t)m * 8),
+               o_rows = o_sel + up((size_t)m * 8), o_cub = o_rows + up((size_t)std::min(cap, m) * pool->d * resz);
+  if (ombo_ws_reserve(&ctx->ws_prune1, &ctx->ws_prune1_bytes, o_cub + cub_bytes)) {
+    (void)cudaGetLastError();
+    return prune_depth1(ctx, gps, pool, acq, best_dev, s, done);
+  }
+  int rc;
+  char *ws = (char *)ctx->ws_prune1;
+  PruneHdr *h = (PruneHdr *)ws;
+  long long *top_idx = (long long *)(ws + o_top);
+  void *trows = ws + o_trows;
+  double *ub = (double *)(ws + o_ub);
+  long long *sel = (long long *)(ws + o_sel);
+  void *rows = ws + o_rows;
+  k_prune_init<<<1, 1, 0, s>>>(h);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  PoolDev pd;
+  fill_pool_dev(pd, pool);
+  pd.X = pool->X;
+  // stage 1: UB1 of every candidate, the per-CTA maxima (ctx->ws_partial) and the largest
+  int n_cta = 0;
+  rc = ombo_mean8_bound(ctx, gd, pd, m, acq->stripes, acq->n_pf, (float)acq->cache_c00, (float)acq->cache_c01, ub,
+                        &h->ub, nullptr, &n_cta, s);
+  if (rc) return rc;
+  k_prune1_top<<<(unsigned)((n_cta * pool->d + 255) / 256), 256, 0, s>>>(pd, m, (const ombo_best *)ctx->ws_partial,
+                                                                         n_cta, top_idx, trows, out_f32);
+  ctx->launches += 1;
+  OMBO_CUDA(cudaGetLastError());
+  // threshold: the best full score among them (local index into top_idx)
+  ombo_pool sub = *pool;
+  sub.X = trows; sub.dtype = out_f32; sub.m = n_cta; sub.index_base = 0;
+  rc = score_passes(ctx, gps, 2, &sub, acq, OMBO_PREC_FAST, nullptr, nullptr, nullptr, &h->v0, s);
+  if (rc) return rc;
+  OMBO_CUDA(cub::DeviceSelect::If(ws + o_cub, cub_bytes, ids, sel, &h->n_sel, m, PruneKeep{ub, h}, s));
+  ctx->launches += 1;
+  PruneHdr hh;
+  OMBO_CUDA(cudaMemcpyAsync(ctx->pinned_best, h, sizeof(PruneHdr), cudaMemcpyDeviceToHost, s));
+  OMBO_CUDA(cudaStreamSynchronize(s));
+  memcpy(&hh, ctx->pinned_best, sizeof(PruneHdr));
+  if (ctx->knobs.prune_log)
+    fprintf(stderr, "[prune1] m %lld survivors %lld ub_max %.9g at %lld v0 %.9g top %d cap %lld\n", m, hh.n_sel,
+            hh.ub.value, (long long)hh.ub.index, hh.v0.value, n_cta, cap);
+  if (!std::isfinite(hh.ub.value) || !(hh.v0.value - OMBO_PRUNE_TAU * hh.ub.value > 0.0) || hh.n_sel > cap)
+    return prune_depth1(ctx, gps, pool, acq, best_dev, s, done);
+  // stage 2: the depth-1 path on the survivors (local indices into sel), in full if it declines
+  if (hh.n_sel > 0) {
+    const long long n = hh.n_sel;
+    k_prune_gather<<<(unsigned)((n * pool->d + 255) / 256), 256, 0, s>>>(pd, m, sel, h, n, rows, out_f32);
+    ctx->launches += 1;
+    OMBO_CUDA(cudaGetLastError());
+    sub.X = rows; sub.m = n;
+    bool done2 = false;
+    rc = prune_depth1(ctx, gps, &sub, acq, &h->loc, s, &done2);
+    if (rc) return rc;
+    if (!done2) {
+      rc = score_passes(ctx, gps, 2, &sub, acq, OMBO_PREC_FAST, nullptr, nullptr, nullptr, &h->loc, s);
+      if (rc) return rc;
+    }
+  }
+  k_prune1_merge<<<1, 1, 0, s>>>(h, top_idx, sel, pool->index_base, best_dev);
   ctx->launches += 1;
   OMBO_CUDA(cudaGetLastError());
   *done = true;
@@ -722,6 +848,27 @@ int ombo_debug_posterior_bound(ombo_ctx *ctx, const ombo_gp *gp, const ombo_pool
                                      nullptr, bound_chunks);
   ctx->knobs.fast_gen_warps = keep;
   return rc;
+}
+
+// the stage-1 launch of the pruned arg-max on its own: mu [2][m] (the FP32 means as doubles), ub [m], the largest
+// bound into *best_dev
+int ombo_debug_mean8(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, const ombo_acq *acq, double *mu,
+                     double *ub, ombo_best *best_dev, void *stream) {
+  OMBO_CHECK(ctx && gps && pool && acq && mu && ub && best_dev, "debug_mean8: NULL argument");
+  OMBO_CHECK(acq->kind == OMBO_ACQ_EHVI2D && acq->stripes && acq->n_pf >= 1, "debug_mean8: needs an EHVI2D spec");
+  for (int g = 0; g < 2; ++g)
+    OMBO_CHECK(gps[g].state && (gps[g].reserved & OMBO_GP_F8C_PLANES) && gps[g].d == pool->d,
+               "debug_mean8: gp %d has no f8c planes or the wrong d", g);
+  OMBO_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  PoolDev pd;
+  fill_pool_dev(pd, pool);
+  pd.X = pool->X;
+  const GpDev gd[2] = {gp_dev_view(gps[0]), gp_dev_view(gps[1])};
+  int rc = ombo_best_init(ctx, best_dev, s);
+  if (rc) return rc;
+  return ombo_mean8_bound(ctx, gd, pd, pool->m, acq->stripes, acq->n_pf, (float)acq->cache_c00,
+                          (float)acq->cache_c01, ub, best_dev, mu, nullptr, s);
 }
 
 int64_t ombo_launch_count(ombo_ctx *ctx, int reset) {

@@ -56,6 +56,9 @@ struct ombo_knobs {
   int prune_depth;        // OMBO_PRUNE_DEPTH: 256-column chunks of V behind the variance bound (1 or 2)
   long long prune_cap;    // OMBO_PRUNE_CAP: most survivors scored in full before falling back (0: max(2^16, m / 64))
   int prune_log;          // OMBO_PRUNE_LOG: one stderr line per pruned call (survivors, bound, threshold)
+  int prune_stage1;       // OMBO_PRUNE_STAGE1=0: no mean-only first stage in front of the variance bound
+  long long prune_cap1;   // OMBO_PRUNE_STAGE1_CAP: most stage-1 survivors before the depth-1 path takes the whole pool
+                          //   (0: max(2^16, m / 8))
 };
 
 struct ombo_ctx {
@@ -72,6 +75,7 @@ struct ombo_ctx {
   void *ws_partial;   size_t ws_partial_bytes;   // per-block arg-max partials
   void *ws_box;       size_t ws_box_bytes;       // EHVI_BOX boxes as packed 16-bit breakpoint indices
   void *ws_prune;     size_t ws_prune_bytes;     // pruned scoring: per-candidate upper bounds, survivors, cub scratch
+  void *ws_prune1;    size_t ws_prune1_bytes;    // its mean-only first stage: bounds, survivors and their rows
   void *ws_topk;      size_t ws_topk_bytes;      // top-k: one pass's keys, the running k-list, selections, cub scratch
   void *ws_boxprep;   size_t ws_boxprep_bytes;   // ombo_ehvi_boxes: flags, ranks, slice lists, tuples, counts, table
   void *ws_stage[2];  size_t ws_stage_bytes;     // host-entry H2D staging (double buffered)
@@ -219,6 +223,14 @@ int ombo_posterior_fast8(ombo_ctx *ctx, const GpDev &gp, const PoolDev &pool, lo
                          const FuseAcq *fuse_req = nullptr, int *fused = nullptr, int bound_chunks = 0);
 // whether an f8c launch for this GP can carry the fused 2-D EHVI of a front of n_pf points (shared memory)
 bool ombo_f8_can_fuse(ombo_ctx *ctx, const GpDev &gp, int n_pf, int bound_chunks, cudaStream_t s);
+// posterior_mean8.cu: stage 1 of the pruned arg-max, the mean-only bound of the exact 2-D EHVI of an f8c pair for every
+// candidate of a pool (ub[m], mu_out [2][m] optional) and the largest into *best_dev; covers d <= 12 while both
+// training sets fit in shared memory.  *grid_out (optional): the CTAs launched, whose per-CTA maxima are left in
+// ctx->ws_partial
+bool ombo_mean8_covers(const GpDev gp[2], int n_pf);
+int ombo_mean8_bound(ombo_ctx *ctx, const GpDev gp[2], const PoolDev &pool, long long m, const double *stripes,
+                     int n_pf, float c00, float c01, double *ub, ombo_best *best_dev, double *mu_out, int *grid_out,
+                     cudaStream_t s);
 // merges n_partials per-block (value, index) pairs in ctx->ws_partial with the running best
 int ombo_argmax_merge(ombo_ctx *ctx, int n_partials, ombo_best *best_dev, cudaStream_t s);
 int ombo_fast_path_built();

@@ -42,6 +42,7 @@
 
 #include "umma.cuh"
 #include "acq_math.cuh"
+#include "gen8.cuh"
 
 #define F8_HI_BYTES 16384   // 128 rows x 64 fp16 (SWIZZLE_128B)
 #define F8_P8_BYTES 8192    // 128 rows x 64 e4m3 (SWIZZLE_64B)
@@ -322,9 +323,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
       for (int e = lane; e < FM * DP; e += 32) {
         const int r_ = e & (FM - 1), j = e >> 7;
         const long long cg = tile * FM + r_;
-        xcb[j * FM + r_] = (cg < prm.m && j < d)
-                               ? -2.0f * (float)((ombo_pool_coord(prm.pool, cg, j) - prm.gp.center[j]) * inv_ell[j])
-                               : 0.f;
+        xcb[j * FM + r_] = (cg < prm.m && j < d) ? gen8_coord(ombo_pool_coord(prm.pool, cg, j), prm.gp.center[j], inv_ell[j]) : 0.f;
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&xc_full[b]));
@@ -460,7 +459,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
         const int b = (int)(it & 1);
         mbar_wait_sleep(smem_u32(&mu_full[b]), (uint32_t)(it >> 1) & 1, 64);
         const float *mub = mu_sm + (size_t)b * 4 * FM;
-        const float mu_s = (mub[row] + mub[FM + row]) + (mub[2 * FM + row] + mub[3 * FM + row]);
+        const float mu_s = gen8_mean_sum(mub[row], mub[FM + row], mub[2 * FM + row], mub[3 * FM + row]);
         if (cg < prm.m) {
           const int P = prm.fuse.n_pf;
           const bool s0 = prm.fuse.self_model == 0;
@@ -537,75 +536,13 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
       float x[ROWS][DP], a2[ROWS];
 #pragma unroll
       for (int rr = 0; rr < ROWS; ++rr) {
-        float acc = 0.f;
         mu_acc[rr] = 0.f;
-#pragma unroll
-        for (int j = 0; j < DP; ++j) { x[rr][j] = xcb[j * FM + row0 + 16 * rr]; acc = fmaf(x[rr][j], x[rr][j], acc); }
-        a2[rr] = 0.25f * acc;
+        a2[rr] = gen8_load_row<DP>(xcb + row0 + 16 * rr, FM, x[rr]);
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&xc_empty[b]));                   // xc[b] may be refilled
-      // the K1 math of one K-block, shared by the full and the mean-only steps (the same operations in the same order,
-      // so both see the same k' and accumulate the same mean): squared distances of this lane's rows to the block's
-      // eight training points of column group g, k'(r) of one row, and that row's share of the mean
-      auto dist2 = [&](const float *xs, float2 (&r2)[ROWS][4]) {
-        {
-          const float4 n0 = *(const float4 *)(xs + (DP + 1) * FK);      // |b_i|^2
-          const float4 n1 = *(const float4 *)(xs + (DP + 1) * FK + 4);
-#pragma unroll
-          for (int rr = 0; rr < ROWS; ++rr) {
-            const float2 aa = make_float2(a2[rr], a2[rr]);
-            r2[rr][0] = __fadd2_rn(aa, make_float2(n0.x, n0.y));
-            r2[rr][1] = __fadd2_rn(aa, make_float2(n0.z, n0.w));
-            r2[rr][2] = __fadd2_rn(aa, make_float2(n1.x, n1.y));
-            r2[rr][3] = __fadd2_rn(aa, make_float2(n1.z, n1.w));
-          }
-        }
-#pragma unroll
-        for (int j = 0; j < DP; ++j) {
-          const float4 t0 = *(const float4 *)(xs + j * FK);
-          const float4 t1 = *(const float4 *)(xs + j * FK + 4);
-#pragma unroll
-          for (int rr = 0; rr < ROWS; ++rr) {
-            const float2 xx = make_float2(x[rr][j], x[rr][j]);            // -2 a_j
-            r2[rr][0] = __ffma2_rn(xx, make_float2(t0.x, t0.y), r2[rr][0]);
-            r2[rr][1] = __ffma2_rn(xx, make_float2(t0.z, t0.w), r2[rr][1]);
-            r2[rr][2] = __ffma2_rn(xx, make_float2(t1.x, t1.y), r2[rr][2]);
-            r2[rr][3] = __ffma2_rn(xx, make_float2(t1.z, t1.w), r2[rr][3]);
-          }
-        }
-      };
-      auto kval = [&](const float2 (&r2r)[4], float2 (&kv)[4]) {
-        if (MATERN) {
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            float2 rad, ex;
-            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad.x) : "f"(fabsf(r2r[e].x)));
-            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad.y) : "f"(fabsf(r2r[e].y)));
-            const float2 arg = __fmul2_rn(rad, make_float2(-3.2259955597f, -3.2259955597f));   // -sqrt5 log2(e)
-            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ex.x) : "f"(arg.x));
-            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ex.y) : "f"(arg.y));
-            const float2 poly = __ffma2_rn(rad, make_float2(2.2360679775f, 2.2360679775f),
-                                           __ffma2_rn(r2r[e], make_float2(1.6666666667f, 1.6666666667f),
-                                                      make_float2(1.0f, 1.0f)));
-            kv[e] = __fmul2_rn(poly, ex);
-          }
-        } else {
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const float2 arg = __fmul2_rn(r2r[e], make_float2(-0.7213475204f, -0.7213475204f));  // -0.5 log2(e)
-            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(kv[e].x) : "f"(arg.x));
-            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(kv[e].y) : "f"(arg.y));
-          }
-        }
-      };
-      auto mean_add = [&](const float2 (&kv)[4], const float4 al0, const float4 al1, float &acc) {
-        float2 m2 = __fmul2_rn(kv[0], make_float2(al0.x, al0.y));
-        m2 = __ffma2_rn(kv[1], make_float2(al0.z, al0.w), m2);
-        m2 = __ffma2_rn(kv[2], make_float2(al1.x, al1.y), m2);
-        m2 = __ffma2_rn(kv[3], make_float2(al1.z, al1.w), m2);
-        acc += m2.x + m2.y;
-      };
+      // the K1 math of one K-block (gen8.cuh) is shared by the full and the mean-only steps -- the same operations in
+      // the same order, so both see the same k' and accumulate the same mean
       {
         for (int si = 0; si < n_steps; ++si) {
           const uint32_t w = sched[si];
@@ -623,14 +560,14 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
             if (!solo) mbar_wait_sleep(s_full_u + sl * 8, slph, 20);
             const float *xs = xt + sl * XT_STRIDE + 8 * g;
             float2 r2[ROWS][4];
-            dist2(xs, r2);
+            gen8_dist2<DP, ROWS>(xs, x, a2, r2);
             const float4 al0 = *(const float4 *)(xs + DP * FK);
             const float4 al1 = *(const float4 *)(xs + DP * FK + 4);
 #pragma unroll
             for (int rr = 0; rr < ROWS; ++rr) {
               float2 kv[4];
-              kval(r2[rr], kv);
-              mean_add(kv, al0, al1, mu_acc[rr]);
+              gen8_kval<MATERN>(r2[rr], kv);
+              gen8_mean_add(kv, al0, al1, mu_acc[rr]);
             }
             __syncwarp();
             if (lane == 0 && !solo) mbar_arrive(s_empty_u + sl * 8);
@@ -645,7 +582,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
           const uint32_t st_hi = st_u + off_hi0, st_c8 = st_u + off_c80;
           if (!(prm.dbg & 2)) {
             float2 r2[ROWS][4];
-            dist2(xs, r2);
+            gen8_dist2<DP, ROWS>(xs, x, a2, r2);
             const float4 al0 = *(const float4 *)(xs + DP * FK);
             const float4 al1 = *(const float4 *)(xs + DP * FK + 4);
             F8_TRACE_G(0x80 | kb);
@@ -654,8 +591,8 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
 #pragma unroll
             for (int rr = 0; rr < ROWS; ++rr) {
               float2 kv[4];
-              kval(r2[rr], kv);
-              mean_add(kv, al0, al1, mu_acc[rr]);
+              gen8_kval<MATERN>(r2[rr], kv);
+              gen8_mean_add(kv, al0, al1, mu_acc[rr]);
               uint32_t hi[4];
               uint32_t c1[2], c2[2];
 #pragma unroll
@@ -708,7 +645,7 @@ k_posterior_fast8(const __grid_constant__ F8Maps maps, const FastParams prm) {
       if (tg < 16 * R) {
         const int row = 16 * R * rg + tg;
         const long long cg = tile * FM + row;
-        if (cg < prm.m) prm.mu_out[cg] = (double)((mub[row] + mub[FM + row]) + (mub[2 * FM + row] + mub[3 * FM + row]));
+        if (cg < prm.m) prm.mu_out[cg] = (double)gen8_mean_sum(mub[row], mub[FM + row], mub[2 * FM + row], mub[3 * FM + row]);
       }
       // mu_sm is double buffered by tile: the rows of buffer b are rewritten two tiles later, after the next
       // tile's barrier of the same row group
