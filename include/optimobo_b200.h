@@ -19,7 +19,8 @@
  *                        keep.py:118 / cparego.py:450 (EI), cparego.py:486 (consraint_ei),
  *                        keep.py:142 (pareto_expected_improvement), emo.py:192
  *                        (hypervolume_based_PoI); EHVI_BOX and EHVI_BOX_FEAS have no
- *                        reference counterpart
+ *                        reference counterpart, HV_POI_BOX extends emo.py:192 to 3 and 4
+ *                        objectives
  *   scalarisation ids <- optimobo/scalarisations.py:37,53,76,113,153,177,201,222,242,277,314,355
  *
  * Conventions: every function returns an int status (0 = ok, negative = error; the message
@@ -67,7 +68,8 @@ enum {
   OMBO_ACQ_PARETO_EI = 6,       /* keep.py:142-150 (gp 0 = pareto model, gp 1 = scalar)   */
   OMBO_ACQ_HV_POI = 7,          /* emo.py:192-228                                         */
   OMBO_ACQ_EHVI_BOX = 8,        /* exact EHVI, 2 <= n_obj <= 4, by box decomposition      */
-  OMBO_ACQ_EHVI_BOX_FEAS = 9    /* EHVI_BOX x probability of feasibility (constraint GPs) */
+  OMBO_ACQ_EHVI_BOX_FEAS = 9,   /* EHVI_BOX x probability of feasibility (constraint GPs) */
+  OMBO_ACQ_HV_POI_BOX = 10      /* HV_POI, 2 <= n_obj <= 4, over the boxes of EHVI_BOX    */
 };
 
 /* OMBO_ACQ_EHVI_BOX: the exact expected hypervolume improvement for k = n_obj independent Gaussian objectives,
@@ -89,7 +91,19 @@ enum {
  *   EHVI_box(mu_0..k-1, sigma_0..k-1) * prod_j Phi(-mu_{k+j} / sqrt(var_{k+j} + var_eps[k+j])),
  * the product taken in j order and in FP64 (also in the fast precision mode, so that a pool far on the infeasible
  * side keeps values below FLT_MIN).  Limits: those of OMBO_ACQ_EHVI_BOX and k + 1 <= n_gp <= OMBO_MAX_GP.  The
- * scoring entries compute every model's variance for this kind, and never prune or fuse it. */
+ * scoring entries compute every model's variance for this kind, and never prune or fuse it.
+ *
+ * OMBO_ACQ_HV_POI_BOX: the hypervolume-based probability of improvement of OMBO_ACQ_HV_POI (emo.py:192-228) for
+ * k = n_obj independent Gaussian objectives, sigma_i = sqrt(var_i + var_eps[i]), over the region
+ * R = {ideal <= z <= r' : no front point dominates z}:
+ *   PoI * Imp,  PoI = sum_c prod_i (Phi((u_ci - mu_i) / sigma_i) - Phi((l_ci - mu_i) / sigma_i)) = P(y in R),
+ *               Imp = sum_c prod_i (max(u_ci - mu_i, 0) - max(l_ci - mu_i, 0))           = vol(R above mu).
+ * Both depend on R only, so any tiling of R gives the value; with r' = max(max_point, the front's maximum) per
+ * objective and k = 2, R is the region the cells of OMBO_ACQ_HV_POI tile.  Every field as for OMBO_ACQ_EHVI_BOX,
+ * except that the (k, B) table in `stripes` is clamped below at the ideal point (row i = max(row i, ideal_i): index 0
+ * is ideal_i, and a box below the ideal has zero width and adds nothing), its last column is r', and
+ * var_eps[0..k-1] = 1e-5 in the reference's formula.  Limits: those of OMBO_ACQ_EHVI_BOX.  The scoring entries
+ * compute the variance of GPs 0..k-1 only, and never prune or fuse this kind. */
 #define OMBO_EHVI_BOX_MAX_BREAKS 514        /* a front of up to 512 points */
 #define OMBO_EHVI_BOX_MAX_BOXES  (1 << 20)
 

@@ -21,6 +21,7 @@ SEM_REFERENCE, SEM_EXACT = 0, 1
  ACQ_PARETO_EI, ACQ_HV_POI) = range(8)
 ACQ_EHVI_BOX = 8
 ACQ_EHVI_BOX_FEAS = 9   # box EHVI x probability of feasibility: GPs n_obj.. are constraint models
+ACQ_HV_POI_BOX = 10     # HV-PoI for 2 to 4 objectives over the box decomposition, table clamped at the ideal point
 ACQ_FRONT_VALID = 1   # ombo_acq.reserved bit: the EHVI2D stripes form a valid staircase (OMBO_ACQ_FRONT_VALID)
 EHVI_BOX_MAX_BREAKS, EHVI_BOX_MAX_BOXES = 514, 1 << 20
 TOPK_MAX = 65536

@@ -7,6 +7,7 @@ Reference seam (SURVEY.md section 8b):
     function(X, model, current_best)                          _expected_improvement    :362
     function(X, agg_model, constraint_models, current_best)   consraint_ei     cparego.py:540
     function(X, models, P, cells)                             hypervolume_based_PoI  emo.py:237
+    function(X, models, ideal_point, max_point, PF)           hypervolume_based_PoI_box (2 to 4 objectives)
 each called with ONE x by scipy differential_evolution or the ParEGO/KEEP EA.  Here the same
 names accept X of shape (d,) or (m, d) and return (m,) values computed on the GPU, and
 `propose*` scores a whole pool (explicit or counter-generated) and returns
@@ -175,8 +176,9 @@ class AcquisitionSpec:
 
         if self.stripes is not None:
             a.stripes = up("stripes", self.stripes)
-            # EHVI2D: stripes are (2, P + 2); EHVI_BOX(_FEAS): the (k, B) breakpoint table
-            a.n_pf = self.stripes.shape[1] - (0 if self.kind in (_cabi.ACQ_EHVI_BOX, _cabi.ACQ_EHVI_BOX_FEAS) else 2)
+            # EHVI2D: stripes are (2, P + 2); EHVI_BOX(_FEAS), HV_POI_BOX: the (k, B) breakpoint table
+            box = self.kind in (_cabi.ACQ_EHVI_BOX, _cabi.ACQ_EHVI_BOX_FEAS, _cabi.ACQ_HV_POI_BOX)
+            a.n_pf = self.stripes.shape[1] - (0 if box else 2)
         if self.cells is not None:
             a.cells = up("cells", self.cells)
             a.n_cells = self.cells.shape[0]
@@ -282,6 +284,33 @@ def spec_hv_poi(cells):
     """emo.py:192-228: cells (n_cells, 2, 2), [c][0] upper / [c][1] lower."""
     cells = np.asarray(cells, dtype=np.float64)
     return AcquisitionSpec(kind=_cabi.ACQ_HV_POI, n_obj=2, var_eps=(1e-5, 1e-5), cells=cells, n_models=2)
+
+
+def spec_hv_poi_box(ideal_point, max_point, PF, device=None):
+    """The hypervolume-based probability of improvement of spec_hv_poi (emo.py:192-228) for 2 <= k <= 4 objectives:
+    PoI * Imp over the region R = {ideal <= z <= r' : no front point dominates z}, r' = max(max_point, PF.max(0)) per
+    objective, with PoI = P(y in R) and Imp = vol(R above mu) at sigma_i = sqrt(var_i + 1e-5).  Both depend on R only;
+    for k = 2, R is the region decompose_into_cells tiles, so the value equals spec_hv_poi's on those cells whenever
+    no front point lies below the ideal point.  R is tiled by the boxes of ehvi_boxes(PF, r') with every breakpoint
+    clamped below at the ideal point; an empty front gives the single box [ideal, max_point].  `device` as for
+    spec_ehvi_box."""
+    ideal = np.asarray(ideal_point, dtype=np.float64).reshape(-1)
+    maxp = np.asarray(max_point, dtype=np.float64).reshape(-1)
+    k = len(maxp)
+    if not 2 <= k <= 4 or len(ideal) != k:
+        raise ValueError(f"HV-PoI over boxes takes 2 to 4 objectives and an ideal point of the same length "
+                         f"(got {len(ideal)} and {k})")
+    P = np.asarray(PF.detach().cpu() if torch.is_tensor(PF) else PF, dtype=np.float64).reshape(-1, k)
+    if not (np.all(np.isfinite(ideal)) and np.all(np.isfinite(maxp)) and np.all(np.isfinite(P))):
+        raise ValueError("HV-PoI over boxes needs a finite ideal point, max point and front")
+    r = np.maximum(maxp, P.max(0)) if len(P) else maxp
+    table, boxes = _box_tables(P, r, device)
+    if torch.is_tensor(table):
+        table = torch.maximum(table, torch.as_tensor(ideal, device=table.device)[:, None])
+    else:
+        table = np.maximum(table, ideal[:, None])
+    return AcquisitionSpec(kind=_cabi.ACQ_HV_POI_BOX, n_obj=k, ref=tuple(r), var_eps=(1e-5,) * k, stripes=table,
+                           cells=boxes, n_models=k)
 
 
 def adopt_scalarisation(obj):
@@ -725,3 +754,7 @@ def pareto_expected_improvement(X, pareto_model, scalarised_model, opt_value, pr
 
 def hypervolume_based_PoI(X, models, P, cells, precision="fp64"):
     return evaluate(models, spec_hv_poi(cells), X, precision)
+
+
+def hypervolume_based_PoI_box(X, models, ideal_point, max_point, PF, precision="fp64"):
+    return evaluate(models, spec_hv_poi_box(ideal_point, max_point, PF), X, precision)

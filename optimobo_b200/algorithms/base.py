@@ -23,6 +23,11 @@ from ..acquisition import CandidatePool, propose, propose_batch
 from ..fit import fit_hyperparameters, fit_hyperparameters_device
 from ..gp import GPModel
 
+# "auto" builds the box decomposition on the device from this front size on: on the B200 the device is faster at every
+# front size measured, and from 16 points the host takes 4.6x (k = 3) to 24x (k = 4) its time (DESIGN.md section 4)
+BOX_DEVICE_MIN_FRONT = 16
+BOX_DEVICE_MAX_FRONT = 512      # ombo_ehvi_boxes takes fronts of up to 512 distinct points
+
 
 class PoolOptimiserBase:
     def __init__(self, test_problem, ideal_point=None, max_point=None, n_candidates=1 << 16, precision="auto",
@@ -49,7 +54,7 @@ class PoolOptimiserBase:
         self.refine_rounds = refine_rounds       # zoom rounds around the pool winner (DE's polish step)
         # first front / hypervolume / cells on the device (bit-identical to host_prep; "auto": once the sample
         # holds >= 512 rows, where the O(n^2) host versions start to show next to a ~100 ms scoring pass); the box
-        # decomposition of ehvi="box" follows its own rule (MultiSurrogateOptimiser._box_device)
+        # decomposition (box EHVI, EMO for 3 and 4 objectives) follows its own rule (_box_device)
         self.prep_on_device = prep_on_device
         self.timings = []
 
@@ -91,6 +96,21 @@ class PoolOptimiserBase:
         if self._prep_device(len(ysample)):
             return device_prep.calc_pf(ysample, self.device)
         return host_prep.calc_pf(ysample)
+
+    def _box_device(self, front):
+        """Where the box decomposition of `front` is built: self.device when prep_on_device is True (or "auto" and the
+        front has at least BOX_DEVICE_MIN_FRONT rows) and the front is finite and within the device limit, else None
+        (the host)."""
+        front = np.asarray(front, dtype=float)
+        n = len(front)
+        if self.prep_on_device is True:
+            wanted = True
+        elif self.prep_on_device == "auto":
+            wanted = n >= BOX_DEVICE_MIN_FRONT
+        else:
+            wanted = False
+        ok = n <= BOX_DEVICE_MAX_FRONT and bool(np.all(np.isfinite(front)))
+        return self.device if wanted and ok else None
 
     # ---- surrogate ---------------------------------------------------------------------------------
     def _fit_model(self, X, y):

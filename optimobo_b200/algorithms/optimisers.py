@@ -7,13 +7,7 @@ import numpy as np
 from .. import host_prep, result
 from ..acquisition import (spec_ehvi, spec_ehvi3d, spec_ehvi_box, spec_ehvi_box_feasible, spec_ei,
                            spec_expected_decomposition)
-from .base import PoolOptimiserBase
-
-
-# "auto" builds the box decomposition on the device from this front size on: on the B200 the device is faster at every
-# front size measured, and from 16 points the host takes 4.6x (k = 3) to 24x (k = 4) its time (DESIGN.md section 4)
-BOX_DEVICE_MIN_FRONT = 16
-BOX_DEVICE_MAX_FRONT = 512      # ombo_ehvi_boxes takes fronts of up to 512 distinct points
+from .base import BOX_DEVICE_MAX_FRONT, BOX_DEVICE_MIN_FRONT, PoolOptimiserBase  # noqa: F401
 
 
 class MultiSurrogateOptimiser(PoolOptimiserBase):
@@ -56,21 +50,6 @@ class MultiSurrogateOptimiser(PoolOptimiserBase):
         super().__init__(test_problem, *args, **kwargs)
         self.ehvi = ehvi
         self.batch_size = self._check_batch_size(batch_size)
-
-    def _box_device(self, front):
-        """Where the box decomposition of `front` is built: self.device when prep_on_device is True (or "auto" and the
-        front has at least BOX_DEVICE_MIN_FRONT rows) and the front is finite and within the device limit, else None
-        (the host)."""
-        front = np.asarray(front, dtype=float)
-        n = len(front)
-        if self.prep_on_device is True:
-            wanted = True
-        elif self.prep_on_device == "auto":
-            wanted = n >= BOX_DEVICE_MIN_FRONT
-        else:
-            wanted = False
-        ok = n <= BOX_DEVICE_MAX_FRONT and bool(np.all(np.isfinite(front)))
-        return self.device if wanted and ok else None
 
     def _get_cached_samples(self, dimensions, sample_exponent):
         return host_prep.cached_samples(dimensions, sample_exponent, seed=int(self.rng.integers(0, 2 ** 31)))

@@ -12,6 +12,7 @@
 //   HV_POI            emo.py:176-228
 //   EHVI_BOX          not in the reference: the exact k-objective EHVI over a box decomposition (k_acquire_box)
 //   EHVI_BOX_FEAS     not in the reference: EHVI_BOX times the probability of feasibility of CONSTRAINED_EI
+//   HV_POI_BOX        HV_POI for 2 to 4 objectives: the same region, tiled by the boxes of EHVI_BOX (k_acquire_box)
 // Arg-max replaces the inner optimiser call sites (differential_evolution at optimisers.py:87,
 // :118,:366; cparego.py:94,:544; emo.py:240; EA loops parego.py:242-270, keep.py:260-292):
 // warp shuffle -> block (smem) -> per-block partial -> one final block; ties resolve to the
@@ -356,14 +357,25 @@ __host__ __device__ inline size_t box_smem_bytes(int k, int B, int tile, bool fe
          (size_t)tile * box_cand_stride(k, B) * sizeof(T) + (feas ? (size_t)tile * 8 : 0);
 }
 
-// FEAS (OMBO_ACQ_EHVI_BOX_FEAS): GPs K..n_gp-1 are constraint models, and the value is the box sum times the
-// probability of feasibility prod_j Phi(-mu_j / sqrt(var_j + var_eps[j])), formed in FP64 exactly as the
-// constrained EI forms it (k_acquire), once per candidate in the prologue
-template <typename T, int K, bool FEAS>
+// MODE selects what the box sum adds up:
+//   BOX_EHVI  (OMBO_ACQ_EHVI_BOX): the EHVI above.
+//   BOX_FEAS  (OMBO_ACQ_EHVI_BOX_FEAS): GPs K..n_gp-1 are constraint models, and the value is the box sum times the
+//             probability of feasibility prod_j Phi(-mu_j / sqrt(var_j + var_eps[j])), formed in FP64 exactly as the
+//             constrained EI forms it (k_acquire), once per candidate in the prologue.
+//   BOX_HVPOI (OMBO_ACQ_HV_POI_BOX): the table's index 0 is the ideal point, sigma = sqrt(var + var_eps), and the
+//             value is PoI * Imp with PoI = sum_c prod_i P(l_ci < y_i <= u_ci) and Imp = sum_c prod_i
+//             (max(u_ci - mu_i, 0) - max(l_ci - mu_i, 0)).  V keeps Phi(z) below the mean and Phi(z) - 1 = -Phi(-z) at
+//             or above it, so a box above the mean takes Phi(-z_l) - Phi(-z_u) (two upper tails, not two numbers
+//             near 1) and a box that straddles the mean adds back 1.  The extents come from the t - r row and r - mu;
+//             a box above the mean takes (u - r) - (l - r), not a difference of two numbers ~ t - mu.
+enum { BOX_EHVI = 0, BOX_FEAS = 1, BOX_HVPOI = 2 };
+
+template <typename T, int K, int MODE>
 __global__ void __launch_bounds__(ACQ_THREADS)
 k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double *__restrict__ var, long long m,
               long long ld, long long index_base, const uint4 *__restrict__ boxes, double *__restrict__ out_acq,
               ombo_best *__restrict__ partials, int n_gp) {
+  constexpr bool FEAS = MODE == BOX_FEAS, HVPOI = MODE == BOX_HVPOI;
   const int B = a.n_pf, n_boxes = a.n_cells, G = ACQ_THREADS / tile, cs = box_cand_stride(K, B);
   uint4 *bx = reinterpret_cast<uint4 *>(acq_smem);                  // BOX_CHUNK staged boxes
   double *pof = reinterpret_cast<double *>(bx + BOX_CHUNK);         // FEAS: (tile,) feasibility products
@@ -382,7 +394,7 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
     const int j = e / K, i = e - j * K;
     const long long c = c0 + j;
     const double mv = c < m ? mu[i * ld + c] : 0.0, vv = c < m ? var[i * ld + c] : 1.0;
-    sd[e] = sqrt_t((T)vv);
+    sd[e] = HVPOI ? sqrt_t((T)(vv + a.var_eps[i])) : sqrt_t((T)vv);
     rsd[e] = (T)1 / sd[e];
     shift[e] = (T)(a.stripes[i * B + B - 1] - mv);
     split[e] = B;                                                   // mu above every breakpoint
@@ -401,7 +413,12 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
   for (int e = threadIdx.x; e < tile * K * B; e += ACQ_THREADS) {
     const int j = e / (K * B), ib = e - j * (K * B), i = ib / B, b = ib - i * B, jk = j * K + i;
     T v = 0;                                                        // H(-inf) = 0
-    if (b > 0) {
+    if constexpr (HVPOI) {                                          // index 0 is the ideal point: evaluated too
+      const T c = shift[jk], w = tr[ib] + c;                        // t - mu
+      const T z = w * rsd[jk];
+      v = w >= (T)0 ? -Phi(-z) : Phi(z);
+      if (w >= (T)0 && (b == 0 || tr[ib - 1] + c < (T)0)) split[jk] = b;
+    } else if (b > 0) {
       const T c = shift[jk], s = sd[jk];
       const T w = tr[ib] + c;                                       // t - mu
       const T az = fabs(w * rsd[jk]);
@@ -421,7 +438,7 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
 #pragma unroll
   for (int i = 0; i < K; ++i) { shj[i] = shift[j * K + i]; spj[i] = split[j * K + i]; }
   const T *Vj = V + j * cs;
-  T acc = 0;
+  T acc = 0, vol = 0;                                               // HVPOI: the PoI and the Imp sums
   for (int base = 0; base < n_boxes; base += BOX_CHUNK) {
     const int n = min(BOX_CHUNK, n_boxes - base);
     for (int e = threadIdx.x; e < n; e += ACQ_THREADS) bx[e] = boxes[base + e];
@@ -431,15 +448,20 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
         const uint4 p = bx[q];
         const unsigned uu[4] = {p.x & 0xffffu, p.x >> 16, p.y & 0xffffu, p.y >> 16};
         const unsigned ll[4] = {p.z & 0xffffu, p.z >> 16, p.w & 0xffffu, p.w >> 16};
-        T prod = 1;
+        T prod = 1, ext = 1;
 #pragma unroll
         for (int i = 0; i < K; ++i) {
           const int u = (int)uu[i], l = (int)ll[i];
           T d = Vj[i * B + u] - Vj[i * B + l];
-          if (l < spj[i] && u >= spj[i]) d += shj[i];
+          if (l < spj[i] && u >= spj[i]) d += HVPOI ? (T)1 : shj[i];
           prod = i == 0 ? d : prod * d;
+          if constexpr (HVPOI) {
+            const T x = l >= spj[i] ? tr[i * B + u] - tr[i * B + l] : (u >= spj[i] ? tr[i * B + u] + shj[i] : (T)0);
+            ext = i == 0 ? x : ext * x;
+          }
         }
         acc += prod;
+        if constexpr (HVPOI) vol += ext;
       }
     }
     __syncthreads();
@@ -447,13 +469,20 @@ k_acquire_box(ombo_acq a, int tile, const double *__restrict__ mu, const double 
   // the G slots of each candidate summed in a fixed order (bit-reproducible); the box stage is free after the loop
   T *red = reinterpret_cast<T *>(bx);
   red[threadIdx.x] = acc;
+  if constexpr (HVPOI) red[ACQ_THREADS + threadIdx.x] = vol;
   __syncthreads();
   double val = -INFINITY;
   const bool owner = threadIdx.x < tile && c0 + threadIdx.x < m;
   if (owner) {
     T sum = 0;
     for (int g = 0; g < G; ++g) sum += red[g * tile + threadIdx.x];
-    if (FEAS) {
+    if constexpr (HVPOI) {
+      T imp = 0;
+      for (int g = 0; g < G; ++g) imp += red[ACQ_THREADS + g * tile + threadIdx.x];
+      const double v = (double)sum * (double)imp;
+      if (out_acq) out_acq[c0 + threadIdx.x] = v;
+      val = isnan(v) ? -INFINITY : v;
+    } else if (FEAS) {
       const double v = (double)sum * pof[threadIdx.x];
       if (out_acq) out_acq[c0 + threadIdx.x] = v;
       val = isnan(v) ? -INFINITY : v;
@@ -487,38 +516,39 @@ static int box_tile(int k, int B, bool feas) {
   return box_smem_bytes<T>(k, B, 8, feas) <= 220 * 1024 ? 8 : 0;    // + the static arg-max slots, under 227 KB
 }
 
-template <typename T, int K, bool FEAS>
+template <typename T, int K, int MODE>
 static int launch_box(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var, long long m,
                       long long ld, long long index_base, double *out_acq, cudaStream_t s) {
+  constexpr bool FEAS = MODE == BOX_FEAS;
   const int tile = box_tile<T>(K, acq->n_pf, FEAS);
   OMBO_CHECK(tile > 0, "EHVI_BOX: %d breakpoints x %d objectives do not fit in shared memory", acq->n_pf, K);
   const size_t smem = box_smem_bytes<T>(K, acq->n_pf, tile, FEAS);
   if (smem > 48 * 1024)
-    OMBO_CUDA(cudaFuncSetAttribute(k_acquire_box<T, K, FEAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    OMBO_CUDA(cudaFuncSetAttribute(k_acquire_box<T, K, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long blocks = (m + tile - 1) / tile;
   int rc = ombo_ws_reserve(&ctx->ws_partial, &ctx->ws_partial_bytes, (size_t)blocks * sizeof(ombo_best));
   if (rc) return rc;
-  k_acquire_box<T, K, FEAS><<<(unsigned)blocks, ACQ_THREADS, smem, s>>>(*acq, tile, mu, var, m, ld, index_base,
+  k_acquire_box<T, K, MODE><<<(unsigned)blocks, ACQ_THREADS, smem, s>>>(*acq, tile, mu, var, m, ld, index_base,
                                                                         (const uint4 *)ctx->ws_box, out_acq,
                                                                         (ombo_best *)ctx->ws_partial, n_gp);
   ctx->launches += 1;
   return (int)blocks;
 }
 
-template <bool FEAS>
+template <int MODE>
 static int launch_box_k(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var,
                         long long m, long long ld, long long index_base, double *out_acq, cudaStream_t s, bool fp32) {
   switch (acq->n_obj) {
-    case 2: return fp32 ? launch_box<float, 2, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
-                        : launch_box<double, 2, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
-    case 3: return fp32 ? launch_box<float, 3, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
-                        : launch_box<double, 3, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
-    default: return fp32 ? launch_box<float, 4, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
-                         : launch_box<double, 4, FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
+    case 2: return fp32 ? launch_box<float, 2, MODE>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
+                        : launch_box<double, 2, MODE>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
+    case 3: return fp32 ? launch_box<float, 3, MODE>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
+                        : launch_box<double, 3, MODE>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
+    default: return fp32 ? launch_box<float, 4, MODE>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s)
+                         : launch_box<double, 4, MODE>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s);
   }
 }
 
-// OMBO_ACQ_EHVI_BOX and OMBO_ACQ_EHVI_BOX_FEAS
+// OMBO_ACQ_EHVI_BOX, OMBO_ACQ_EHVI_BOX_FEAS and OMBO_ACQ_HV_POI_BOX
 static int ombo_acquire_box(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu, const double *var,
                             long long m, long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
                             cudaStream_t s, bool fp32) {
@@ -529,9 +559,10 @@ static int ombo_acquire_box(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const 
                                                           (uint4 *)ctx->ws_box);
   ctx->launches += 1;
   fp32 = fp32 && !ctx->knobs.acq_fp64;
-  const int blocks = acq->kind == OMBO_ACQ_EHVI_BOX_FEAS
-                         ? launch_box_k<true>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32)
-                         : launch_box_k<false>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32);
+  const int blocks =
+      acq->kind == OMBO_ACQ_EHVI_BOX_FEAS ? launch_box_k<BOX_FEAS>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32)
+      : acq->kind == OMBO_ACQ_HV_POI_BOX  ? launch_box_k<BOX_HVPOI>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32)
+                                          : launch_box_k<BOX_EHVI>(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, s, fp32);
   if (blocks < 0) return blocks;
   if (best_dev) {
     k_argmax_final<<<1, 1024, 0, s>>>((const ombo_best *)ctx->ws_partial, blocks, best_dev);
@@ -545,7 +576,7 @@ int ombo_acquire(ombo_ctx *ctx, const ombo_acq *acq, int n_gp, const double *mu,
                  long long m, long long ld, long long index_base, double *out_acq, ombo_best *best_dev,
                  cudaStream_t s, bool fp32) {
   if (m <= 0) return OMBO_OK;
-  if (acq->kind == OMBO_ACQ_EHVI_BOX || acq->kind == OMBO_ACQ_EHVI_BOX_FEAS)
+  if (acq->kind == OMBO_ACQ_EHVI_BOX || acq->kind == OMBO_ACQ_EHVI_BOX_FEAS || acq->kind == OMBO_ACQ_HV_POI_BOX)
     return ombo_acquire_box(ctx, acq, n_gp, mu, var, m, ld, index_base, out_acq, best_dev, s, fp32);
   int n_stage = 0;
   if (acq->kind == OMBO_ACQ_EHVI2D) n_stage = 2 * (acq->n_pf + 2);

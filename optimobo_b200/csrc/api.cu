@@ -213,9 +213,10 @@ int ombo_validate_score(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_
       break;
     case OMBO_ACQ_EHVI_BOX:
     case OMBO_ACQ_EHVI_BOX_FEAS:
+    case OMBO_ACQ_HV_POI_BOX:
       OMBO_CHECK(k >= 2 && k <= OMBO_MAX_OBJ && n_gp >= k && acq->stripes && acq->cells,
                  "EHVI_BOX needs 2 <= n_obj <= %d, n_obj GPs, the breakpoint table and the boxes", OMBO_MAX_OBJ);
-      OMBO_CHECK(acq->kind == OMBO_ACQ_EHVI_BOX || n_gp >= k + 1,
+      OMBO_CHECK(acq->kind != OMBO_ACQ_EHVI_BOX_FEAS || n_gp >= k + 1,
                  "EHVI_BOX_FEAS needs n_obj objective GPs and at least one constraint GP (n_gp = %d, n_obj = %d)",
                  n_gp, k);
       OMBO_CHECK(acq->n_pf >= 2 && acq->n_pf <= OMBO_EHVI_BOX_MAX_BREAKS,
@@ -281,7 +282,7 @@ int ombo_score_pass(ombo_ctx *ctx, const ombo_gp *gps, int n_gp, const ombo_pool
         case OMBO_ACQ_EI: want_var = (g == 0); break;
         case OMBO_ACQ_PARETO_EI: want_var = (g == 1); break;
         case OMBO_ACQ_HV_POI: want_var = (g < 2); break;
-        case OMBO_ACQ_EHVI_BOX: want_var = (g < acq->n_obj); break;
+        case OMBO_ACQ_EHVI_BOX: case OMBO_ACQ_HV_POI_BOX: want_var = (g < acq->n_obj); break;
         default: want_var = true;           // EHVI_BOX_FEAS: the objectives and every constraint
       }
     }
