@@ -85,6 +85,7 @@ int ombo_ctx_create(int device, ombo_ctx **out) {
     k.prune_log = getenv("OMBO_PRUNE_LOG") != nullptr;
     k.prune_stage1 = geti("OMBO_PRUNE_STAGE1", 1) != 0;
     { const char *e = getenv("OMBO_PRUNE_STAGE1_CAP"); k.prune_cap1 = e ? atoll(e) : 0; }
+    { const char *e = getenv("OMBO_STAGE1_KERNEL"); k.stage1_mean8 = e && strcmp(e, "mean8") == 0; }
   }
   OMBO_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; ++i) {
@@ -522,7 +523,10 @@ static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool
                         ombo_best *best_dev, cudaStream_t s, bool *done) {
   *done = false;
   const GpDev gd[2] = {gp_dev_view(gps[0]), gp_dev_view(gps[1])};
-  if (!ctx->knobs.prune_stage1 || !ombo_mean8_covers(gd, acq->n_pf))
+  // stage 1 on the tensor core where it covers the shape and its margin stays small for this pool (decided below),
+  // else (or with OMBO_STAGE1_KERNEL=mean8) the exact-mean kernel
+  bool tc = !ctx->knobs.stage1_mean8 && ombo_stage1_tc_covers(gd, acq->n_pf);
+  if (!ctx->knobs.prune_stage1 || !(tc || ombo_mean8_covers(gd, acq->n_pf)))
     return prune_depth1(ctx, gps, pool, acq, best_dev, s, done);
   const long long m = pool->m;
   const long long cap = ctx->knobs.prune_cap1 > 0 ? ctx->knobs.prune_cap1 : std::max(1LL << 16, m / 8);
@@ -534,7 +538,7 @@ static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool
   size_t cub_bytes = 0;
   OMBO_CUDA(cub::DeviceSelect::If(nullptr, cub_bytes, ids, (long long *)nullptr, (long long *)nullptr, m,
                                   PruneKeep{nullptr, nullptr}, s));
-  const size_t o_top = up(sizeof(PruneHdr)), o_trows = o_top + up((size_t)n_top * 8),
+  const size_t o_ext = up(sizeof(PruneHdr)), o_top = o_ext + 256, o_trows = o_top + up((size_t)n_top * 8),
                o_ub = o_trows + up((size_t)n_top * pool->d * resz), o_sel = o_ub + up((size_t)m * 8),
                o_rows = o_sel + up((size_t)m * 8), o_cub = o_rows + up((size_t)std::min(cap, m) * pool->d * resz);
   if (ombo_ws_reserve(&ctx->ws_prune1, &ctx->ws_prune1_bytes, o_cub + cub_bytes)) {
@@ -555,10 +559,17 @@ static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool
   PoolDev pd;
   fill_pool_dev(pd, pool);
   pd.X = pool->X;
+  if (tc) {
+    rc = ombo_stage1_tc_useful(ctx, gd, pd, m, ws + o_ext, &tc, s);
+    if (rc) return rc;
+    if (!tc && !ombo_mean8_covers(gd, acq->n_pf)) return prune_depth1(ctx, gps, pool, acq, best_dev, s, done);
+  }
   // stage 1: UB1 of every candidate, the per-CTA maxima (ctx->ws_partial) and the largest
   int n_cta = 0;
-  rc = ombo_mean8_bound(ctx, gd, pd, m, acq->stripes, acq->n_pf, (float)acq->cache_c00, (float)acq->cache_c01, ub,
-                        &h->ub, nullptr, &n_cta, s);
+  rc = tc ? ombo_stage1_tc_bound(ctx, gd, pd, m, acq->stripes, acq->n_pf, (float)acq->cache_c00,
+                                 (float)acq->cache_c01, ub, &h->ub, nullptr, nullptr, &n_cta, s)
+          : ombo_mean8_bound(ctx, gd, pd, m, acq->stripes, acq->n_pf, (float)acq->cache_c00, (float)acq->cache_c01, ub,
+                             &h->ub, nullptr, &n_cta, s);
   if (rc) return rc;
   k_prune1_top<<<(unsigned)((n_cta * pool->d + 255) / 256), 256, 0, s>>>(pd, m, (const ombo_best *)ctx->ws_partial,
                                                                          n_cta, top_idx, trows, out_f32);
@@ -576,8 +587,8 @@ static int score_pruned(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool
   OMBO_CUDA(cudaStreamSynchronize(s));
   memcpy(&hh, ctx->pinned_best, sizeof(PruneHdr));
   if (ctx->knobs.prune_log)
-    fprintf(stderr, "[prune1] m %lld survivors %lld ub_max %.9g at %lld v0 %.9g top %d cap %lld\n", m, hh.n_sel,
-            hh.ub.value, (long long)hh.ub.index, hh.v0.value, n_cta, cap);
+    fprintf(stderr, "[prune1] m %lld survivors %lld ub_max %.9g at %lld v0 %.9g top %d cap %lld stage1 %s\n", m,
+            hh.n_sel, hh.ub.value, (long long)hh.ub.index, hh.v0.value, n_cta, cap, tc ? "tc" : "mean8");
   if (!std::isfinite(hh.ub.value) || !(hh.v0.value - OMBO_PRUNE_TAU * hh.ub.value > 0.0) || hh.n_sel > cap)
     return prune_depth1(ctx, gps, pool, acq, best_dev, s, done);
   // stage 2: the depth-1 path on the survivors (local indices into sel), in full if it declines
@@ -870,6 +881,27 @@ int ombo_debug_mean8(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, c
   if (rc) return rc;
   return ombo_mean8_bound(ctx, gd, pd, pool->m, acq->stripes, acq->n_pf, (float)acq->cache_c00,
                           (float)acq->cache_c01, ub, best_dev, mu, nullptr, s);
+}
+
+// the tensor-core stage-1 launch on its own: mu [2][m] (the stage-1 means), marg [2][m] (their margins M), ub [m],
+// the largest bound into *best_dev; OMBO_ERR_UNSUPPORTED where the kernel does not cover the shape
+int ombo_debug_stage1_tc(ombo_ctx *ctx, const ombo_gp *gps, const ombo_pool *pool, const ombo_acq *acq, double *mu,
+                         double *marg, double *ub, ombo_best *best_dev, void *stream) {
+  OMBO_CHECK(ctx && gps && pool && acq && mu && marg && ub && best_dev, "debug_stage1_tc: NULL argument");
+  OMBO_CHECK(acq->kind == OMBO_ACQ_EHVI2D && acq->stripes && acq->n_pf >= 1, "debug_stage1_tc: needs an EHVI2D spec");
+  for (int g = 0; g < 2; ++g)
+    OMBO_CHECK(gps[g].state && (gps[g].reserved & OMBO_GP_F8C_PLANES) && gps[g].d == pool->d,
+               "debug_stage1_tc: gp %d has no f8c planes or the wrong d", g);
+  OMBO_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  PoolDev pd;
+  fill_pool_dev(pd, pool);
+  pd.X = pool->X;
+  const GpDev gd[2] = {gp_dev_view(gps[0]), gp_dev_view(gps[1])};
+  int rc = ombo_best_init(ctx, best_dev, s);
+  if (rc) return rc;
+  return ombo_stage1_tc_bound(ctx, gd, pd, pool->m, acq->stripes, acq->n_pf, (float)acq->cache_c00,
+                              (float)acq->cache_c01, ub, best_dev, mu, marg, nullptr, s);
 }
 
 int64_t ombo_launch_count(ombo_ctx *ctx, int reset) {

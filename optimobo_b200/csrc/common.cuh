@@ -59,6 +59,7 @@ struct ombo_knobs {
   int prune_stage1;       // OMBO_PRUNE_STAGE1=0: no mean-only first stage in front of the variance bound
   long long prune_cap1;   // OMBO_PRUNE_STAGE1_CAP: most stage-1 survivors before the depth-1 path takes the whole pool
                           //   (0: max(2^16, m / 8))
+  int stage1_mean8;       // OMBO_STAGE1_KERNEL=mean8: stage 1 on k_posterior_mean8 even where the tensor-core kernel covers
 };
 
 struct ombo_ctx {
@@ -231,6 +232,17 @@ bool ombo_mean8_covers(const GpDev gp[2], int n_pf);
 int ombo_mean8_bound(ombo_ctx *ctx, const GpDev gp[2], const PoolDev &pool, long long m, const double *stripes,
                      int n_pf, float c00, float c01, double *ub, ombo_best *best_dev, double *mu_out, int *grid_out,
                      cudaStream_t s);
+// posterior_stage1_tc.cu: the same bound with tcgen05 distances and a certified margin on each mean (the default stage
+// 1 where it covers the shape: d <= 12, both training sets' fp16 planes in shared memory); mu_out / marg_out
+// (optional, [2][m] each): the stage-1 means and their margins
+bool ombo_stage1_tc_covers(const GpDev gp[2], int n_pf);
+// whether its margin stays small enough to prune well for this pool (the largest a2 and |b|^2 of both GPs, from the
+// pool's box or a scan; ws: 32 bytes of device workspace; one stream synchronise)
+int ombo_stage1_tc_useful(ombo_ctx *ctx, const GpDev gp[2], const PoolDev &pool, long long m, void *ws, bool *useful,
+                          cudaStream_t s);
+int ombo_stage1_tc_bound(ombo_ctx *ctx, const GpDev gp[2], const PoolDev &pool, long long m, const double *stripes,
+                         int n_pf, float c00, float c01, double *ub, ombo_best *best_dev, double *mu_out,
+                         double *marg_out, int *grid_out, cudaStream_t s);
 // merges n_partials per-block (value, index) pairs in ctx->ws_partial with the running best
 int ombo_argmax_merge(ombo_ctx *ctx, int n_partials, ombo_best *best_dev, cudaStream_t s);
 int ombo_fast_path_built();
